@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the VPP + rSGM hot path (BASELINE.json: "VPP pairs/s & rSGM fps @1242x375, 5% hints, D=192; % of HBM peak").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path (VPP random-pattern projection, then compute_rsgm: census, Hamming cost volume,
 8-path SGM, WTA + sub-pixel, LR check, speckle filter, fills) over one batch of synthetic KITTI-shape pairs
@@ -14,6 +14,8 @@ One step = one pass of the hot path (VPP random-pattern projection, then compute
              MEASURED_PEAKS.json hbm_gbs; the whole aggregation against SURVEY.md 8d's 4*W*H*D + W*H is reported beside it
   cpu_baseline  the reference's own CPU code (oracle/_ref) on the host cores, bounded sample, rank 0 at N=1
 --impl reference: times that CPU path instead, same metric/config, all host cores.
+--dump-outputs DIR: writes what the last timed step computed as float32 .npy files (see dump_outputs); the inputs and the
+pattern seeds depend on the arguments only, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -311,6 +313,26 @@ def ncu_traffic():
         return None, None
 
 
+DUMP_FRAMES = 16              # disparity maps written by --dump-outputs: a fixed, seeded choice of frames of the batch
+DUMP_PAIRS = 2                # ... and the projected pairs of the first two of them
+
+
+def dump_outputs(outdir, disp, lv, rv):
+    """Writes what one step of the pipeline computed, as float32: disparity.npy [16,H,W] (the disparities run_device returns, for
+    16 frames chosen with a fixed seed: the whole batch is 119 MB), left_vpp.npy / right_vpp.npy [2,H,W,C] (the projected pair
+    of the first two of those frames, uint8 values) and disparity_frames.npy (the batch indices of the 16 frames).  52 MB."""
+    import numpy as np
+    import torch
+    frames = np.sort(np.random.default_rng(0).choice(disp.shape[0], min(DUMP_FRAMES, disp.shape[0]), replace=False))
+    idx = torch.from_numpy(frames).to(disp.device)
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {"disparity": disp.index_select(0, idx), "left_vpp": lv.index_select(0, idx[:DUMP_PAIRS]),
+              "right_vpp": rv.index_select(0, idx[:DUMP_PAIRS])}
+    for name, t in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), t.float().cpu().numpy())
+    np.save(os.path.join(outdir, "disparity_frames.npy"), frames.astype(np.float32))
+
+
 def time_steps(step, n, sync_all, torch):
     """n calls of step() between two CUDA events on the current stream, barrier + synchronize on both sides -> ms"""
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -326,18 +348,28 @@ def time_steps(step, n, sync_all, torch):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps, exactly (default: 200 for --workload K, 3 for M, 30 for nets)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch", type=int, default=64, help="frames per GPU per step (configs[1]: 64)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="K", choices=["K", "M", "nets"],
                     help="K = configs[1] (default, the metric's configuration); M = configs[2] (Middlebury frame, maxDistance + occlusion "
                          "mask, row bands across the GPUs); nets = configs[3] (VPP -> RAFT-Stereo / PSMNet as device tensors)")
-    ap.add_argument("--sustained-steps", type=int, default=200, help="steps of the additional >= 5 s measurement (0 = off)")
+    ap.add_argument("--sustained-steps", type=int, default=0,
+                    help="steps of an additional measurement reported beside the --steps one, e.g. 200 for >= 5 s (0 = off)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-frames", type=int, default=0, help="frames in the cpu_baseline sample (default: one per core)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (rank 0's batch) to DIR/*.npy, float32, 52 MB")
     ap.add_argument("--cpu-worker", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "K" or args.impl != "b200"):
+        ap.error("--dump-outputs is implemented for --workload K --impl b200 only")
+    if args.steps is None and args.workload == "K":
+        args.steps = 200
     if args.cpu_worker:
         return cpu_worker_main(args.cpu_worker)
     if args.impl == "reference" and args.workload == "nets":
@@ -432,6 +464,9 @@ def main():
     launches0 = _lib.launch_count()
     ms_total = time_steps(step_device, args.steps, sync_all, torch)
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        # run_device returns pipe.disp; pipe.lv / pipe.rv hold the projected pair of the latest call (the steps below overwrite them)
+        dump_outputs(args.dump_outputs, pipe.disp, pipe.lv, pipe.rv)
     # the same, sustained over >= 5 s (power and clocks settle): reported beside the --steps figure
     sus_n = args.sustained_steps if args.sustained_steps > args.steps else 0
     ms_sus = time_steps(step_device, sus_n, sync_all, torch) if sus_n else None
@@ -581,4 +616,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True        # the benchmark writes nothing into the tree it runs from (which may be read-only)
     main()

@@ -87,7 +87,7 @@ def main(args, reference=False):
     # (8 M frames = 8 teams of 18 SMs in the v-sweeps, ~8.5 GB of workspace each)
     B = args.batch if args.batch != 64 else 48
     CHUNK = 8
-    steps = min(args.steps, 5) if args.steps != 200 else 3
+    steps = args.steps if args.steps is not None else 3
     uniq = [synth.make_pair(rank * 100 + f, shape="M", hints="random") for f in range(2)]
     idx = [i % 2 for i in range(B)]
     host = tuple(torch.from_numpy(np.stack([uniq[i][k] for i in idx])).pin_memory() for k in ("left", "right", "hints"))

@@ -42,7 +42,7 @@ def main(args, reference=False):
     import bench
     torch.cuda.set_device(0)
     dev = torch.device("cuda", 0)
-    steps = min(args.steps, 30)
+    steps = args.steps if args.steps is not None else 30
     frames = [synth.make_pair(f, shape="K", hints="lidar") for f in range(4)]
     pinned = [tuple(torch.from_numpy(p[k]).pin_memory() for k in ("left", "right", "hints")) for p in frames]
     resident = [tuple(t.to(dev) for t in fr) for fr in pinned]
