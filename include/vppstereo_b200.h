@@ -134,7 +134,7 @@ int vppb200_median3x3(const float *src, float *dst, int W, int H, int n, void *s
  * compute_rsgm(left, left_vpp, right_vpp, hints, validhints, dmax, ..., subpixel)   models/rsgm/rsgm.py:250-294.
  * Inputs uint8 [n][H][W][C] (C = 1 or 3; `left` is the adaptive-P2 guide), optional hints/validhints float32
  * [n][H][W] (both NULL = unguided), output float32 [n][H][W].  p1/p2min/alpha/gamma do not exist here because
- * the reference ignores them.  flags: bit0 = subpixel. */
+ * the reference ignores them (vppb200_compute_rsgm_ex honours them on request).  flags: bit0 = subpixel. */
 size_t vppb200_rsgm_workspace_bytes(int H, int W, int C, int D, int n);
 int vppb200_compute_rsgm(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp,
                          const float *hints, const float *validhints, float *disp_out,
@@ -174,6 +174,37 @@ int vppb200_compute_rsgm_tapped(const uint8_t *left, const uint8_t *left_vpp, co
                                 void *workspace, size_t workspace_bytes, int n, void *stream,
                                 const vppb200_rsgm_taps *taps);
 
+/* ---- honoured SGM parameters (an opt-in the reference does not have: it parses P1..Gamma and overwrites them with 7, 17,
+ * 0.25, 50, RSGM/pyrSGM.cpp:519 vs :557-560).  Semantics: the reference's StereoSGM recursion with the parameters as arguments
+ * (RSGM/StereoSGM_SSE.hpp:13-515), P2 = max(p2min, (int32)(-alpha * |I_p - I_pr| + gamma)) in float32 with the two operations
+ * rounded separately (RSGM/StereoSGM.hpp:92-99).
+ *   vppb200_compute_rsgm_ex: vppb200_compute_rsgm_phases + taps (phases == 7 only, as vppb200_compute_rsgm_tapped) + params.
+ *       params == NULL: the reference's effective values (7, 17, 0.25, 50) -- exactly what the other entry points do.  Every
+ *       phase of one batch must be called with the same params and hints (they select the layout of the cost volume).
+ *   vppb200_sgm_band_ex: vppb200_sgm_band + params; refuses parameters outside the sweep domain (there is no per-path band path).
+ *   vppb200_sgm_params_fast: 1 = the four sweeps compute these parameters, 0 = compute_rsgm falls back to the per-path kernels,
+ *       VPPB200_ERR_ARG = invalid.  guided: costs modulated by hints (up to 240) instead of plain Hamming costs (up to 24).
+ * Validation (before any CUDA call, VPPB200_ERR_ARG otherwise): 0 <= p1, p2min, gamma <= 65535; alpha finite and >= 0, so that
+ * P2 lies in [p2min, P2max], P2max = max(p2min, gamma).
+ * Sweep domain, Cmax = 24 (Hamming) or 240 (guided): p1 <= p2min, P2max - p1 <= 255 and Cmax + P2max <= 4095.  Inside it the four
+ * sweeps run as for the default parameters (same speed, no saturation reachable).  Outside it the aggregation runs on the
+ * saturating per-path kernels (8 launches, each a read-modify-write of the whole aggregated volume: several times slower),
+ * bit-exact with the recursion including its uint16 saturation.  Parameters are kernel arguments: calls with different
+ * parameters may run concurrently on different streams. */
+typedef struct {
+    int p1;
+    int p2min;
+    float alpha;
+    int gamma;
+} vppb200_sgm_params;
+int vppb200_compute_rsgm_ex(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp,
+                            const float *hints, const float *validhints, float *disp_out,
+                            int H, int W, int C, int D, int flags, const float *rcp_lut,
+                            void *workspace, size_t workspace_bytes, int n, void *stream,
+                            int phases, int sets, int set, const vppb200_rsgm_taps *taps,
+                            const vppb200_sgm_params *params);
+int vppb200_sgm_params_fast(const vppb200_sgm_params *params, int guided);
+
 /* ---- one frame split into row bands over several GPUs (SURVEY.md 8e: an oversized frame) -------------------------------
  * compute_rsgm (models/rsgm/rsgm.py:250-294) as three calls so that the aggregation -- the 2.2 GB of volumes of a Middlebury
  * frame -- runs band by band on different GPUs, EXACTLY (unlike the reference's approximate StripedStereoSGM,
@@ -198,6 +229,10 @@ int vppb200_sgm_band(const uint8_t *guide, const uint32_t *census_l, const uint3
                      uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
                      uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
                      size_t workspace_bytes, void *stream);
+int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                        uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
+                        uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
+                        size_t workspace_bytes, void *stream, const vppb200_sgm_params *params);
 int vppb200_rsgm_tail(float *dl, float *dr, float *disp_out, int H, int W, int C, int D, int flags, void *workspace,
                       size_t workspace_bytes, void *stream);
 

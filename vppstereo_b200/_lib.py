@@ -28,6 +28,7 @@ SYMBOLS = [
     "vppb200_u8hwc_to_f32chw", "vppb200_set_tuning",
     "vppb200_occlusion_workspace_bytes", "vppb200_occlusion_heuristic",
     "vppb200_banded_workspace_bytes", "vppb200_banded_dims", "vppb200_rsgm_front_census", "vppb200_sgm_band", "vppb200_rsgm_tail",
+    "vppb200_compute_rsgm_ex", "vppb200_sgm_band_ex", "vppb200_sgm_params_fast",
 ]
 
 _lib = None
@@ -36,6 +37,40 @@ _lib = None
 class RsgmTaps(C.Structure):
     _fields_ = [("census_l", C.c_void_p), ("census_r", C.c_void_p), ("dsi_agg", C.c_void_p),
                 ("disp_l", C.c_void_p), ("disp_r", C.c_void_p)]
+
+
+class VppSgmParams(C.Structure):
+    """vppb200_sgm_params: the SGM penalties a caller asks compute_rsgm to honour"""
+    _fields_ = [("p1", C.c_int), ("p2min", C.c_int), ("alpha", C.c_float), ("gamma", C.c_int)]
+
+
+def sgm_params(p1, p2min, alpha, gamma):
+    """(p1, p2min, alpha, gamma) -> VppSgmParams, validated on the host (no device needed): ValueError unless
+    0 <= p1, p2min, gamma <= 65535 are integers and alpha is finite and >= 0 (include/vppstereo_b200.h)."""
+    vals = {}
+    for name, v in (("p1", p1), ("p2min", p2min), ("gamma", gamma)):
+        try:
+            iv = int(v)
+        except (TypeError, ValueError, OverflowError):
+            raise ValueError(f"{name} must be an integer in [0, 65535], got {v!r}") from None
+        if iv != v or not 0 <= iv <= 65535:
+            raise ValueError(f"{name} must be an integer in [0, 65535], got {v!r}")
+        vals[name] = iv
+    try:
+        a = float(alpha)
+    except (TypeError, ValueError):
+        raise ValueError(f"alpha must be a finite number >= 0, got {alpha!r}") from None
+    if not (np.isfinite(a) and a >= 0.0) or not np.isfinite(np.float32(a)):
+        raise ValueError(f"alpha must be a finite number >= 0, got {alpha!r}")
+    prm = VppSgmParams(vals["p1"], vals["p2min"], a, vals["gamma"])
+    if lib().vppb200_sgm_params_fast(C.byref(prm), 0) < 0:           # the library's own validation (same rules)
+        raise ValueError(f"invalid SGM parameters {(p1, p2min, alpha, gamma)}")
+    return prm
+
+
+def sgm_params_fast(prm, guided=False):
+    """True if the four sweeps compute these parameters (otherwise compute_rsgm falls back to the per-path kernels)."""
+    return lib().vppb200_sgm_params_fast(C.byref(prm), int(bool(guided))) == 1
 
 
 def lib():

@@ -27,7 +27,15 @@ PH_COST, PH_H_FWD, PH_V_DOWN, PH_V_UP, PH_H_BWD = 1, 2, 4, 8, 16
 
 
 class BandedRsgm:
-    def __init__(self, H, W, channels=3, dmax=192, n_bands=2, subpixel=True, device=None):
+    def __init__(self, H, W, channels=3, dmax=192, n_bands=2, subpixel=True, device=None, sgm_params=None):
+        # sgm_params: (p1, p2min, alpha, gamma) honoured by the sweeps; None = the reference's effective values.  Bands exist on the
+        # sweeps only, so parameters outside their domain (include/vppstereo_b200.h) are refused here.
+        self.sgm_params = None
+        if sgm_params is not None:
+            prm = _lib.sgm_params(*sgm_params)
+            if not _lib.sgm_params_fast(prm, guided=False):
+                raise ValueError(f"SGM parameters {tuple(sgm_params)} are outside the sweep domain (no banded path for them)")
+            self.sgm_params = prm
         torch = _lib.require_cuda()
         self.torch = torch
         self.H, self.W, self.C, self.D = int(H), int(W), int(channels), int(dmax)
@@ -98,9 +106,11 @@ class BandedRsgm:
         dr = self.dr[row0:row0 + rows]
         with torch.cuda.device(self.device):
             st = _lib.stream_ptr(self.device) if stream is None else C.c_void_p(stream.cuda_stream)
-            rc = self.lib.vppb200_sgm_band(_lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost), _lib.ptr(S),
-                                           self.H, self.W, self.C, self.D, row0, rows, int(phases), _lib.ptr(state_in), _lib.ptr(state_out),
-                                           _lib.ptr(dl), _lib.ptr(dr), None, _lib.ptr(self.ws), C.c_size_t(self.ws.numel()), st)
+            prm = None if self.sgm_params is None else C.byref(self.sgm_params)
+            rc = self.lib.vppb200_sgm_band_ex(_lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost), _lib.ptr(S),
+                                              self.H, self.W, self.C, self.D, row0, rows, int(phases), _lib.ptr(state_in),
+                                              _lib.ptr(state_out), _lib.ptr(dl), _lib.ptr(dr), None, _lib.ptr(self.ws),
+                                              C.c_size_t(self.ws.numel()), st, prm)
         _lib.check(rc, "sgm_band")
 
     def tail(self, out=None):
@@ -138,13 +148,13 @@ class BandedRsgmDist(BandedRsgm):
     travels rank r -> r+1 (pass 0) and r -> r-1 (pass 1), the raw disparity bands go to every rank, every rank runs the (cheap,
     whole-frame) tail and returns the full disparity map.  Transfers: dist.PeerGather (peer-mapped buffers, DMA, flag words)."""
 
-    def __init__(self, H, W, channels=3, dmax=192, subpixel=True, device=None, group=None):
+    def __init__(self, H, W, channels=3, dmax=192, subpixel=True, device=None, group=None, sgm_params=None):
         import torch.distributed as dist
         from .dist import PeerGather
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
-        super().__init__(H, W, channels, dmax, n_bands=self.world, subpixel=subpixel, device=device)
+        super().__init__(H, W, channels, dmax, n_bands=self.world, subpixel=subpixel, device=device, sgm_params=sgm_params)
         if len(self.bands) != self.world:
             raise ValueError("frame too small for one band per rank")
         torch = self.torch

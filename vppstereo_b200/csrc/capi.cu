@@ -4,6 +4,7 @@
 #include "common.cuh"
 
 #include <atomic>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <mutex>
@@ -143,6 +144,17 @@ static int stream_chain(cudaStream_t from, cudaStream_t to)
 }
 
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// vppb200_sgm_params -> SgmParams; NULL = the reference's effective values.  Host only: runs before any CUDA call.
+static int sgm_params_from(const vppb200_sgm_params *q, SgmParams *out)
+{
+    if (!q) { *out = default_sgm_params(); return VPPB200_OK; }
+    auto u16 = [](int v) { return v >= 0 && v <= 65535; };
+    if (!u16(q->p1) || !u16(q->p2min) || !u16(q->gamma)) return VPPB200_ERR_ARG;
+    if (!std::isfinite(q->alpha) || !(q->alpha >= 0.0f)) return VPPB200_ERR_ARG;     // then P2 in [P2min, max(P2min, gamma)]
+    *out = SgmParams{q->p1, q->p2min, q->gamma, q->alpha};
+    return VPPB200_OK;
+}
 
 struct RsgmWs {
     uint8_t *gray_l, *gray_r, *guide;
@@ -409,8 +421,10 @@ extern "C" size_t vppb200_rsgm_workspace_bytes_sets(int H, int W, int C, int D, 
 static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
                        const float *validhints, float *disp_out, int H, int W, int C, int D, int flags, const float *rcp_lut,
                        void *workspace, size_t workspace_bytes, int n, void *stream, const vppb200_rsgm_taps *taps, int phases,
-                       int sets, int set)
+                       int sets, int set, const vppb200_sgm_params *params)
 {
+    SgmParams prm;
+    if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
     if (H <= 0 || W <= 0 || n <= 0 || (C != 1 && C != 3)) return VPPB200_ERR_ARG;
     if (D <= 0 || D % 8 != 0 || D > 256) return VPPB200_ERR_DISP;      // models/rsgm/rsgm.py:31-35
     if (phases <= 0 || phases > 7 || sets < 1 || sets > 4 || set < 0 || set >= sets) return VPPB200_ERR_ARG;
@@ -430,7 +444,10 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
     int rc;
     StageMarks tm;
     if (phases == 7) tm.begin(st);                           // per-stage timing covers whole-pipeline calls only
-    const bool tiled = aggregate_tile_supported(d.Wp, d.Hp, D, n);
+    // the sweeps for parameters of their domain (the layout of the cost volume follows: every phase of a batch must see the same
+    // parameters and hints); otherwise the per-path kernels, saturating where the parameters make that reachable
+    const bool fast_params = sweep_params_supported(prm, hints == nullptr);
+    const bool tiled = fast_params && aggregate_tile_supported(d.Wp, d.Hp, D, n);
     const bool want_volume = taps && taps->dsi_agg;          // only the test tap needs the aggregated volume itself
     const uint16_t *S_final = w.S;
     if (front) {
@@ -464,23 +481,27 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
         tm.done(VPPB200_STAGE_COST);
     }
     if (mainp) {
-        // rsgm.py:270  8-path aggregation (effective default parameters); rsgm.py:272-273  WTA left (+ equiangular
-        // sub-pixel) and right
+        // rsgm.py:270  8-path aggregation (the reference's effective parameters unless the caller passed its own);
+        // rsgm.py:272-273  WTA left (+ equiangular sub-pixel) and right
         if (tiled) {
             const StageHook hook = {StageMarks::hook, &tm};
             if (!want_volume) {
                 // the last sweep consumes the final S on the fly: WTA left (+ sub-pixel) and right come out of the aggregation
-                if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, w.dl, w.dr, rcp_lut, hints == nullptr, &hook, st)))
+                if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, w.dl, w.dr, rcp_lut, hints == nullptr, prm, &hook,
+                                                st)))
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
             } else {
-                if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, nullptr, nullptr, nullptr, hints == nullptr, &hook, st)))
+                if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, nullptr, nullptr, nullptr, hints == nullptr, prm,
+                                                &hook, st)))
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
                 if ((rc = launch_s_tile_to_xyd(w.S, w.S_xyd, d.Wp, d.Hp, D, n, st))) return rc;
                 S_final = w.S_xyd;
                 if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, 0, n, st))) return rc;
             }
         } else {
-            if ((rc = launch_aggregate_fast(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, n, st))) return rc;
+            if (fast_params) rc = launch_aggregate_fast(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
+            else rc = launch_aggregate_generic_u8(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
+            if (rc) return rc;
             tm.done(VPPB200_STAGE_SGM_H_BWD);                // the per-path fallback is booked on the last sweep's slot
             if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, 0, n, st))) return rc;
         }
@@ -518,7 +539,7 @@ extern "C" int vppb200_compute_rsgm_tapped(const uint8_t *left, const uint8_t *l
                                            int n, void *stream, const vppb200_rsgm_taps *taps)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, taps, 7, 1, 0);
+                       workspace_bytes, n, stream, taps, 7, 1, 0, nullptr);
 }
 
 extern "C" int vppb200_compute_rsgm(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
@@ -526,7 +547,7 @@ extern "C" int vppb200_compute_rsgm(const uint8_t *left, const uint8_t *left_vpp
                                     const float *rcp_lut, void *workspace, size_t workspace_bytes, int n, void *stream)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, nullptr, 7, 1, 0);
+                       workspace_bytes, n, stream, nullptr, 7, 1, 0, nullptr);
 }
 
 extern "C" int vppb200_compute_rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp,
@@ -535,7 +556,23 @@ extern "C" int vppb200_compute_rsgm_phases(const uint8_t *left, const uint8_t *l
                                            int n, void *stream, int phases, int sets, int set)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, nullptr, phases, sets, set);
+                       workspace_bytes, n, stream, nullptr, phases, sets, set, nullptr);
+}
+
+extern "C" int vppb200_compute_rsgm_ex(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
+                                       const float *validhints, float *disp_out, int H, int W, int C, int D, int flags,
+                                       const float *rcp_lut, void *workspace, size_t workspace_bytes, int n, void *stream, int phases,
+                                       int sets, int set, const vppb200_rsgm_taps *taps, const vppb200_sgm_params *params)
+{
+    return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
+                       workspace_bytes, n, stream, taps, phases, sets, set, params);
+}
+
+extern "C" int vppb200_sgm_params_fast(const vppb200_sgm_params *params, int guided)
+{
+    SgmParams prm;
+    if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
+    return sweep_params_supported(prm, !guided) ? 1 : 0;
 }
 
 // ---- one frame split into row bands over several GPUs (SURVEY.md 8e rows 2 and 5) ------------------------------
@@ -599,11 +636,14 @@ extern "C" int vppb200_rsgm_front_census(const uint8_t *left, const uint8_t *lef
     return launch_census(w.gray_l, census_l, d.Wp, d.Hp, 1, st);
 }
 
-extern "C" int vppb200_sgm_band(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
-                                uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
-                                uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
-                                size_t workspace_bytes, void *stream)
+extern "C" int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                                   uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
+                                   uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
+                                   size_t workspace_bytes, void *stream, const vppb200_sgm_params *params)
 {
+    SgmParams prm;
+    if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
+    if (!sweep_params_supported(prm, true)) return VPPB200_ERR_ARG;      // bands exist on the sweeps only
     if (!guide || !cost_band || !S_band || H <= 0 || W <= 0 || (C != 1 && C != 3) || phases <= 0 || phases > 31) return VPPB200_ERR_ARG;
     if (D <= 0 || D % 8 != 0 || D > 256) return VPPB200_ERR_DISP;
     if ((phases & 1) && (!census_l || !census_r)) return VPPB200_ERR_ARG;
@@ -616,7 +656,16 @@ extern "C" int vppb200_sgm_band(const uint8_t *guide, const uint32_t *census_l, 
     if (!rcp_lut) rcp_lut = device_rcp_lut(st);
     if (!rcp_lut) return cuda_fail("device_rcp_lut", cudaGetLastError());
     return launch_aggregate_band(guide, census_l, census_r, cost_band, S_band, w.halo, d.Wp, d.Hp, D, row0, rows, 1, phases, state_in,
-                                 state_out, dl_band, dr_band, rcp_lut, true, st);
+                                 state_out, dl_band, dr_band, rcp_lut, true, prm, st);
+}
+
+extern "C" int vppb200_sgm_band(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                                uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
+                                uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
+                                size_t workspace_bytes, void *stream)
+{
+    return vppb200_sgm_band_ex(guide, census_l, census_r, cost_band, S_band, H, W, C, D, row0, rows, phases, state_in, state_out,
+                               dl_band, dr_band, rcp_lut, workspace, workspace_bytes, stream, nullptr);
 }
 
 extern "C" int vppb200_rsgm_tail(float *dl, float *dr, float *disp_out, int H, int W, int C, int D, int flags, void *workspace,

@@ -42,6 +42,22 @@ static inline RsgmDims make_dims(int H, int W, int C, int D)
     return d;
 }
 
+// The four SGM penalties (RSGM/StereoSGM.h:33-47).  The reference's effective values are P1 = 7, P2min = 17, alpha = 0.25,
+// gamma = 50 (RSGM/pyrSGM.cpp:557-560); callers that honour their own parameters pass them through vppb200_sgm_params.
+struct SgmParams {
+    int P1, P2min, gamma;
+    float alpha;
+};
+static inline SgmParams default_sgm_params() { return SgmParams{7, 17, 50, 0.25f}; }
+
+// adaptP2 (RSGM/StereoSGM.hpp:92-99): (sint32)(-alpha * |I_p - I_pr| + gamma), clamped below by P2min.  Two separately rounded
+// float operations, as the reference's expression compiles without contraction; the only evaluation of P2 in the library.
+__device__ __forceinline__ int adapt_p2(const SgmParams &p, int ip, int ipr)
+{
+    const int r = (int)__fadd_rn(__fmul_rn(-p.alpha, (float)abs(ip - ipr)), (float)p.gamma);
+    return r < p.P2min ? p.P2min : r;
+}
+
 // ---- stage launchers (defined in the .cu files, all asynchronous on `st`) -------------------------------
 int launch_pad_gray(const uint8_t *src, uint8_t *gray, const RsgmDims &d, int n, cudaStream_t st);
 int launch_pad_flatbytes(const uint8_t *src, uint8_t *guide, const RsgmDims &d, int n, cudaStream_t st);
@@ -51,12 +67,18 @@ int launch_census_fused(const uint8_t *src, uint32_t *dst, const RsgmDims &d, in
 int launch_cost_u16(const uint32_t *cl, const uint32_t *cr, uint16_t *dsi, int W, int H, int D, int n, cudaStream_t st);
 int launch_cost_u8(const uint32_t *cl, const uint32_t *cr, uint8_t *dsi, int W, int H, int D, int n, cudaStream_t st);
 int launch_guided_u8(uint8_t *dsi, const float *hints, const float *valid, const RsgmDims &d, int n, cudaStream_t st);
-// generic (saturating, u16 cost) and fast (u8 cost, default params) 8-path aggregation
+// generic (saturating, u16 or u8 costs, any parameters) and fast (u8 costs, parameters of the sweep domain) 8-path aggregation
 int launch_aggregate_generic(const uint8_t *img, const uint16_t *dsi, uint16_t *S, int W, int H, int D, int P1, int P2min,
                              float alpha, int gamma, int n, cudaStream_t st);
-int launch_aggregate_fast(const uint8_t *img, const uint8_t *dsi, uint16_t *S, int W, int H, int D, int n, cudaStream_t st);
+int launch_aggregate_generic_u8(const uint8_t *img, const uint8_t *dsi, uint16_t *S, int W, int H, int D, const SgmParams &p, int n,
+                                cudaStream_t st);
+int launch_aggregate_fast(const uint8_t *img, const uint8_t *dsi, uint16_t *S, int W, int H, int D, const SgmParams &p, int n,
+                          cudaStream_t st);
 // sgm_sweep.cu: layout-T cost volume + 4-sweep aggregation with on-chip path state (cluster per frame)
 bool aggregate_tile_supported(int W, int H, int D, int n);
+// do the sweeps (and the fast per-path kernels) compute these parameters exactly?  plain_costs: Hamming costs (<= 24), otherwise
+// guided costs (<= 240)
+bool sweep_params_supported(const SgmParams &p, bool plain_costs);
 size_t tile_volume_elems(int W, int H, int D, int n);
 int launch_cost_tile(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int H, int D, int n, cudaStream_t st);
 int launch_cost_tile_band(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int Hfull, int D, int row0, int rows, int n,
@@ -64,13 +86,15 @@ int launch_cost_tile_band(const uint32_t *cl, const uint32_t *cr, uint8_t *cost,
 long sweep_state_words(int W, int D);
 int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full, const uint32_t *cen_r_full, uint8_t *cost8, uint16_t *S16,
                           void *halo_ws, int W, int Hfull, int D, int row0, int rows, int n, int phases, const uint32_t *state_in,
-                          uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, cudaStream_t st);
+                          uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &p,
+                          cudaStream_t st);
 int launch_guided_tile(uint8_t *cost, const float *hints, const float *valid, const RsgmDims &d, int n, cudaStream_t st);
 struct StageHook { void (*fn)(void *, int); void *ctx; };   // called with VPPB200_STAGE_* when that stage has been queued
 size_t sweep_halo_bytes(int W, int H, int D, int n);       // workspace of the v-sweep: inter-CTA halo lines, abort flag, P2 table
 // plain_costs: the costs are plain Hamming distances (<= 24, no guided modulation): un-normalised path state in the v-sweeps
+// p must satisfy sweep_params_supported(p, plain_costs)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost, uint16_t *S, void *halo_ws, int W, int H, int D, int n, float *dl,
-                          float *dr, const float *lut, bool plain_costs, const StageHook *hook, cudaStream_t st);
+                          float *dr, const float *lut, bool plain_costs, const SgmParams &p, const StageHook *hook, cudaStream_t st);
 void sweep_set_v_red(int on);
 void sweep_set_v_split(int on);
 int sweep_take_abort_flag(int *out);

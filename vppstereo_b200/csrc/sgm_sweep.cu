@@ -19,9 +19,16 @@
 // words in global memory (4 tag bits per word, polled: no fence, no barrier between CTAs); one __syncthreads per row.
 // Lines that enter through the image border read a constant "border slot".
 //
-// Arithmetic: the "fast" domain of sgm.cu -- uint8 costs, the effective default parameters (P1=7, P2min=17,
-// Alpha=0.25, Gamma=50 => P2 in [17,50]), so no uint16 saturation is reachable (L <= 255+50, S <= 8*305); packed
-// u16x2 DPX min/add (VIMNMX3 / VIADDMNMX).
+// Arithmetic: packed u16x2 DPX min/add (VIMNMX3 / VIADDMNMX) without saturation, exact inside the parameter domain that
+// sweep_params_supported() states (P1, P2min, alpha, gamma are kernel arguments; P2 in [P2min, P2max], P2max = max(P2min,
+// gamma); Cmax = 24 for Hamming costs, 240 for guided costs):
+//   P1 <= P2min                 the recurrences form min(L[d-1], L[d+1], min + P2 - P1) + P1 in unsigned halves
+//   P2max - P1 <= 255           sgm_p2_kernel packs P2 - P1 of three paths into bytes
+//   Cmax + P2max <= 4095        a line handed to the neighbour CTA, relative to its part minimum, leaves the 4 tag bits of
+//                               its word free; then L <= Cmax + P2max and S <= 8 * (Cmax + P2max) never saturate either
+// and the v-sweeps keep their path state un-normalised only while 24 * H + P2max + 78 < 65536 (Hamming costs; see
+// sgm_v2_kernel).  With the reference's effective values (7, 17, 0.25, 50) that is the fixed 24 * H + 128 rule of old.
+// Parameters outside the domain are aggregated by the saturating per-path kernels of sgm.cu instead.
 //
 // Internal "tile" layout T of the cost volume and of S (K2 = D/2 words per pixel, G = ceil(W/32) column groups):
 //   word (y, x, k) = (((y*G + x/32)*K2 + k)*32 + x%32), low half = disparity k, high half = disparity k + K2 ("split-half"
@@ -41,9 +48,6 @@ namespace cg = cooperative_groups;
 namespace vppb200 {
 
 #define SW_BIG2 0x3FFF3FFFu
-static constexpr int SW_P1 = 7, SW_P2MIN = 17, SW_GAMMA = 50;
-static constexpr float SW_ALPHA = 0.25f;
-static constexpr uint32_t SW_P1X2 = 0x00070007u;
 
 struct TL {
     int W, H, D, K2, G;
@@ -55,16 +59,6 @@ static TL make_tl(int W, int H, int D)
     t.W = W; t.H = H; t.D = D; t.K2 = D / 2; t.G = (W + 31) / 32;
     t.frame = (long)H * t.G * t.K2 * 32;
     return t;
-}
-
-__device__ __forceinline__ int sw_adapt_p2(int ip, int ipr)
-{
-    // (sint32)(-alpha * abs(I_p - I_pr) + gamma), clamped below by P2min  (RSGM/StereoSGM.hpp:92-99)
-    // With alpha = 1/4 and gamma = 50 the float expression is exact and its truncation is 50 - ceil(|dI| / 4) (checked for all 256
-    // differences against the float form): three integer instructions
-    static_assert(SW_ALPHA == 0.25f && SW_GAMMA == 50, "the closed form below is for alpha = 1/4, gamma = 50");
-    const int r = SW_GAMMA - ((abs(ip - ipr) + 3) >> 2);
-    return r < SW_P2MIN ? SW_P2MIN : r;
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -256,12 +250,12 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// one SGM step on normalised state: nw = c + min(w[k], min(w[k-1], w[k+1]) + P1, P2);  p2m = (P2 - P1) * 0x10001.
+// one SGM step on normalised state: nw = c + min(w[k], min(w[k-1], w[k+1]) + P1, P2);  p2m = (P2 - P1) * 0x10001, p1x2 = P1 * 0x10001.
 // FULLK: K2 == 32 * NW (every word of every lane is real); otherwise jl = index of this lane's last real word (-1: none),
 // `last` = this lane holds word K2-1.
 template <int NW, bool FULLK>
-__device__ __forceinline__ void sw_step(const uint32_t (&w)[NW], const uint32_t (&c)[NW], uint32_t p2m, int lane, int lane_last,
-                                        int jl, uint32_t (&nw)[NW])
+__device__ __forceinline__ void sw_step(const uint32_t (&w)[NW], const uint32_t (&c)[NW], uint32_t p2m, uint32_t p1x2, int lane,
+                                        int lane_last, int jl, uint32_t (&nw)[NW])
 {
     uint32_t ext[NW + 2];
 #pragma unroll
@@ -291,7 +285,7 @@ __device__ __forceinline__ void sw_step(const uint32_t (&w)[NW], const uint32_t 
 #pragma unroll
     for (int k = 0; k < NW; k++) {
         uint32_t t = __vimin3_u16x2(ext[k], ext[k + 2], p2m);       // min(L[d-1], L[d+1], P2 - P1)
-        t = __viaddmin_u16x2(t, SW_P1X2, w[k]);                     // min(. + P1, L[d])
+        t = __viaddmin_u16x2(t, p1x2, w[k]);                        // min(. + P1, L[d])
         nw[k] = t + c[k];
     }
 }
@@ -319,7 +313,7 @@ template <int NW, int MODE, int DIR, bool FULLK>
 __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__restrict__ img, const uint16_t *__restrict__ cost,
                                                             uint32_t *__restrict__ S, TL t, long total_rows,
                                                             float *__restrict__ disp_l, float *__restrict__ disp_r,
-                                                            const float *__restrict__ lut)
+                                                            const float *__restrict__ lut, SgmParams prm)
 {
     constexpr bool STORE = MODE == 0, WTA = MODE == 2;
     static_assert(!WTA || DIR < 0, "the fused WTA rides the backward sweep");
@@ -371,13 +365,14 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
     auto p2_block = [&](int t0) -> uint32_t {
         // (P2 - P1) * 0x10001 for step t0 + lane: |I(x) - I(x - dirn)| inside the row (step 0 has no predecessor)
         const int tt = t0 + lane;
-        int p2 = SW_P2MIN;
+        int p2 = prm.P2min;
         if (tt > 0 && tt < W) {
             const int xx = xs + DIR * tt;
-            p2 = sw_adapt_p2(irow[xx], irow[xx - DIR]);
+            p2 = adapt_p2(prm, irow[xx], irow[xx - DIR]);
         }
-        return (uint32_t)(p2 - SW_P1) * 0x10001u;
+        return (uint32_t)(p2 - prm.P1) * 0x10001u;
     };
+    const uint32_t p1x2 = (uint32_t)prm.P1 * 0x10001u;
     uint32_t p2v = p2_block(0), p2n = p2_block(32);
     uint32_t w[NW];
 #pragma unroll
@@ -428,7 +423,7 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
 #pragma unroll
                 for (int j = 0; j < NW; j++) nw[j] = cc[j];
             } else {
-                sw_step<NW, FULLK>(w, cc, p2m, lane, lane_last, jl, nw);
+                sw_step<NW, FULLK>(w, cc, p2m, p1x2, lane, lane_last, jl, nw);
             }
 #pragma unroll
             for (int j = 0; j < NW; j++) if (!wv[j]) nw[j] = SW_BIG2;
@@ -553,7 +548,7 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
 
 template <int NW, int MODE, int DIR>
 static int run_h_t(const uint8_t *img, const uint16_t *cost, uint32_t *S, const TL &t, int n, float *dl, float *dr,
-                   const float *lut, cudaStream_t st)
+                   const float *lut, const SgmParams &prm, cudaStream_t st)
 {
     const long rows = (long)n * t.H;
     const int blocks = cdiv(rows, HWARPS);
@@ -561,19 +556,19 @@ static int run_h_t(const uint8_t *img, const uint16_t *cost, uint32_t *S, const 
     const size_t smem = (size_t)HWARPS * 2 * stage + (MODE == 2 ? (size_t)HWARPS * 16 * 4 : 0);
     auto kern = t.K2 == NW * 32 ? sgm_h_kernel<NW, MODE, DIR, true> : sgm_h_kernel<NW, MODE, DIR, false>;
     if (smem > 48 * 1024) VPP_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<blocks, HWARPS * 32, smem, st>>>(img, cost, S, t, rows, dl, dr, lut);
+    kern<<<blocks, HWARPS * 32, smem, st>>>(img, cost, S, t, rows, dl, dr, lut, prm);
     VPP_LAUNCH_CHECK("sgm_h_kernel");
     return VPPB200_OK;
 }
 
 // mode 0: forward sweep, S = L;  mode 1: backward sweep, S += L;  mode 2: backward sweep fused with WTA (dl, dr, lut)
 static int run_h(const uint8_t *img, const uint16_t *cost, uint32_t *S, const TL &t, int mode, int n, float *dl, float *dr,
-                 const float *lut, cudaStream_t st)
+                 const float *lut, const SgmParams &prm, cudaStream_t st)
 {
 #define VPP_RUN_H(NW)                                                                                                  \
-    return mode == 0 ? run_h_t<NW, 0, 1>(img, cost, S, t, n, nullptr, nullptr, nullptr, st)                            \
-         : mode == 1 ? run_h_t<NW, 1, -1>(img, cost, S, t, n, nullptr, nullptr, nullptr, st)                           \
-                     : run_h_t<NW, 2, -1>(img, cost, S, t, n, dl, dr, lut, st)
+    return mode == 0 ? run_h_t<NW, 0, 1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, st)                       \
+         : mode == 1 ? run_h_t<NW, 1, -1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, st)                      \
+                     : run_h_t<NW, 2, -1>(img, cost, S, t, n, dl, dr, lut, prm, st)
     switch ((t.K2 + 31) / 32) {
         case 1: VPP_RUN_H(1);
         case 2: VPP_RUN_H(2);
@@ -592,6 +587,7 @@ struct VArgs {
     int pass;          // 0: top-down (di = dj = +1), 1: bottom-up (di = dj = -1)
     int csize;         // CTAs per team (one frame)
     int GC;            // 32-column groups per CTA, ceil(G / csize)
+    uint32_t p1x2;     // P1 * 0x10001
     // Row bands (a frame split over several GPUs, SURVEY.md 8e row 5): t.H is the band's row count, the volumes hold the band's
     // rows only.  pass_start = the band begins with the pass's first image row (L = C there); otherwise the sweep continues from
     // `state_in`, the path state of the row before the band as another band's sweep left it in `state_out`:
@@ -623,7 +619,8 @@ __device__ __forceinline__ uint32_t add3(uint32_t a, uint32_t b, uint32_t c)
 __device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 // ---- halo exchange between the CTAs of a team (the CTAs that share one frame): self-validating words in global
-// memory.  Handed-over state words are < 2^28 (two uint16 values <= 290 once taken relative to their line's minimum), so the
+// memory.  Handed-over state words are < 2^28 (two uint16 values <= Cmax + P2max <= 4095 once taken relative to their line's
+// part minimum: sweep_params_supported), so the
 // top four bits carry a tag that changes with the row; the consumer polls a word until its tag is the expected one.  No
 // fence, no barrier between CTAs: every word is its own flag (relaxed gpu-scope stores and loads go through L2).
 __device__ __forceinline__ void st_relaxed_gpu(uint32_t *p, uint32_t v)
@@ -655,9 +652,10 @@ static constexpr uint32_t HALO_INVALID = 0xF0000000u;
 //  * L is kept WITHOUT subtracting the predecessor's minimum per path (NORM = false): with Lt = L + (running sum of the minima)
 //    the recurrence is Lt = C + min(Lt[d], Lt[d+-1] + P1, min Lt + P2) and the reference's value is Lt - min_prev, so the three
 //    subtractions per disparity pair collapse into ONE constant per pixel folded into the S update:
-//    S += Lt1 + Lt2 + Lt3 - (m1 + m2 + m3).  Lt grows by at most max(C) per row: 24 * H + 74 < 65536 for Hamming costs
-//    (H <= 2700); guided costs (<= 240) take NORM = true.  Lines handed to a neighbour CTA travel normalised by their own
-//    part minimum (<= 74 / 290 per half word), which keeps the 4 tag bits of the self-validating words free.
+//    S += Lt1 + Lt2 + Lt3 - (m1 + m2 + m3).  The minimum grows by at most max(C) per row, so Lt <= 24 * H + P2max: the state
+//    stays un-normalised while 24 * H + P2max + 78 < 65536 for Hamming costs (H <= 2700 with the default P2max = 50);
+//    guided costs (<= 240) take NORM = true.  Lines handed to a neighbour CTA travel normalised by their own part minimum
+//    (<= Cmax + P2max per half word), which keeps the 4 tag bits of the self-validating words free.
 //  * P2 of the three paths comes from a per-pixel table (sgm_p2_kernel: one word instead of four image loads and three
 //    float evaluations per warp and row, and the flat-stream wrap rules live in one place).
 //  * a timed-out halo wait raises a flag in global memory (checked by the host) and lets the grid run to completion with
@@ -671,7 +669,7 @@ static constexpr uint32_t HALO_INVALID = 0xF0000000u;
 // Row bands: the table covers rows [row0, row0 + Hb) of frames of H rows (img_all = the full guide images).
 // One thread = 4 adjacent pixels of a row (one 16-byte store); grid.y = frame * Hb + band row.
 __global__ void __launch_bounds__(256) sgm_p2_kernel(const uint8_t *__restrict__ img_all, uint32_t *__restrict__ p2q, int W, int H,
-                                                     int G32, int pass, int row0, int Hb)
+                                                     int G32, int pass, int row0, int Hb, SgmParams prm)
 {
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (x0 >= G32) return;
@@ -695,8 +693,8 @@ __global__ void __launch_bounds__(256) sgm_p2_kernel(const uint8_t *__restrict__
             q1 = q1 < 0 ? 0 : (q1 >= npx ? npx - 1 : q1);
             q3 = q3 < 0 ? 0 : (q3 >= npx ? npx - 1 : q3);
             const int ipc = rc[xr], ip1 = img[q1], ip2 = rl[xr], ip3 = img[q3];
-            o[u] = (uint32_t)(sw_adapt_p2(ipc, ip1) - SW_P1) | ((uint32_t)(sw_adapt_p2(ipc, ip2) - SW_P1) << 8) |
-                   ((uint32_t)(sw_adapt_p2(ipc, ip3) - SW_P1) << 16);
+            o[u] = (uint32_t)(adapt_p2(prm, ipc, ip1) - prm.P1) | ((uint32_t)(adapt_p2(prm, ipc, ip2) - prm.P1) << 8) |
+                   ((uint32_t)(adapt_p2(prm, ipc, ip3) - prm.P1) << 16);
         }
         out = make_uint4(o[0], o[1], o[2], o[3]);
     }
@@ -749,13 +747,13 @@ __device__ __forceinline__ void red_add_u32(uint32_t *p, uint32_t v)
 // One block of up to VU words for the three paths.  s* = predecessor state rows of the block (stride NS), w* = this row's state
 // rows (same slots), Sg = the block's S words (stride 32).  GUARD: only the first `cnt` words exist; `last`: the block ends this
 // warp's share, whose upper neighbour word was read before the column group's barrier (wr*).
-// RED: S += goes out as a fire-and-forget reduction to L2 (the addend's halves are <= 3 * 74 resp. 3 * 305 and S's halves never
+// RED: S += goes out as a fire-and-forget reduction to L2 (the addend's halves are <= 3 * (Cmax + P2max) and S's halves never
 // overflow, so the 32-bit add is exact for both halves): no load of S, no operand registers, no latency to hide
 template <int NS, bool GUARD, bool NORM, bool RED>
 __device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_t (&sb)[VU], const uint32_t *s1,
                                          const uint32_t *s2, const uint32_t *s3, uint32_t *w1, uint32_t *w2, uint32_t *w3,
                                          uint32_t wr1, uint32_t wr2, uint32_t wr3, VPath2 &p1, VPath2 &p2, VPath2 &p3,
-                                         uint32_t negm, uint32_t *Sg, int cnt, bool last)
+                                         uint32_t negm, uint32_t p1x2, uint32_t *Sg, int cnt, bool last)
 {
     uint32_t nx1[VU], nx2[VU], nx3[VU];
     uint32_t tp1 = 0, tp2 = 0, tp3 = 0;
@@ -776,15 +774,15 @@ __device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_
             // split-half packing: the neighbours d-1 / d+1 of both halves are the words k-1 / k+1 as they stand
             uint32_t t1 = __vimin3_u16x2(p1.prev, nx1[u], p1.q), t2 = __vimin3_u16x2(p2.prev, nx2[u], p2.q),
                      t3 = __vimin3_u16x2(p3.prev, nx3[u], p3.q);                     // min(Lt[d-1], Lt[d+1], min + P2 - P1)
-            t1 = __viaddmin_u16x2(t1, SW_P1X2, p1.cur);                              // min(. + P1, Lt[d])
-            t2 = __viaddmin_u16x2(t2, SW_P1X2, p2.cur);
-            t3 = __viaddmin_u16x2(t3, SW_P1X2, p3.cur);
+            t1 = __viaddmin_u16x2(t1, p1x2, p1.cur);                                 // min(. + P1, Lt[d])
+            t2 = __viaddmin_u16x2(t2, p1x2, p2.cur);
+            t3 = __viaddmin_u16x2(t3, p1x2, p3.cur);
             uint32_t sum;
             if (NORM) {
                 t1 = (t1 + c) + p1.ng * 0xFFFEFFFFu; t2 = (t2 + c) + p2.ng * 0xFFFEFFFFu; t3 = (t3 + c) + p3.ng * 0xFFFEFFFFu;
                 sum = (t1 + t2) + t3;
             } else {
-                // packed halves may carry into each other inside the sum; the final halves (<= 3 * 74) are exact mod 2^32
+                // packed halves may carry into each other inside the sum; the final halves (<= 3 * (Cmax + P2max)) are exact mod 2^32
                 t1 += c; t2 += c; t3 += c;
                 sum = add3(t1, t2, t3) + negm;
             }
@@ -810,9 +808,11 @@ __device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_
 // leaves a quarter of the register file and ~30 KB of shared memory per SM to the front / tail kernels of the neighbouring
 // batches, which run beside the sweep (measured: the sweep alone 6.09 -> 6.39 ms, the pipelined step 23.7 -> 23.3 ms)
 // BAND: the launch covers a row band of taller frames (state import / export at the band's ends); whole-frame launches are
-// compiled without that code (it costs the hot loop 0.3 ms per launch under the register cap).
+// compiled without that code (it costs the hot loop 0.3 ms per launch under the register cap).  Band launches take the 128 cap
+// (a band's sweep does not share the SMs with the phases of neighbouring batches; under 96 registers the runtime P1 made the
+// band kernels spill).  The residency plan (v_resident_ctas) is computed for 128 registers either way.
 template <int NS, bool FULL, bool NORM, bool RED, bool BAND>
-__global__ void __maxnreg__(RED ? VPP_VREGS : 128) sgm_v2_kernel(const uint32_t *__restrict__ p2q_all,
+__global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const uint32_t *__restrict__ p2q_all,
                                                                                  const uint16_t *__restrict__ cost_all,
                                                                                  uint32_t *__restrict__ S_all, uint32_t *halo,
                                                                                  uint32_t *abort_flag, VArgs a)
@@ -823,6 +823,7 @@ __global__ void __maxnreg__(RED ? VPP_VREGS : 128) sgm_v2_kernel(const uint32_t 
     const int cid = blockIdx.x / a.csize, nteams = gridDim.x / a.csize;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int W = a.t.W, H = a.t.H, K2 = a.t.K2, G = a.t.G;
+    const uint32_t p1x2 = a.p1x2;
     constexpr int BIGS = NS - 1;
     const int part = warp % VPARTS;
     const int g_first = rank * a.GC;
@@ -1056,14 +1057,14 @@ __global__ void __maxnreg__(RED ? VPP_VREGS : 128) sgm_v2_kernel(const uint32_t 
                     uint32_t cn[VU], sn[VU];
                     const bool last1 = kb + VU >= k1;
                     if (!last1) load_block(cp + VU * 32, sp + VU * 32, k1 - kb - VU, cn, sn, true);
-                    v2_block<NS, !FULL, NORM, RED>(cb, sb, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, sp, k1 - kb, last1);
+                    v2_block<NS, !FULL, NORM, RED>(cb, sb, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, p1x2, sp, k1 - kb, last1);
                     VTRACE(trb); trb++;
                     cp += VU * 32; sp += VU * 32;
                     s1 += VU * NS; s2 += VU * NS; s3 += VU * NS; w1 += VU * NS; w2 += VU * NS; w3 += VU * NS;
                     if (last1) break;
                     const bool last2 = kb + 2 * VU >= k1;
                     if (!last2) load_block(cp + VU * 32, sp + VU * 32, k1 - kb - 2 * VU, cb, sb, true);
-                    v2_block<NS, !FULL, NORM, RED>(cn, sn, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, sp, k1 - kb - VU, last2);
+                    v2_block<NS, !FULL, NORM, RED>(cn, sn, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, p1x2, sp, k1 - kb - VU, last2);
                     VTRACE(trb); trb++;
                     cp += VU * 32; sp += VU * 32;
                     s1 += VU * NS; s2 += VU * NS; s3 += VU * NS; w1 += VU * NS; w2 += VU * NS; w3 += VU * NS;
@@ -1304,11 +1305,12 @@ struct VBand { int Hfull, row0, pass_start; const uint32_t *state_in; uint32_t *
 
 template <int GC>
 static int run_v_t(const uint32_t *p2q, const uint16_t *cost, uint32_t *S, uint32_t *halo, uint32_t *abort_flag, const TL &t, int pass,
-                   int n, const VPlan &p, bool norm, const VBand &band, cudaStream_t st)
+                   int n, const VPlan &p, bool norm, const VBand &band, const SgmParams &prm, cudaStream_t st)
 {
     constexpr int NS = GC * 32 + 1;
     VArgs a;
     a.t = t; a.n = n; a.pass = pass; a.csize = p.csize; a.GC = p.GC;
+    a.p1x2 = (uint32_t)prm.P1 * 0x10001u;
     a.pass_start = band.pass_start; a.state_in = band.state_in; a.state_out = band.state_out;
     a.state_words = sweep_state_words(t.W, t.D);
     // FULL: K2 splits into VPARTS equal shares of whole VU-blocks
@@ -1332,7 +1334,7 @@ static int run_v_t(const uint32_t *p2q, const uint16_t *cost, uint32_t *S, uint3
 
 // norm: per-path normalisation (costs above the Hamming range, or frames too tall for the un-normalised state)
 static int run_v(const uint8_t *img, const uint16_t *cost, uint32_t *S, void *halo_ws, const TL &t, int pass, int n,
-                 const VPlan &p, bool norm, cudaStream_t st, const VBand *bandp = nullptr)
+                 const VPlan &p, bool norm, const SgmParams &prm, cudaStream_t st, const VBand *bandp = nullptr)
 {
     const VBand band = bandp ? *bandp : VBand{t.H, 0, 1, nullptr, nullptr};
     uint32_t *halo = static_cast<uint32_t *>(halo_ws);
@@ -1346,15 +1348,15 @@ static int run_v(const uint8_t *img, const uint16_t *cost, uint32_t *S, void *ha
     for (int f0 = 0; f0 < n; f0 += fpl) {
         const int nf = std::min(fpl, n - f0);
         sgm_p2_kernel<<<dim3((unsigned)cdiv(G32 / 4, 256), (unsigned)(nf * t.H)), 256, 0, st>>>(
-            img + (long)f0 * t.W * band.Hfull, p2q + (long)f0 * t.H * G32, t.W, band.Hfull, G32, pass, band.row0, t.H);
+            img + (long)f0 * t.W * band.Hfull, p2q + (long)f0 * t.H * G32, t.W, band.Hfull, G32, pass, band.row0, t.H, prm);
         VPP_LAUNCH_CHECK("sgm_p2_kernel");
     }
     switch (p.GC) {
-        case 1: return run_v_t<1>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, st);
-        case 2: return run_v_t<2>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, st);
-        case 3: return run_v_t<3>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, st);
-        case 4: return run_v_t<4>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, st);
-        default: return run_v_t<5>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, st);
+        case 1: return run_v_t<1>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, prm, st);
+        case 2: return run_v_t<2>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, prm, st);
+        case 3: return run_v_t<3>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, prm, st);
+        case 4: return run_v_t<4>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, prm, st);
+        default: return run_v_t<5>(p2q, cost, S, halo, abort_flag, t, pass, n, p, norm, band, prm, st);
     }
 }
 
@@ -1380,6 +1382,23 @@ bool aggregate_tile_supported(int W, int H, int D, int n)
     return plan_v(t, n, &plan) == VPPB200_OK;
 }
 
+// The parameter domain of the sweeps (file header): with these the packed u16 arithmetic of the sweeps and of the fast per-path
+// kernels never saturates, the P2 table's bytes hold P2 - P1, and the hand-off words keep their tag bits.  Outside it,
+// compute_rsgm aggregates with the saturating generic kernels of sgm.cu.  Expects 0 <= P1, P2min, gamma <= 65535, alpha >= 0.
+bool sweep_params_supported(const SgmParams &p, bool plain_costs)
+{
+    const int cmax = plain_costs ? 24 : 240;
+    const int p2max = std::max(p.P2min, p.gamma);
+    return p.P1 <= p.P2min && p2max - p.P1 <= 255 && cmax + p2max <= 4095;
+}
+
+// un-normalised v-sweep state (Hamming costs only): the running Lt <= 24 * H + P2max must stay inside uint16 (with slack; the
+// default parameters give the 24 * H + 128 bound)
+static bool v_norm(bool plain_costs, int H, const SgmParams &p)
+{
+    return !plain_costs || 24L * H + std::max(p.P2min, p.gamma) + 78 > 65535;
+}
+
 // 0 = done; 1 = this shape does not fit the sweep (caller uses sgm.cu); < 0 = error.
 // dl != NULL: the last sweep is fused with the winner-takes-all step (left + sub-pixel into dl, right into dr) and the
 // final S is never written; dl == NULL: S holds the aggregated volume in layout T.
@@ -1393,31 +1412,32 @@ bool aggregate_tile_supported(int W, int H, int D, int n)
 // only bring it from 3.59 to 3.06 ms and the v-sweep with an operand load instead of the fire-and-forget reduction goes from 5.93 to
 // 6.78 ms: step 22.3 vs 22.0 ms.)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S16, void *halo_ws, int W, int H, int D, int n,
-                          float *dl, float *dr, const float *lut, bool plain_costs, const StageHook *hook, cudaStream_t st)
+                          float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &prm, const StageHook *hook,
+                          cudaStream_t st)
 {
+    if (!sweep_params_supported(prm, plain_costs)) return VPPB200_ERR_ARG;
     const TL t = make_tl(W, H, D);
     VSplit sp;
     int rc = plan_v_split(t, n, &sp);
     if (rc) return rc;
     const uint16_t *cost = reinterpret_cast<const uint16_t *>(cost8);
     uint32_t *S = reinterpret_cast<uint32_t *>(S16);
-    // un-normalised path state: Hamming costs only, and 24 per row must stay inside uint16
-    const bool norm = !plain_costs || 24L * H + 128 > 65535;
+    const bool norm = v_norm(plain_costs, H, prm);
     auto done = [&](int stage) { if (hook) hook->fn(hook->ctx, stage); };
     auto sweep = [&](int pass) -> int {
-        int r = run_v(img, cost, S, halo_ws, t, pass, sp.n1, sp.p1, norm, st);
+        int r = run_v(img, cost, S, halo_ws, t, pass, sp.n1, sp.p1, norm, prm, st);
         if (r == VPPB200_OK && sp.n2 > 0)
             r = run_v(img + (long)sp.n1 * t.W * t.H, cost + (long)sp.n1 * t.frame, S + (long)sp.n1 * t.frame, halo_ws, t, pass, sp.n2,
-                      sp.p2, norm, st);
+                      sp.p2, norm, prm, st);
         return r;
     };
-    if ((rc = run_h(img, cost, S, t, 0, n, nullptr, nullptr, nullptr, st))) return rc;
+    if ((rc = run_h(img, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, st))) return rc;
     done(VPPB200_STAGE_SGM_H_FWD);
     if ((rc = sweep(0))) return rc;
     done(VPPB200_STAGE_SGM_V_DOWN);
     if ((rc = sweep(1))) return rc;
     done(VPPB200_STAGE_SGM_V_UP);
-    if ((rc = run_h(img, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, st))) return rc;
+    if ((rc = run_h(img, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, st))) return rc;
     done(VPPB200_STAGE_SGM_H_BWD);
     return VPPB200_OK;
 }
@@ -1430,35 +1450,37 @@ int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S1
 // band below); state_out == NULL: nothing is exported.  cost8 / S16 / dl / dr hold the band's rows only.
 int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full, const uint32_t *cen_r_full, uint8_t *cost8, uint16_t *S16,
                           void *halo_ws, int W, int Hfull, int D, int row0, int rows, int n, int phases, const uint32_t *state_in,
-                          uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, cudaStream_t st)
+                          uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &prm,
+                          cudaStream_t st)
 {
     const TL t = make_tl(W, rows, D);
     if (row0 < 0 || rows < 3 || row0 + rows > Hfull) return VPPB200_ERR_ARG;
+    if (!sweep_params_supported(prm, plain_costs)) return VPPB200_ERR_ARG;
     VPlan plan;
     int rc = plan_v(t, n, &plan);
     if (rc) return rc < 0 ? rc : VPPB200_ERR_ARG;
     const uint16_t *cost = reinterpret_cast<const uint16_t *>(cost8);
     uint32_t *S = reinterpret_cast<uint32_t *>(S16);
     const uint8_t *guide_band = guide_full + (long)row0 * W;       // the h-sweeps read the band's own rows of the guide (per frame: + f * W * Hfull)
-    const bool norm = !plain_costs || 24L * Hfull + 128 > 65535;
+    const bool norm = v_norm(plain_costs, Hfull, prm);
     if (n != 1 && Hfull != rows) {
         // frames are Hfull * W apart in the guide but rows * W apart in an h-sweep's row numbering: one frame per call when banded
         return VPPB200_ERR_ARG;
     }
     if (phases & 1) if ((rc = launch_cost_tile_band(cen_l_full, cen_r_full, cost8, W, Hfull, D, row0, rows, n, st))) return rc;
-    if (phases & 2) if ((rc = run_h(guide_band, cost, S, t, 0, n, nullptr, nullptr, nullptr, st))) return rc;
+    if (phases & 2) if ((rc = run_h(guide_band, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, st))) return rc;
     if (phases & 4) {
         const VBand b{Hfull, row0, row0 == 0 ? 1 : 0, row0 == 0 ? nullptr : state_in, state_out};
         if (!b.pass_start && !state_in) return VPPB200_ERR_ARG;
-        if ((rc = run_v(guide_full, cost, S, halo_ws, t, 0, n, plan, norm, st, &b))) return rc;
+        if ((rc = run_v(guide_full, cost, S, halo_ws, t, 0, n, plan, norm, prm, st, &b))) return rc;
     }
     if (phases & 8) {
         const bool last = row0 + rows == Hfull;
         const VBand b{Hfull, row0, last ? 1 : 0, last ? nullptr : state_in, state_out};
         if (!b.pass_start && !state_in) return VPPB200_ERR_ARG;
-        if ((rc = run_v(guide_full, cost, S, halo_ws, t, 1, n, plan, norm, st, &b))) return rc;
+        if ((rc = run_v(guide_full, cost, S, halo_ws, t, 1, n, plan, norm, prm, st, &b))) return rc;
     }
-    if (phases & 16) if ((rc = run_h(guide_band, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, st))) return rc;
+    if (phases & 16) if ((rc = run_h(guide_band, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, st))) return rc;
     return VPPB200_OK;
 }
 

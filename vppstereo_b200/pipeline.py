@@ -22,7 +22,9 @@ from . import vpp_core_opt as _core
 
 class VppRsgmPipeline:
     def __init__(self, H, W, channels=3, batch=64, dmax=192, wsize=3, blending=0.4, c_occ=0.0, left2right=True,
-                 interpolate=True, subpixel=True, device=None, seed=1234):
+                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None):
+        # sgm_params: (p1, p2min, alpha, gamma) honoured by the matcher; None = the reference's effective values (7, 17, 0.25, 50)
+        self.sgm_params = None if sgm_params is None else _lib.sgm_params(*sgm_params)
         torch = _lib.require_cuda()
         self.torch = torch
         self.H, self.W, self.C, self.N, self.D = int(H), int(W), int(channels), int(batch), int(dmax)
@@ -145,9 +147,10 @@ class VppRsgmPipeline:
 
     def _phase(self, phases, b, left, lv, rv, out, N, stream):
         L = self.lib
-        rc = L.vppb200_compute_rsgm_phases(_lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), None, None, _lib.ptr(out), self.H, self.W,
-                                           self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm),
-                                           C.c_size_t(self.ws_rsgm.numel()), N, C.c_void_p(stream.cuda_stream), phases, 2, b)
+        prm = None if self.sgm_params is None else C.byref(self.sgm_params)
+        rc = L.vppb200_compute_rsgm_ex(_lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), None, None, _lib.ptr(out), self.H, self.W,
+                                       self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm),
+                                       C.c_size_t(self.ws_rsgm.numel()), N, C.c_void_p(stream.cuda_stream), phases, 2, b, None, prm)
         _lib.check(rc, "compute_rsgm_phases")
 
     def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None):
