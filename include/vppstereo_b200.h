@@ -91,14 +91,15 @@ int vppb200_stage_times(float *ms_out, int *calls_out);
 #define VPPB200_TUNE_SGM_MAX_STRIP 0
 #define VPPB200_TUNE_SGM_SWEEP 1
 #define VPPB200_TUNE_VPP_ROWS 3       /* 0 = VPP rnd by the ordered per-row replay only, 1 = per-pixel replay where possible (default) */
-#define VPPB200_TUNE_SGM_CLUSTERS 2   /* upper bound on frames in flight in the v-sweep (0 = all SMs); experiments only */
+#define VPPB200_TUNE_SGM_CLUSTERS 2   /* upper bound on frames in flight in the v-sweep (0 = all SMs); test hook: forces multi-round teams on small batches */
 #define VPPB200_TUNE_VPP_MD_WAVE 5    /* 0 = VPP maxDistance by the serial one-warp-per-(frame, channel) kernel, 1 = row wavefront (default) */
-#define VPPB200_TUNE_SGM_FUSE_COST 6  /* round-1 option (forward h-sweep producing the cost volume), measured slower and removed: accepted, no effect */
 #define VPPB200_TUNE_RCP_HOST 7       /* 0 = sub-pixel reciprocal from the fixed Intel RCPSS table (default), 1 = from the host CPU's RCPSS instruction */
-#define VPPB200_TUNE_SGM_V_RED 8      /* 1 = the v-sweeps add into S with red.global.add (no load of S; default), 0 = load + add + store */
-#define VPPB200_TUNE_CENSUS_FUSED 10  /* 1 = compute_rsgm's pad + gray + census run as one kernel per image (default), 0 = pad_gray then census */
-#define VPPB200_TUNE_SGM_V_SPLIT 9    /* 1 = a batch whose last round would leave teams idle is swept in two launches with different strip widths (default) */
-#define VPPB200_TUNE_SGM_BYTE_SUMS 4  /* round-1 option (uint8 partial-sum volumes), measured slower and removed: accepted, no effect */
+/* Retired keys: accepted, no effect.  Each selected an alternative to the default path that is no longer built. */
+#define VPPB200_TUNE_SGM_BYTE_SUMS 4  /* uint8 partial-sum volumes (measured slower) */
+#define VPPB200_TUNE_SGM_FUSE_COST 6  /* a forward h-sweep producing the cost volume (measured slower) */
+#define VPPB200_TUNE_SGM_V_RED 8      /* 0 = the v-sweeps update S by load + add + store (measured slower than red.global.add) */
+#define VPPB200_TUNE_SGM_V_SPLIT 9    /* 0 = one strip width per batch (the planner already keeps one where splitting does not pay) */
+#define VPPB200_TUNE_CENSUS_FUSED 10  /* 0 = pad_gray then census (still run wherever the fused kernel does not apply) */
 int vppb200_set_tuning(int key, int value);
 
 /* ---- pyrSGM operators ----------------------------------------------------------------------------------- */

@@ -179,9 +179,6 @@ def tuning(mods):
     yield lambda key, value: _lib.set_tuning(key, value)
     _lib.set_tuning(_lib.TUNE_SGM_MAX_STRIP, 0)
     _lib.set_tuning(_lib.TUNE_SGM_SWEEP, 1)
-    _lib.set_tuning(_lib.TUNE_SGM_V_RED, 1)
-    _lib.set_tuning(_lib.TUNE_SGM_V_SPLIT, 1)
-    _lib.set_tuning(_lib.TUNE_CENSUS_FUSED, 1)
 
 
 @pytest.mark.parametrize("strip", [32, 64, 100])
@@ -198,13 +195,9 @@ def test_sweep_cluster_strips(mods, orc, tuning, strip, shape, D, channels):
     for f, p in enumerate(frames):
         want = orc.compute_rsgm(p["left"], p["left"], p["right"], dmax=D)
         assert_same(st["out"][f], want, f"sweep strip={strip} {shape} D={D} frame {f}")
-    # the production path (last sweep fused with WTA, the final S never written), with both forms of the S update
+    # the production path (last sweep fused with WTA, the final S never written)
     fused16 = rsgm.compute_rsgm(left, left, right, dmax=D)
     assert_same(fused16, st["out"], f"fused sweep, strip={strip}")
-    tuning(_lib.TUNE_SGM_V_RED, 0)
-    fused_ls = rsgm.compute_rsgm(left, left, right, dmax=D)
-    assert_same(fused_ls, st["out"], f"fused sweep with load + add + store instead of red.add, strip={strip}")
-    tuning(_lib.TUNE_SGM_V_RED, 1)
     # the aggregated volume itself, against the stand-alone operator (generic per-path kernel) on the same inputs
     tuning(_lib.TUNE_SGM_SWEEP, 0)
     st0 = rsgm.compute_rsgm_stages(left, left, right, dmax=D)
@@ -212,37 +205,63 @@ def test_sweep_cluster_strips(mods, orc, tuning, strip, shape, D, channels):
     assert_same(st["out"], st0["out"], "sweep vs per-path kernels, final disparity")
 
 
+def _kernels(fn):
+    """names of the kernels fn() launches, one entry per launch"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return [e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA]
+
+
 @pytest.mark.parametrize("shape,channels", [((37, 70), 3), ((5, 17), 1), ((64, 333), 3), ((23, 1242), 3), ((130, 64), 1)])
-def test_census_fused_front(mods, orc, tuning, shape, channels):
+def test_census_fused_front(mods, orc, shape, channels):
     """pad + gray + census as one kernel per image (bulk-copied source window, gray band in shared memory) against the two-kernel
-    front and the oracle; frames 1.. of a batch start at addresses that are not 16-byte aligned"""
-    rsgm, synth, _lib = mods[1], mods[2], mods[3]
+    front and the oracle; frames 1.. of a batch start at addresses that are not 16-byte aligned.  The two-kernel front is what
+    runs when the batch itself does not start on a 16-byte boundary: the same batch from such a source is the reference."""
+    import torch
+    rsgm, synth = mods[1], mods[2]
     D = 32 if shape[1] >= 64 else 8
     frames = [synth.make_pair(900 + f, shape=shape, hints="random", channels=channels) for f in range(3)]
     left = np.stack([p["left"] for p in frames]); right = np.stack([p["right"] for p in frames])
+
+    def misaligned(a):                              # the same bytes on the device, starting one byte past an aligned address
+        buf = torch.empty(a.size + 1, dtype=torch.uint8, device="cuda")
+        buf[1:].copy_(torch.from_numpy(a).reshape(-1))
+        view = buf[1:].view(a.shape)
+        assert view.data_ptr() % 16 == 1
+        return view
+    left_m, right_m = misaligned(left), misaligned(right)
     got = rsgm.compute_rsgm(left, left, right, dmax=D)
-    tuning(_lib.TUNE_CENSUS_FUSED, 0)
-    two = rsgm.compute_rsgm(left, left, right, dmax=D)
-    tuning(_lib.TUNE_CENSUS_FUSED, 1)
+    two = rsgm.compute_rsgm(left_m, left_m, right_m, dmax=D).cpu().numpy()
     assert_same(got, two, f"fused front vs pad_gray + census {shape} C={channels}")
+    names = _kernels(lambda: rsgm.compute_rsgm(left, left, right, dmax=D))
+    assert any("census_fused_kernel" in n for n in names) and not any("census5x5_kernel" in n for n in names), sorted(names)
+    names = _kernels(lambda: rsgm.compute_rsgm(left_m, left_m, right_m, dmax=D))
+    assert any("census5x5_kernel" in n for n in names) and not any("census_fused_kernel" in n for n in names), sorted(names)
     for f in (0, 2):
         want = orc.compute_rsgm(frames[f]["left"], frames[f]["left"], frames[f]["right"], dmax=D)
         assert_same(got[f], want, f"fused front {shape} C={channels} frame {f}")
 
 
-def test_sweep_split_launches(mods, orc, tuning):
+def test_sweep_split_launches(mods, orc):
     """a batch that does not fill its last round of teams is swept in two launches with different strip widths (plan_v_split):
-    same result as the single-plan sweep, and as the oracle on the frames either side of the split"""
-    rsgm, synth, _lib = mods[1], mods[2], mods[3]
-    shape, D, n = (24, 200), 16, 90
+    same result as the same frames swept one per call (a single frame never splits), and as the oracle on the frames either
+    side of the split.  On 148 SMs these 80 frames go as 37 frames on 2-group strips + 43 frames on 3-group strips."""
+    rsgm, synth = mods[1], mods[2]
+    shape, D, n = (24, 200), 16, 80
     frames = [synth.make_pair(500 + f, shape=shape, hints="random", channels=1) for f in range(n)]
     left = np.stack([p["left"] for p in frames]); right = np.stack([p["right"] for p in frames])
     got = rsgm.compute_rsgm(left, left, right, dmax=D)
-    tuning(_lib.TUNE_SGM_V_SPLIT, 0)
-    single = rsgm.compute_rsgm(left, left, right, dmax=D)
-    tuning(_lib.TUNE_SGM_V_SPLIT, 1)
-    assert_same(got, single, "split sweep vs single-plan sweep")
-    for f in (0, 73, 74, 89):
+    single = np.stack([rsgm.compute_rsgm(left[f], left[f], right[f], dmax=D) for f in range(n)])
+    assert_same(got, single, "split sweep vs one frame per call")
+    # two v-sweeps per plan: four launches when the batch splits, two for one frame
+    count = lambda fn: sum(1 for e in _kernels(fn) if "sgm_v2_kernel" in e)
+    assert count(lambda: rsgm.compute_rsgm(left, left, right, dmax=D)) == 4
+    assert count(lambda: rsgm.compute_rsgm(left[0], left[0], right[0], dmax=D)) == 2
+    for f in (0, 36, 37, 79):
         want = orc.compute_rsgm(frames[f]["left"], frames[f]["left"], frames[f]["right"], dmax=D)
         assert_same(got[f], want, f"split sweep frame {f}")
 

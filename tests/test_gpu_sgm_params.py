@@ -199,7 +199,6 @@ def tuning(mods):
     yield lambda key, value: _lib.set_tuning(key, value)
     _lib.set_tuning(_lib.TUNE_SGM_MAX_STRIP, 0)
     _lib.set_tuning(_lib.TUNE_SGM_SWEEP, 1)
-    _lib.set_tuning(_lib.TUNE_SGM_V_RED, 1)
 
 
 def _honoured(prm):
@@ -283,12 +282,12 @@ def test_sweeps_run_for_in_domain_params(mods):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("strip,red", [(32, 1), (64, 0), (64, 1), (0, 0)])
-def test_strips_red_and_guided(mods, orc, tuning, strip, red):
-    """forced narrow strips (halo hand-off between CTAs), both forms of the S update, and guided costs (normalised state)"""
+@pytest.mark.parametrize("strip", [32, 64, 96, 0])
+def test_strips_and_guided(mods, orc, tuning, strip):
+    """forced narrow strips (halo hand-off between CTAs; at 96 columns the team's last CTA holds a single column group) and
+    guided costs (normalised state)"""
     rsgm, synth, _lib = mods
     tuning(_lib.TUNE_SGM_MAX_STRIP, strip)
-    tuning(_lib.TUNE_SGM_V_RED, red)
     prm = (3, 30, 0.3, 80)
     frames = [synth.make_pair(300 + f, shape=(30, 200), hints="random") for f in range(2)]
     left = np.stack([q["left"] for q in frames]); right = np.stack([q["right"] for q in frames])
@@ -297,9 +296,9 @@ def test_strips_red_and_guided(mods, orc, tuning, strip, red):
     got_g = rsgm.compute_rsgm(left, left, right, hints=hints, validhints=valid, dmax=64, **_honoured(prm))
     for f, q in enumerate(frames):
         want = oracle_rsgm(orc, q["left"], q["left"], q["right"], dmax=64, params=prm)
-        assert_same(got[f], want, f"strip={strip} red={red} frame {f}")
+        assert_same(got[f], want, f"strip={strip} frame {f}")
         want = oracle_rsgm(orc, q["left"], q["left"], q["right"], hints=q["hints"], validhints=valid[f], dmax=64, params=prm)
-        assert_same(got_g[f], want, f"guided strip={strip} red={red} frame {f}")
+        assert_same(got_g[f], want, f"guided strip={strip} frame {f}")
 
 
 @pytest.mark.gpu

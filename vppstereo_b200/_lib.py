@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.path.join(HERE, "libvppstereo_b200%s.so" % os.environ.get("VPPB200_LIB_SUFFIX", ""))
+LIB_PATH = os.path.join(HERE, "libvppstereo_b200.so")
 
 OK = 0
 ERR_WIDTH, ERR_DISP, ERR_THREADS, ERR_UNIQUENESS, ERR_METHOD, ERR_WORKSPACE, ERR_ARG, ERR_CUDA = -1, -2, -3, -4, -5, -6, -7, -100

@@ -12,9 +12,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-# experiments: VPPB200_BUILD_DEFINES="-DVPP_VPARTS=4" VPPB200_LIB_SUFFIX=_vp4 builds a second library beside the default one
-SUFFIX = os.environ.get("VPPB200_LIB_SUFFIX", "")
-LIB = os.path.join(HERE, f"libvppstereo_b200{SUFFIX}.so")
+LIB = os.path.join(HERE, "libvppstereo_b200.so")
 SOURCES = ["capi.cu", "rsgm_ops.cu", "sgm.cu", "sgm_sweep.cu", "vpp.cu", "filter.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(HERE, "..", "include", "vppstereo_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
@@ -31,8 +29,7 @@ def _stale(target, deps):
 
 def build(force=False, verbose=False):
     objs = []
-    bdir = os.path.join(HERE, "build" + SUFFIX)
-    extra = os.environ.get("VPPB200_BUILD_DEFINES", "").split()
+    bdir = os.path.join(HERE, "build")
     os.makedirs(bdir, exist_ok=True)
     procs = []
     for s in SOURCES:
@@ -40,7 +37,7 @@ def build(force=False, verbose=False):
         obj = os.path.join(bdir, s.replace(".cu", ".o"))
         objs.append(obj)
         if force or _stale(obj, [src] + HEADERS):
-            cmd = [NVCC] + FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+            cmd = [NVCC] + FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
             procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
     for cmd, p in procs:
         out, _ = p.communicate()

@@ -314,11 +314,11 @@ extern "C" int vppb200_set_tuning(int key, int value)
         case VPPB200_TUNE_SGM_CLUSTERS: sweep_set_clusters(value); return VPPB200_OK;
         case VPPB200_TUNE_VPP_ROWS: vpp_set_rows_kernel(value); return VPPB200_OK;
         case VPPB200_TUNE_VPP_MD_WAVE: vpp_set_md_wave(value); return VPPB200_OK;
-        case VPPB200_TUNE_SGM_BYTE_SUMS: return VPPB200_OK;      // options of round 1, removed (measured slower): accepted, no effect
-        case VPPB200_TUNE_SGM_FUSE_COST: return VPPB200_OK;
-        case VPPB200_TUNE_SGM_V_RED: sweep_set_v_red(value); return VPPB200_OK;
-        case VPPB200_TUNE_SGM_V_SPLIT: sweep_set_v_split(value); return VPPB200_OK;
-        case VPPB200_TUNE_CENSUS_FUSED: census_set_fused(value); return VPPB200_OK;
+        case VPPB200_TUNE_SGM_BYTE_SUMS:                         // retired options (the header says why): accepted, no effect
+        case VPPB200_TUNE_SGM_FUSE_COST:
+        case VPPB200_TUNE_SGM_V_RED:
+        case VPPB200_TUNE_SGM_V_SPLIT:
+        case VPPB200_TUNE_CENSUS_FUSED: return VPPB200_OK;
         case VPPB200_TUNE_RCP_HOST: g_rcp_host.store(value != 0); return VPPB200_OK;
         default: return VPPB200_ERR_ARG;
     }
@@ -496,14 +496,14 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
                 if ((rc = launch_s_tile_to_xyd(w.S, w.S_xyd, d.Wp, d.Hp, D, n, st))) return rc;
                 S_final = w.S_xyd;
-                if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, 0, n, st))) return rc;
+                if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, st))) return rc;
             }
         } else {
             if (fast_params) rc = launch_aggregate_fast(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
             else rc = launch_aggregate_generic_u8(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
             if (rc) return rc;
             tm.done(VPPB200_STAGE_SGM_H_BWD);                // the per-path fallback is booked on the last sweep's slot
-            if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, 0, n, st))) return rc;
+            if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, st))) return rc;
         }
         tm.done(VPPB200_STAGE_WTA);
     }

@@ -62,7 +62,6 @@ __device__ __forceinline__ int adapt_p2(const SgmParams &p, int ip, int ipr)
 int launch_pad_gray(const uint8_t *src, uint8_t *gray, const RsgmDims &d, int n, cudaStream_t st);
 int launch_pad_flatbytes(const uint8_t *src, uint8_t *guide, const RsgmDims &d, int n, cudaStream_t st);
 int launch_census(const uint8_t *src, uint32_t *dst, int W, int H, int n, cudaStream_t st);
-void census_set_fused(int on);
 int launch_census_fused(const uint8_t *src, uint32_t *dst, const RsgmDims &d, int n, cudaStream_t st);   // pad + gray + census, 1 = n/a
 int launch_cost_u16(const uint32_t *cl, const uint32_t *cr, uint16_t *dsi, int W, int H, int D, int n, cudaStream_t st);
 int launch_cost_u8(const uint32_t *cl, const uint32_t *cr, uint8_t *dsi, int W, int H, int D, int n, cudaStream_t st);
@@ -95,8 +94,6 @@ size_t sweep_halo_bytes(int W, int H, int D, int n);       // workspace of the v
 // p must satisfy sweep_params_supported(p, plain_costs)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost, uint16_t *S, void *halo_ws, int W, int H, int D, int n, float *dl,
                           float *dr, const float *lut, bool plain_costs, const SgmParams &p, const StageHook *hook, cudaStream_t st);
-void sweep_set_v_red(int on);
-void sweep_set_v_split(int on);
 int sweep_take_abort_flag(int *out);
 int launch_s_tile_to_xyd(const uint16_t *St, uint16_t *Sx, int W, int H, int D, int n, cudaStream_t st);
 void sweep_set_max_strip(int cols);
@@ -105,8 +102,7 @@ void sweep_set_clusters(int c);
 void vpp_set_rows_kernel(int on);
 void vpp_set_md_wave(int on);
 int vpp_take_md_abort_flag(int *out);
-int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int plane, int n,
-                           cudaStream_t st);
+int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, cudaStream_t st);
 int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st);
 int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st);
 int launch_subpixel(const uint16_t *S, float *disp, int W, int H, int D, int method, const float *lut, int n, cudaStream_t st);

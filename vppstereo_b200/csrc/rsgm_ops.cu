@@ -188,13 +188,7 @@ __global__ void __launch_bounds__(256) census5x5_kernel(const uint8_t *__restric
 // that the v-sweeps of the neighbouring batch have left, and the pipelined step loses 0.5 ms (22.2 vs 21.7 ms); with 8 rows the step
 // is where the two-kernel front was (21.7 ms), the gray image's round trip through HBM is gone and so is one launch per image.
 // ------------------------------------------------------------------------------------------------------------
-#ifndef VPP_CB_ROWS
-#define VPP_CB_ROWS 8
-#endif
-#ifndef VPP_CB_NT
-#define VPP_CB_NT 256
-#endif
-static constexpr int CB_ROWS = VPP_CB_ROWS, CB_HALO = 3, CB_NT = VPP_CB_NT, CB_BAND = CB_ROWS + 2 * CB_HALO;
+static constexpr int CB_ROWS = 8, CB_HALO = 3, CB_NT = 256, CB_BAND = CB_ROWS + 2 * CB_HALO;
 
 __device__ __forceinline__ uint32_t cb_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -333,9 +327,6 @@ __global__ void __launch_bounds__(CB_NT) census_fused_kernel(const uint8_t *__re
     }
 }
 
-static int g_census_fused = 1;      // test hook: 0 = always the two-kernel path
-void census_set_fused(int on) { g_census_fused = on != 0; }
-
 // 0 = done; 1 = not applicable here (source not 16-byte aligned, band beyond shared memory): the caller runs pad_gray + census
 int launch_census_fused(const uint8_t *src, uint32_t *dst, const RsgmDims &d, int n, cudaStream_t st)
 {
@@ -346,7 +337,7 @@ int launch_census_fused(const uint8_t *src, uint32_t *dst, const RsgmDims &d, in
     int dev = 0, smem_optin = 0;
     VPP_CUDA_TRY(cudaGetDevice(&dev));
     VPP_CUDA_TRY(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    if (smem > (size_t)smem_optin || !g_census_fused) return 1;
+    if (smem > (size_t)smem_optin) return 1;
     const int bands = cdiv(d.Hp, CB_ROWS);
     if ((long)bands * n > 0x7FFFFFFFL) return 1;
     VPP_CUDA_TRY(cudaFuncSetAttribute(census_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -451,15 +442,9 @@ int launch_guided_u8(uint8_t *dsi, const float *hints, const float *valid, const
 //          retires to disp_r[x'].  No atomics, no re-reads.
 //   sub-pixel (method 0, :1072-1102) optionally fused into the left result.
 // ------------------------------------------------------------------------------------------------------------
-// PLANE: S is in the internal plane layout of sgm_sweep.cu (word k*32 + lane of a pixel = disparities 2*NW*lane + 2k, +1)
-template <int NW, bool PLANE>
-__device__ __forceinline__ int s_at(const uint16_t *Srow, int x, int d, int D)
-{
-    if (PLANE) return Srow[((long)x * (NW * 32) + ((d % (2 * NW)) >> 1) * 32 + d / (2 * NW)) * 2 + (d & 1)];
-    return Srow[(long)x * D + d];
-}
+__device__ __forceinline__ int s_at(const uint16_t *Srow, int x, int d, int D) { return Srow[(long)x * D + d]; }
 
-template <int NW, bool LEFT, bool RIGHT, bool SUBPIX, bool PLANE>
+template <int NW, bool LEFT, bool RIGHT, bool SUBPIX>
 __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restrict__ S, float *__restrict__ disp_l,
                                                        float *__restrict__ disp_r, int W, int H, int D,
                                                        const float *__restrict__ lut, long total_rows)
@@ -468,7 +453,7 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
     if (row >= total_rows) return;
     const int lane = threadIdx.x & 31;
     const int d0 = 2 * NW * lane;
-    const uint16_t *Srow = S + row * (long)W * (PLANE ? NW * 64 : D);
+    const uint16_t *Srow = S + row * (long)W * D;
     const bool lane_valid = d0 < D;            // D % 8 == 0 and 2*NW in {2,4,6,8}: a lane is all-valid or partly valid
     uint32_t bucket[2 * NW];
 #pragma unroll
@@ -481,9 +466,7 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
         for (int k = 0; k < NW; k++) {
             const int d = d0 + 2 * k;
             uint32_t w = 0xFFFFFFFFu;
-            if (lane_valid && d < D)
-                w = PLANE ? reinterpret_cast<const uint32_t *>(Srow)[(long)x * (NW * 32) + k * 32 + lane]
-                          : *reinterpret_cast<const uint32_t *>(Srow + (long)x * D + d);
+            if (lane_valid && d < D) w = *reinterpret_cast<const uint32_t *>(Srow + (long)x * D + d);
             key[2 * k] = (d < D) ? ((w << 16) | (uint32_t)d) : 0xFFFFFFFFu;
             key[2 * k + 1] = (d + 1 < D) ? ((w & 0xFFFF0000u) | (uint32_t)(d + 1)) : 0xFFFFFFFFu;
         }
@@ -499,8 +482,8 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
                 if (SUBPIX && x >= 1 && x <= W - 2) {
                     if (best > 0) {
                         // best = D-1 reads the next pixel's d = 0 (xyd stream order)
-                        const int c0 = s_at<NW, PLANE>(Srow, x, best - 1, D), c1 = (int)(m >> 16);
-                        const int c2 = best + 1 < D ? s_at<NW, PLANE>(Srow, x, best + 1, D) : s_at<NW, PLANE>(Srow, x + 1, 0, D);
+                        const int c0 = s_at(Srow, x, best - 1, D), c1 = (int)(m >> 16);
+                        const int c2 = best + 1 < D ? s_at(Srow, x, best + 1, D) : s_at(Srow, x + 1, 0, D);
                         const int lower = min(c1 - c0, c1 - c2);            // <= 0
                         out = __fadd_rn((float)best, __fmul_rn((float)(c2 - c0), lut[-lower]));
                     } else {
@@ -524,34 +507,32 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
     }
 }
 
-template <bool LEFT, bool RIGHT, bool SUBPIX, bool PLANE>
+template <bool LEFT, bool RIGHT, bool SUBPIX>
 static int launch_wta_t(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, cudaStream_t st)
 {
     const long rows = (long)n * H;
     const int blocks = cdiv(rows * 32, 128);
     const int nw = (D + 63) / 64;
     switch (nw) {
-        case 1: wta_rows_kernel<1, LEFT, RIGHT, SUBPIX, PLANE><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
-        case 2: wta_rows_kernel<2, LEFT, RIGHT, SUBPIX, PLANE><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
-        case 3: wta_rows_kernel<3, LEFT, RIGHT, SUBPIX, PLANE><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
-        default: wta_rows_kernel<4, LEFT, RIGHT, SUBPIX, PLANE><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
+        case 1: wta_rows_kernel<1, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
+        case 2: wta_rows_kernel<2, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
+        case 3: wta_rows_kernel<3, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
+        default: wta_rows_kernel<4, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
     }
     VPP_LAUNCH_CHECK("wta_rows_kernel");
     return VPPB200_OK;
 }
 int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st)
 {
-    return launch_wta_t<true, false, false, false>(S, disp, nullptr, W, H, D, nullptr, n, st);
+    return launch_wta_t<true, false, false>(S, disp, nullptr, W, H, D, nullptr, n, st);
 }
 int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st)
 {
-    return launch_wta_t<false, true, false, false>(S, nullptr, disp, W, H, D, nullptr, n, st);
+    return launch_wta_t<false, true, false>(S, nullptr, disp, W, H, D, nullptr, n, st);
 }
-int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int plane, int n,
-                           cudaStream_t st)
+int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, cudaStream_t st)
 {
-    if (plane) return launch_wta_t<true, true, true, true>(S, dl, dr, W, H, D, lut, n, st);
-    return launch_wta_t<true, true, true, false>(S, dl, dr, W, H, D, lut, n, st);
+    return launch_wta_t<true, true, true>(S, dl, dr, W, H, D, lut, n, st);
 }
 
 // subPixelRefine as a stand-alone operator (RSGM/StereoBMHelper.cpp:1065-1135), one thread per pixel

@@ -235,10 +235,7 @@ int launch_s_tile_to_xyd(const uint16_t *St, uint16_t *Sx, int W, int H, int D, 
 // ------------------------------------------------------------------------------------------------------------
 static constexpr int HWARPS = 4;   // warps per CTA
 static constexpr int HCROW = 16;   // bytes of a staged cost row: 8 columns x uint16 (16-byte pieces, dense)
-#ifndef VPP_HSROW_WTA
-#define VPP_HSROW_WTA 32
-#endif
-static constexpr int HSROW_WTA = VPP_HSROW_WTA;   // the same for the fused WTA sweep (read only)
+static constexpr int HSROW_WTA = 32;   // the same for the fused WTA sweep (read only)
 static constexpr int HSROW = 48;   // bytes of a staged S row: 8 columns x uint32 + 16 B pad (3 pieces: odd => LDS.128 conflict-free)
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -598,17 +595,9 @@ struct VArgs {
     long state_words;
 };
 
-#ifndef VPP_VREGS
-#define VPP_VREGS 96
-#endif
-#ifndef VPP_VPARTS
-#define VPP_VPARTS 3
-#endif
-#ifndef VPP_VU
-#define VPP_VU 8
-#endif
-static constexpr int VPARTS = VPP_VPARTS;   // warps per column group (each owns a share of the disparity pairs)
-static constexpr int VU = VPP_VU;           // disparity pairs per operand block (software pipelined)
+static constexpr int VREGS = 96;    // register cap of the whole-frame v-sweep (see sgm_v2_kernel)
+static constexpr int VPARTS = 3;    // warps per column group (each owns a share of the disparity pairs)
+static constexpr int VU = 8;        // disparity pairs per operand block (software pipelined)
 
 __device__ __forceinline__ uint32_t add3(uint32_t a, uint32_t b, uint32_t c)
 {
@@ -718,19 +707,6 @@ __device__ __noinline__ uint32_t halo_wait2(const uint32_t *p, uint32_t tag, uin
     return 0u;
 }
 
-#ifdef VPP_TRACE
-// debug build only (tools/vtrace.py): clock64 stamps of one CTA's warps over a window of rows
-static constexpr int TR_ROW0 = 100, TR_ROWS = 24, TR_STAMPS = 12, TR_CTA = 3;
-__device__ unsigned long long g_vtrace[32 * TR_ROWS * TR_STAMPS];
-#define VTRACE(k)                                                                                                      \
-    do {                                                                                                               \
-        if (blockIdx.x == TR_CTA && lane == 0 && t >= TR_ROW0 && t < TR_ROW0 + TR_ROWS)                                 \
-            g_vtrace[(warp * TR_ROWS + (t - TR_ROW0)) * TR_STAMPS + (k)] = clock64();                                  \
-    } while (0)
-#else
-#define VTRACE(k) do { } while (0)
-#endif
-
 struct VPath2 {
     uint32_t cur;      // word k of the predecessor: Lt[k], Lt[k + K2]
     uint32_t prev;     // word k-1 (for word 0: the seam (inf, Lt[K2-1]))
@@ -747,10 +723,10 @@ __device__ __forceinline__ void red_add_u32(uint32_t *p, uint32_t v)
 // One block of up to VU words for the three paths.  s* = predecessor state rows of the block (stride NS), w* = this row's state
 // rows (same slots), Sg = the block's S words (stride 32).  GUARD: only the first `cnt` words exist; `last`: the block ends this
 // warp's share, whose upper neighbour word was read before the column group's barrier (wr*).
-// RED: S += goes out as a fire-and-forget reduction to L2 (the addend's halves are <= 3 * (Cmax + P2max) and S's halves never
+// S += goes out as a fire-and-forget reduction to L2 (the addend's halves are <= 3 * (Cmax + P2max) and S's halves never
 // overflow, so the 32-bit add is exact for both halves): no load of S, no operand registers, no latency to hide
-template <int NS, bool GUARD, bool NORM, bool RED>
-__device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_t (&sb)[VU], const uint32_t *s1,
+template <int NS, bool GUARD, bool NORM>
+__device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_t *s1,
                                          const uint32_t *s2, const uint32_t *s3, uint32_t *w1, uint32_t *w2, uint32_t *w3,
                                          uint32_t wr1, uint32_t wr2, uint32_t wr3, VPath2 &p1, VPath2 &p2, VPath2 &p3,
                                          uint32_t negm, uint32_t p1x2, uint32_t *Sg, int cnt, bool last)
@@ -793,8 +769,7 @@ __device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_
                 p1.mr = __vminu2(p1.mr, t1); p2.mr = __vminu2(p2.mr, t2); p3.mr = __vminu2(p3.mr, t3);
             }
             tp1 = t1; tp2 = t2; tp3 = t3;
-            if (RED) red_add_u32(Sg + u * 32, sum);
-            else Sg[u * 32] = sum + sb[u];
+            red_add_u32(Sg + u * 32, sum);
             p1.prev = p1.cur; p2.prev = p2.cur; p3.prev = p3.cur;
             p1.cur = nx1[u]; p2.cur = nx2[u]; p3.cur = nx3[u];
         }
@@ -802,20 +777,20 @@ __device__ __forceinline__ void v2_block(const uint32_t (&cb)[VU], const uint32_
 }
 
 // NS = GC * 32 ring slots + the border slot.
-// FULL: every warp's share of the words is a whole number of VU-blocks (no guards in the inner loop).  NORM, RED: see above.
+// FULL: every warp's share of the words is a whole number of VU-blocks (no guards in the inner loop).  NORM: see above.
 // halo: [CTA][r1 | r3][row parity][K2 state words + VPARTS part minima] inbound buffers, then one abort word at the end
-// Register cap: 96 where the S update is a reduction (no operand registers for S; no spills): the one-CTA-per-SM grid then
+// Register cap: VREGS = 96 (the S update is a reduction: no operand registers for S; no spills): the one-CTA-per-SM grid then
 // leaves a quarter of the register file and ~30 KB of shared memory per SM to the front / tail kernels of the neighbouring
 // batches, which run beside the sweep (measured: the sweep alone 6.09 -> 6.39 ms, the pipelined step 23.7 -> 23.3 ms)
 // BAND: the launch covers a row band of taller frames (state import / export at the band's ends); whole-frame launches are
 // compiled without that code (it costs the hot loop 0.3 ms per launch under the register cap).  Band launches take the 128 cap
 // (a band's sweep does not share the SMs with the phases of neighbouring batches; under 96 registers the runtime P1 made the
 // band kernels spill).  The residency plan (v_resident_ctas) is computed for 128 registers either way.
-template <int NS, bool FULL, bool NORM, bool RED, bool BAND>
-__global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const uint32_t *__restrict__ p2q_all,
-                                                                                 const uint16_t *__restrict__ cost_all,
-                                                                                 uint32_t *__restrict__ S_all, uint32_t *halo,
-                                                                                 uint32_t *abort_flag, VArgs a)
+template <int NS, bool FULL, bool NORM, bool BAND>
+__global__ void __maxnreg__(BAND ? 128 : VREGS) sgm_v2_kernel(const uint32_t *__restrict__ p2q_all,
+                                                              const uint16_t *__restrict__ cost_all,
+                                                              uint32_t *__restrict__ S_all, uint32_t *halo,
+                                                              uint32_t *abort_flag, VArgs a)
 {
     extern __shared__ __align__(16) uint32_t smem[];
     using SW = uint32_t;
@@ -915,36 +890,30 @@ __global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const 
 
     unsigned t = 0;                                 // rows processed by this team so far, over all its frames
     int sh = 0;                                     // t mod n: the ring phase runs on across frames
-    uint32_t cb[VU], sb[VU];
+    uint32_t cb[VU];
 #pragma unroll
-    for (int u = 0; u < VU; u++) { cb[u] = 0; sb[u] = 0; }
+    for (int u = 0; u < VU; u++) cb[u] = 0;
     uint32_t p2w = 0;                               // packed (P2 - P1) of the three paths for the coming row
     for (int f = cid; f < a.n; f += nteams) {
         const uint16_t *cost_f = cost_all + f * a.t.frame + lane;
         SW *S_f = reinterpret_cast<SW *>(S_all) + f * a.t.frame + lane;
         const uint32_t *p2_f = p2q_all + (long)f * H * G32 + x;
-        auto load_block = [&](const uint16_t *cp, const SW *sp, int cnt, uint32_t (&c)[VU], uint32_t (&sv)[VU], bool with_s) {
+        auto load_block = [&](const uint16_t *cp, int cnt, uint32_t (&c)[VU]) {
 #pragma unroll
-            for (int u = 0; u < VU; u++) {
-                if (FULL || u < cnt) {
-                    c[u] = cp[u * 32];
-                    sv[u] = (!RED && with_s) ? sp[u * 32] : 0u;
-                }
-            }
+            for (int u = 0; u < VU; u++)
+                if (FULL || u < cnt) c[u] = cp[u * 32];
         };
         const bool cont = BAND && !a.pass_start;    // row band that continues a sweep: its first row is an ordinary row
-        if (f == cid) load_block(cost_f + (((long)i1 * G + g) * K2 + k0) * 32, S_f + (((long)i1 * G + g) * K2 + k0) * 32, k1 - k0, cb, sb, cont);
+        if (f == cid) load_block(cost_f + (((long)i1 * G + g) * K2 + k0) * 32, k1 - k0, cb);
         for (int s = 0; s < H; s++, t++) {
             const int i = i1 + s * di;
             // ring slots: a line moving +1 column per row sits in slot (lc - t) mod n, one moving -1 in (lc + t) mod n
             int slotA = lc - sh; if (slotA < 0) slotA += n;
             int slotB = lc + sh; if (slotB >= n) slotB -= n;
             const int d1 = dj > 0 ? slotA : slotB, d2 = lc, d3 = dj > 0 ? slotB : slotA;
-            VTRACE(0);
             if (t > 0) {
                 // ---- rows t-1 of the groups this row depends on
                 wait_rows(t - 1u);
-                VTRACE(1);
                 // ---- lines entering from the neighbour CTAs: row t-1 of their edge column, into the ring slot of the entering lane
                 if (enter1 | enter3) {
                     const unsigned pp = (t - 1u) & 1u, tag = ((t - 1u) >> 1) & 7u;
@@ -989,15 +958,14 @@ __global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const 
                 p2w = p2_f[(long)i * G32];
                 group_barrier();
             }
-            VTRACE(2);
             const long tb0 = (((long)i * G + g) * K2 + k0) * 32;
             const uint16_t *cp = cost_f + tb0;
             SW *sp = S_f + tb0;
+            const long tbn = (((long)(i + di) * G + g) * K2 + k0) * 32;     // the next row's tile offset
             if (s + 1 < H) {
                 // pull the next row's operands of this warp into L2 while this row is being processed
-                const long tbn = (((long)(i + di) * G + g) * K2 + k0) * 32 - lane;
-                if (k0 + lane < k1) prefetch_l2(S_f + tbn + lane * 32);       // (RED: the line is in L2 when the reduction arrives)
-                if (k0 + 2 * lane < k1) prefetch_l2(cost_f + tbn + lane * 64);
+                if (k0 + lane < k1) prefetch_l2(S_f + (tbn - lane) + lane * 32);       // (the line is in L2 when the reduction arrives)
+                if (k0 + 2 * lane < k1) prefetch_l2(cost_f + (tbn - lane) + lane * 64);
             }
             uint32_t *w1 = st + (0 * K2 + k0) * NS + d1, *w2 = st + (1 * K2 + k0) * NS + d2, *w3 = st + (2 * K2 + k0) * NS + d3;
             VPath2 p1, p2, p3;
@@ -1005,10 +973,10 @@ __global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const 
             if (s == 0 && !cont) {
                 // first row of the pass: L = C on all three paths, nothing is summed (StereoSGM_SSE.hpp:116-218)
                 for (int kb = k0; kb < k1; kb += VU) {
-                    uint32_t cn[VU], sn[VU];
+                    uint32_t cn[VU];
 #pragma unroll
-                    for (int u = 0; u < VU; u++) { cn[u] = 0; sn[u] = 0; }
-                    if (kb + VU < k1) load_block(cp + VU * 32, nullptr, k1 - kb - VU, cn, sn, false);
+                    for (int u = 0; u < VU; u++) cn[u] = 0;
+                    if (kb + VU < k1) load_block(cp + VU * 32, k1 - kb - VU, cn);
 #pragma unroll
                     for (int u = 0; u < VU; u++) {
                         if (FULL || kb + u < k1) {
@@ -1051,21 +1019,17 @@ __global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const 
                                wr3 = k1 < K2 ? s3[ke] : __byte_perm(s3[kz], SW_INF2, 0x5432);
                 p1.cur = s1[0]; p2.cur = s2[0]; p3.cur = s3[0];
                 group_barrier();                    // every warp of the group has read its neighbours' boundary pairs and minima
-                VTRACE(3);
-                int trb = 4;
                 for (int kb = k0; kb < k1; kb += 2 * VU) {
-                    uint32_t cn[VU], sn[VU];
+                    uint32_t cn[VU];
                     const bool last1 = kb + VU >= k1;
-                    if (!last1) load_block(cp + VU * 32, sp + VU * 32, k1 - kb - VU, cn, sn, true);
-                    v2_block<NS, !FULL, NORM, RED>(cb, sb, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, p1x2, sp, k1 - kb, last1);
-                    VTRACE(trb); trb++;
+                    if (!last1) load_block(cp + VU * 32, k1 - kb - VU, cn);
+                    v2_block<NS, !FULL, NORM>(cb, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, p1x2, sp, k1 - kb, last1);
                     cp += VU * 32; sp += VU * 32;
                     s1 += VU * NS; s2 += VU * NS; s3 += VU * NS; w1 += VU * NS; w2 += VU * NS; w3 += VU * NS;
                     if (last1) break;
                     const bool last2 = kb + 2 * VU >= k1;
-                    if (!last2) load_block(cp + VU * 32, sp + VU * 32, k1 - kb - 2 * VU, cb, sb, true);
-                    v2_block<NS, !FULL, NORM, RED>(cn, sn, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, p1x2, sp, k1 - kb - VU, last2);
-                    VTRACE(trb); trb++;
+                    if (!last2) load_block(cp + VU * 32, k1 - kb - 2 * VU, cb);
+                    v2_block<NS, !FULL, NORM>(cn, s1, s2, s3, w1, w2, w3, wr1, wr2, wr3, p1, p2, p3, negm, p1x2, sp, k1 - kb - VU, last2);
                     cp += VU * 32; sp += VU * 32;
                     s1 += VU * NS; s2 += VU * NS; s3 += VU * NS; w1 += VU * NS; w2 += VU * NS; w3 += VU * NS;
                 }
@@ -1110,39 +1074,27 @@ __global__ void __maxnreg__(RED && !BAND ? VPP_VREGS : 128) sgm_v2_kernel(const 
                 for (int k = k0 + lane; k < k1; k += 32) st_relaxed_gpu(dst + k, (st[(2 * K2 + k) * NS + sl] - mv * 0x10001u) | otag);
                 if (lane == 0) st_relaxed_gpu(dst + K2 + part, mv | otag);
             }
-            VTRACE(8);
             row_done(t);
-            VTRACE(9);
             // prefetch for the next row: its P2 word and first operand block
             if (s + 1 < H) {
                 const int in = i + di;
                 p2w = p2_f[(long)in * G32];
-                const long tbn = (((long)in * G + g) * K2 + k0) * 32;
-                load_block(cost_f + tbn, S_f + tbn, k1 - k0, cb, sb, true);
+                load_block(cost_f + tbn, k1 - k0, cb);
             } else if (f + nteams < a.n) {
                 const uint16_t *cost_n = cost_all + (long)(f + nteams) * a.t.frame + lane;
-                const SW *S_n = reinterpret_cast<SW *>(S_all) + (long)(f + nteams) * a.t.frame + lane;
-                load_block(cost_n + (((long)i1 * G + g) * K2 + k0) * 32, S_n + (((long)i1 * G + g) * K2 + k0) * 32, k1 - k0, cb, sb, cont);
+                load_block(cost_n + (((long)i1 * G + g) * K2 + k0) * 32, k1 - k0, cb);
             }
-            VTRACE(10);
             if (++sh == n) sh = 0;
         }
     }
 }
-
-#ifdef VPP_TRACE
-extern "C" int vppb200_debug_vtrace(unsigned long long *host, int n)
-{
-    return cudaMemcpyFromSymbol(host, g_vtrace, sizeof(unsigned long long) * (size_t)n) == cudaSuccess ? 0 : -1;
-}
-#endif
 
 static size_t v_smem_bytes(int GC, int K2) { return ((size_t)3 * K2 * (GC * 32 + 1) + (size_t)3 * VPARTS * (GC * 32 + 1) + 4 + 4 * GC) * 4; }
 
 // tuning / test hook: upper bound on the strip width in columns (0 = chosen by the planner)
 static int g_max_strip = 0;
 void sweep_set_max_strip(int cols) { g_max_strip = cols < 0 ? 0 : cols; }
-static int g_force_teams = 0;       // experiment hook: frames in flight instead of the occupancy estimate
+static int g_force_teams = 0;       // test hook: upper bound on frames in flight (forces multi-round teams on small batches)
 void sweep_set_clusters(int c) { g_force_teams = c < 0 ? 0 : c; }
 
 // a team = the csize CTAs (one per SM) that hold one frame; nteams frames are in flight
@@ -1155,8 +1107,8 @@ static int v_resident_ctas(size_t smem, int threads, int *out)
     VPP_CUDA_TRY(cudaGetDevice(&dev));
     VPP_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     constexpr int NS = GC * 32 + 1;
-    VPP_CUDA_TRY(cudaFuncSetAttribute(sgm_v2_kernel<NS, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    VPP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sgm_v2_kernel<NS, true, false, false, true>, threads, smem));
+    VPP_CUDA_TRY(cudaFuncSetAttribute(sgm_v2_kernel<NS, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VPP_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sgm_v2_kernel<NS, true, false, true>, threads, smem));
     // One CTA per SM.  (Measured: two CTAs of different frames per SM on 64-column strips take 3.83 us per row for their 4
     // column groups, one CTA with 5 groups 3.97 us -- the row time is a latency chain, wait -> hand-off -> setup -> loop ->
     // push, that does not shrink with the strip, so the widest strip that fits wins.)
@@ -1232,15 +1184,13 @@ static int plan_v(const TL &t, int n, VPlan *plan)
 // 3.67 / 3.50 / 3.40 for 5 / 4 / 3 / 2 column groups per CTA), so e.g. 64 K frames run as 36 frames x 8 CTAs (two rounds of 18
 // teams) + 28 frames x 10 CTAs (two rounds of 14 teams) instead of four rounds of 18 teams with the last one 10 / 18 full.
 struct VSplit { int n1; VPlan p1; int n2; VPlan p2; };
-static int g_v_split = 1;
-void sweep_set_v_split(int on) { g_v_split = on != 0; }
 static int plan_v_split(const TL &t, int n, VSplit *out)
 {
-    static thread_local struct { int W, H, D, n, dev, strip, teams, split; VSplit s; bool ok; } memo = {0, 0, 0, 0, -1, 0, 0, 0, {}, false};
+    static thread_local struct { int W, H, D, n, dev, strip, teams; VSplit s; bool ok; } memo = {0, 0, 0, 0, -1, 0, 0, {}, false};
     int dev = 0;
     VPP_CUDA_TRY(cudaGetDevice(&dev));
     if (memo.ok && memo.W == t.W && memo.H == t.H && memo.D == t.D && memo.n == n && memo.dev == dev && memo.strip == g_max_strip &&
-        memo.teams == g_force_teams && memo.split == g_v_split) {
+        memo.teams == g_force_teams) {
         *out = memo.s;
         return VPPB200_OK;
     }
@@ -1248,7 +1198,7 @@ static int plan_v_split(const TL &t, int n, VSplit *out)
     int rc = plan_v(t, n, &best.p1);
     if (rc) return rc;
     best.n1 = n; best.n2 = 0;
-    if (g_v_split && g_max_strip == 0 && g_force_teams == 0 && n > best.p1.nteams) {
+    if (g_max_strip == 0 && g_force_teams == 0 && n > best.p1.nteams) {
         static const double trow[6] = {0.0, 3.30, 3.40, 3.50, 3.67, 3.97};      // relative row time by groups per CTA
         const int gc_max = best.p1.GC;
         VPlan cand[6];
@@ -1282,7 +1232,7 @@ static int plan_v_split(const TL &t, int n, VSplit *out)
         }
     }
     *out = best;
-    memo = {t.W, t.H, t.D, n, dev, g_max_strip, g_force_teams, g_v_split, best, true};
+    memo = {t.W, t.H, t.D, n, dev, g_max_strip, g_force_teams, best, true};
     return VPPB200_OK;
 }
 
@@ -1293,9 +1243,6 @@ size_t sweep_halo_bytes(int W, int H, int D, int n)
     (void)D;
     return HALO_LINES_BYTES + 256 + (size_t)n * H * ((W + 31) / 32) * 32 * 4;
 }
-
-static int g_v_red = 1;             // S += by red.global.add (default) instead of load + add + store
-void sweep_set_v_red(int on) { g_v_red = on != 0; }
 
 // words of one frame's exported row state: [3][G*32][K2] path words + [3][G*32][VPARTS] part minima
 long sweep_state_words(int W, int D) { return (long)3 * ((W + 31) / 32) * 32 * (D / 2 + VPARTS); }
@@ -1318,11 +1265,9 @@ static int run_v_t(const uint32_t *p2q, const uint16_t *cost, uint32_t *S, uint3
     void *args[] = {(void *)&p2q, (void *)&cost, (void *)&S, (void *)&halo, (void *)&abort_flag, (void *)&a};
     const bool banded = !band.pass_start || band.state_in != nullptr || band.state_out != nullptr;
     const void *kern;
-#define VPP_VK(F, N, R) (banded ? (const void *)sgm_v2_kernel<NS, F, N, R, true> : (const void *)sgm_v2_kernel<NS, F, N, R, false>)
-    if (norm && g_v_red) kern = full ? VPP_VK(true, true, true) : VPP_VK(false, true, true);
-    else if (norm) kern = full ? VPP_VK(true, true, false) : VPP_VK(false, true, false);
-    else if (g_v_red) kern = full ? VPP_VK(true, false, true) : VPP_VK(false, false, true);
-    else kern = full ? VPP_VK(true, false, false) : VPP_VK(false, false, false);
+#define VPP_VK(F, N) (banded ? (const void *)sgm_v2_kernel<NS, F, N, true> : (const void *)sgm_v2_kernel<NS, F, N, false>)
+    if (norm) kern = full ? VPP_VK(true, true) : VPP_VK(false, true);
+    else kern = full ? VPP_VK(true, false) : VPP_VK(false, false);
 #undef VPP_VK
     VPP_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
     // cooperative launch: all CTAs resident (they poll each other's halo words), one grid sync at the start

@@ -1032,10 +1032,8 @@ struct MdSplat {
     }
 };
 
-#ifndef VPP_MD_MINB
-#define VPP_MD_MINB 12
-#endif
-__global__ void __launch_bounds__(32, VPP_MD_MINB) vpp_max_dist_wave_kernel(uint8_t *l, uint8_t *r, const float *__restrict__ g,
+static constexpr int MD_MINB = 12;      // minimum resident CTAs (one warp each) per SM: caps the wavefront kernel's registers
+__global__ void __launch_bounds__(32, MD_MINB) vpp_max_dist_wave_kernel(uint8_t *l, uint8_t *r, const float *__restrict__ g,
                                                                const uint8_t *__restrict__ g_occ, VppWs ws, MdWs md, VppArgs a,
                                                                int units, int RD)
 {
@@ -1194,7 +1192,7 @@ int vpp_take_md_abort_flag(int *out)
     return VPPB200_OK;
 }
 
-void vpp_set_md_wave(int on) { g_vpp_md_wave = on < 0 ? 0 : on; }   // > 1: rows in flight per SM (experiments)
+void vpp_set_md_wave(int on) { g_vpp_md_wave = on > 0; }
 
 static VppArgs make_args(int W, int H, int C, int uniform, int wsize, int wax, int way, int direction, double c, double c_occ,
                          int discard, int interpolate, int arith)
@@ -1348,8 +1346,7 @@ static int scan_max_dist_impl(uint8_t *l, uint8_t *r, const float *g, int W, int
         VPP_LAUNCH_CHECK("vpp_md_deps_kernel");
         VPP_CUDA_TRY(cudaFuncSetAttribute(vpp_max_dist_wave_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const long rows = (long)total * H;
-        long resident = (long)sms * (smem <= 4096 ? 32 : max((size_t)1, (size_t)200 * 1024 / (smem + 1024)));
-        if (g_vpp_md_wave > 1) resident = min(resident, (long)sms * g_vpp_md_wave);
+        const long resident = (long)sms * (smem <= 4096 ? 32 : max((size_t)1, (size_t)200 * 1024 / (smem + 1024)));
         vpp_max_dist_wave_kernel<<<(unsigned)min(rows, resident), 32, smem, st>>>(l, r, g, g_occ, ws, md, a, total, RD);
         VPP_LAUNCH_CHECK("vpp_max_dist_wave_kernel");
         return VPPB200_OK;

@@ -53,8 +53,7 @@ class VppRsgmPipeline:
             self.lv2, self.rv2 = [self.lv, torch.empty_like(self.lv)], [self.rv, torch.empty_like(self.lv)]
             self.vpp_stream = torch.cuda.Stream(self.device)      # front phase: VPP + pad/gray/census/cost volume
             # the sweeps are the critical path: their CTAs are scheduled ahead of the front / tail kernels that fill in beside them
-            prio = int(__import__("os").environ.get("VPPB200_MAIN_PRIORITY", "-1"))
-            self.main_stream = torch.cuda.Stream(self.device, priority=prio)     # SGM sweeps + WTA
+            self.main_stream = torch.cuda.Stream(self.device, priority=-1)       # SGM sweeps + WTA
             self.tail_stream = torch.cuda.Stream(self.device)     # median ... background fill
             self.front_done = [torch.cuda.Event(), torch.cuda.Event()]
             self.main_done = [None, None]
