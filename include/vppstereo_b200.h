@@ -234,6 +234,17 @@ int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_l, const ui
                         uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
                         uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
                         size_t workspace_bytes, void *stream, const vppb200_sgm_params *params);
+/*   vppb200_sgm_band_guided: vppb200_sgm_band_ex + guided matching (rsgm.py:115-127, the hints / validhints of
+ *       vppb200_compute_rsgm): hints, validhints float32 [H][W], the WHOLE unpadded frame.  Both NULL: exactly vppb200_sgm_band_ex;
+ *       exactly one NULL: VPPB200_ERR_ARG.  With hints, phase 1 modulates the band's volume (rows of the padded frame map to hint
+ *       rows row0 + r - pad_top) and params must lie in the guided sweep domain (Cmax = 240, see vppb200_sgm_params_fast).  Every
+ *       phase of every band of one frame must be called with the same params and hint nullness (they select the sweeps' state
+ *       representation); hints are only read by phase 1.  Arguments are validated before any CUDA call. */
+int vppb200_sgm_band_guided(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                            uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
+                            uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
+                            size_t workspace_bytes, void *stream, const vppb200_sgm_params *params, const float *hints,
+                            const float *validhints);
 int vppb200_rsgm_tail(float *dl, float *dr, float *disp_out, int H, int W, int C, int D, int flags, void *workspace,
                       size_t workspace_bytes, void *stream);
 

@@ -28,7 +28,7 @@ SYMBOLS = [
     "vppb200_u8hwc_to_f32chw", "vppb200_set_tuning",
     "vppb200_occlusion_workspace_bytes", "vppb200_occlusion_heuristic",
     "vppb200_banded_workspace_bytes", "vppb200_banded_dims", "vppb200_rsgm_front_census", "vppb200_sgm_band", "vppb200_rsgm_tail",
-    "vppb200_compute_rsgm_ex", "vppb200_sgm_band_ex", "vppb200_sgm_params_fast",
+    "vppb200_compute_rsgm_ex", "vppb200_sgm_band_ex", "vppb200_sgm_params_fast", "vppb200_sgm_band_guided",
 ]
 
 _lib = None

@@ -99,7 +99,9 @@ class BandedRsgm:
                                                     C.c_size_t(self.ws.numel()), _lib.stream_ptr(self.device))
         _lib.check(rc, "rsgm_front_census")
 
-    def run_band(self, band, phases, cost, S, state_in=None, state_out=None, stream=None):
+    def run_band(self, band, phases, cost, S, state_in=None, state_out=None, stream=None, hints=None, validhints=None):
+        """phases of one band (vppb200_sgm_band_guided); hints / validhints: float32 [H,W] CUDA tensors of the whole frame or both
+        None, the same nullness for every phase of every band of a frame"""
         row0, rows = band
         torch = self.torch
         dl = self.dl[row0:row0 + rows]
@@ -107,11 +109,32 @@ class BandedRsgm:
         with torch.cuda.device(self.device):
             st = _lib.stream_ptr(self.device) if stream is None else C.c_void_p(stream.cuda_stream)
             prm = None if self.sgm_params is None else C.byref(self.sgm_params)
-            rc = self.lib.vppb200_sgm_band_ex(_lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost), _lib.ptr(S),
-                                              self.H, self.W, self.C, self.D, row0, rows, int(phases), _lib.ptr(state_in),
-                                              _lib.ptr(state_out), _lib.ptr(dl), _lib.ptr(dr), None, _lib.ptr(self.ws),
-                                              C.c_size_t(self.ws.numel()), st, prm)
+            rc = self.lib.vppb200_sgm_band_guided(_lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost),
+                                                  _lib.ptr(S), self.H, self.W, self.C, self.D, row0, rows, int(phases),
+                                                  _lib.ptr(state_in), _lib.ptr(state_out), _lib.ptr(dl), _lib.ptr(dr), None,
+                                                  _lib.ptr(self.ws), C.c_size_t(self.ws.numel()), st, prm, _lib.ptr(hints),
+                                                  _lib.ptr(validhints))
         _lib.check(rc, "sgm_band")
+
+    def _hints(self, hints, validhints):
+        """guided matching operands (rsgm.py:115-127) as compute_rsgm takes them -> (hints, validhints) float32 [H,W] CUDA tensors,
+        or (None, None).  Refused with ValueError before any device work: one operand without the other, and parameters outside the
+        guided sweep domain (there is no per-path band path)."""
+        if (hints is None) != (validhints is None):
+            raise ValueError("hints and validhints must be given together")
+        if hints is None:
+            return None, None
+        if self.sgm_params is not None and not _lib.sgm_params_fast(self.sgm_params, guided=True):
+            p = self.sgm_params
+            raise ValueError(f"SGM parameters {(p.p1, p.p2min, p.alpha, p.gamma)} are outside the guided sweep domain (no banded path "
+                             "for them)")
+        out = []
+        for name, a in (("hints", hints), ("validhints", validhints)):
+            t = _lib.as_device(a, self.torch.float32, self.device)
+            if t.numel() != self.H * self.W:
+                raise ValueError(f"{name}: expected one frame of shape {(self.H, self.W)}, got {tuple(t.shape)}")
+            out.append(t.reshape(self.H, self.W).contiguous())
+        return tuple(out)
 
     def tail(self, out=None):
         """median .. background fill on the raw maps of the whole frame (rsgm.py:273-292)"""
@@ -124,9 +147,11 @@ class BandedRsgm:
         _lib.check(rc, "rsgm_tail")
         return out
 
-    def compute(self, left, left_vpp, right_vpp):
-        """compute_rsgm(left, left_vpp, right_vpp) -> float32 [H,W]: all bands on this GPU, one after the other.  numpy in -> numpy
-        out, CUDA tensors in -> CUDA tensor out."""
+    def compute(self, left, left_vpp, right_vpp, hints=None, validhints=None):
+        """compute_rsgm(left, left_vpp, right_vpp, hints, validhints) -> float32 [H,W]: all bands on this GPU, one after the other.
+        numpy in -> numpy out, CUDA tensors in -> CUDA tensor out.  hints / validhints: guided matching, float32 [H,W], both or
+        neither (ValueError otherwise)."""
+        h, v = self._hints(hints, validhints)
         host = not _lib.is_tensor(left_vpp)
         self.front(left, left_vpp, right_vpp)
         bufs = [self.band_buffers(rows) for _, rows in self.bands]
@@ -134,11 +159,11 @@ class BandedRsgm:
         nb = len(self.bands)
         for k, band in enumerate(self.bands):                          # pass 0 flows down the bands
             self.run_band(band, PH_COST | PH_H_FWD | PH_V_DOWN, *bufs[k], state_in=states[k - 1] if k > 0 else None,
-                          state_out=states[k] if k + 1 < nb else None)
+                          state_out=states[k] if k + 1 < nb else None, hints=h, validhints=v)
         ups = [self.state_buffer() for _ in self.bands]
         for k in reversed(range(nb)):                                  # pass 1 flows back up, then the band's last sweep + WTA
             self.run_band(self.bands[k], PH_V_UP | PH_H_BWD, *bufs[k], state_in=ups[k + 1] if k + 1 < nb else None,
-                          state_out=ups[k] if k > 0 else None)
+                          state_out=ups[k] if k > 0 else None, hints=h, validhints=v)
         out = self.tail()
         return out.cpu().numpy() if host else out
 
@@ -166,21 +191,23 @@ class BandedRsgmDist(BandedRsgm):
         self.disp_box = PeerGather((2, rows_max, self.Wp), torch.float32, self.device, group=group, depth=2)
         self.frame = 0
 
-    def compute(self, left, left_vpp, right_vpp):
+    def compute(self, left, left_vpp, right_vpp, hints=None, validhints=None):
+        """as BandedRsgm.compute (hints / validhints: the whole frame on every rank)"""
+        h, v = self._hints(hints, validhints)
         torch = self.torch
         host = not _lib.is_tensor(left_vpp)
         r, nb, f = self.rank, self.world, self.frame
         self.frame += 1
         sb, db = self.state_box, self.disp_box
         self.front(left, left_vpp, right_vpp)
-        self.run_band(self.band, PH_COST | PH_H_FWD, self.cost, self.S)
+        self.run_band(self.band, PH_COST | PH_H_FWD, self.cost, self.S, hints=h, validhints=v)
         # ---- pass 0: wait for the band above, sweep down, hand the row state to the band below
         state_in = None
         if r > 0:
             sb.wait_from(2 * f, r - 1)
             state_in = sb.bufs[0, r - 1]
         out_state = self.state_buffer() if r + 1 < nb else None
-        self.run_band(self.band, PH_V_DOWN, self.cost, self.S, state_in=state_in, state_out=out_state)
+        self.run_band(self.band, PH_V_DOWN, self.cost, self.S, state_in=state_in, state_out=out_state, hints=h, validhints=v)
         if r > 0:
             sb.release_to(2 * f, r - 1)
         if r + 1 < nb:
@@ -191,7 +218,8 @@ class BandedRsgmDist(BandedRsgm):
             sb.wait_from(2 * f + 1, r + 1)
             state_in = sb.bufs[1, r + 1]
         out_state = self.state_buffer() if r > 0 else None
-        self.run_band(self.band, PH_V_UP | PH_H_BWD, self.cost, self.S, state_in=state_in, state_out=out_state)
+        self.run_band(self.band, PH_V_UP | PH_H_BWD, self.cost, self.S, state_in=state_in, state_out=out_state, hints=h,
+                      validhints=v)
         if r + 1 < nb:
             sb.release_to(2 * f + 1, r + 1)
         if r > 0:

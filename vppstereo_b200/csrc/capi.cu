@@ -470,10 +470,9 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
         }
         if (side != st && (rc = stream_chain(side, st))) return rc;
         tm.done(VPPB200_STAGE_CENSUS);
-        // rsgm.py:263-268  Hamming volume (+ optional guided modulation)
+        // rsgm.py:263-268  Hamming volume (+ optional guided modulation: in the same kernel on the tiled path)
         if (tiled) {
-            if ((rc = launch_cost_tile(w.census_l, w.census_r, w.dsi, d.Wp, d.Hp, D, n, st))) return rc;
-            if (hints && (rc = launch_guided_tile(w.dsi, hints, validhints, d, n, st))) return rc;
+            if ((rc = launch_cost_tile(w.census_l, w.census_r, w.dsi, d.Wp, d.Hp, D, n, guide_ops(hints, validhints, d), st))) return rc;
         } else {
             if ((rc = launch_cost_u8(w.census_l, w.census_r, w.dsi, d.Wp, d.Hp, D, n, st))) return rc;
             if (hints && (rc = launch_guided_u8(w.dsi, hints, validhints, d, n, st))) return rc;
@@ -636,14 +635,17 @@ extern "C" int vppb200_rsgm_front_census(const uint8_t *left, const uint8_t *lef
     return launch_census(w.gray_l, census_l, d.Wp, d.Hp, 1, st);
 }
 
-extern "C" int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
-                                   uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
-                                   uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
-                                   size_t workspace_bytes, void *stream, const vppb200_sgm_params *params)
+extern "C" int vppb200_sgm_band_guided(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                                       uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases,
+                                       const uint32_t *state_in, uint32_t *state_out, float *dl_band, float *dr_band,
+                                       const float *rcp_lut, void *workspace, size_t workspace_bytes, void *stream,
+                                       const vppb200_sgm_params *params, const float *hints, const float *validhints)
 {
     SgmParams prm;
     if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
-    if (!sweep_params_supported(prm, true)) return VPPB200_ERR_ARG;      // bands exist on the sweeps only
+    if ((hints == nullptr) != (validhints == nullptr)) return VPPB200_ERR_ARG;
+    const bool plain = hints == nullptr;
+    if (!sweep_params_supported(prm, plain)) return VPPB200_ERR_ARG;     // bands exist on the sweeps only
     if (!guide || !cost_band || !S_band || H <= 0 || W <= 0 || (C != 1 && C != 3) || phases <= 0 || phases > 31) return VPPB200_ERR_ARG;
     if (D <= 0 || D % 8 != 0 || D > 256) return VPPB200_ERR_DISP;
     if ((phases & 1) && (!census_l || !census_r)) return VPPB200_ERR_ARG;
@@ -656,7 +658,16 @@ extern "C" int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_
     if (!rcp_lut) rcp_lut = device_rcp_lut(st);
     if (!rcp_lut) return cuda_fail("device_rcp_lut", cudaGetLastError());
     return launch_aggregate_band(guide, census_l, census_r, cost_band, S_band, w.halo, d.Wp, d.Hp, D, row0, rows, 1, phases, state_in,
-                                 state_out, dl_band, dr_band, rcp_lut, true, prm, st);
+                                 state_out, dl_band, dr_band, rcp_lut, plain, prm, guide_ops(hints, validhints, d), st);
+}
+
+extern "C" int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                                   uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
+                                   uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
+                                   size_t workspace_bytes, void *stream, const vppb200_sgm_params *params)
+{
+    return vppb200_sgm_band_guided(guide, census_l, census_r, cost_band, S_band, H, W, C, D, row0, rows, phases, state_in, state_out,
+                                   dl_band, dr_band, rcp_lut, workspace, workspace_bytes, stream, params, nullptr, nullptr);
 }
 
 extern "C" int vppb200_sgm_band(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,

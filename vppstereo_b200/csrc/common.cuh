@@ -79,15 +79,25 @@ bool aggregate_tile_supported(int W, int H, int D, int n);
 // guided costs (<= 240)
 bool sweep_params_supported(const SgmParams &p, bool plain_costs);
 size_t tile_volume_elems(int W, int H, int D, int n);
-int launch_cost_tile(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int H, int D, int n, cudaStream_t st);
+// guided modulation of the tiled cost volume (models/rsgm/rsgm.py:115-127), fused into the cost kernel: hints / valid float32
+// [n][H][W] of the user frame (hints == NULL: plain Hamming costs); pl / pt / W / H place the user frame inside the padded one
+struct GuideOps {
+    const float *hints, *valid;
+    int pl, pt, W, H;
+};
+static inline GuideOps guide_ops(const float *hints, const float *valid, const RsgmDims &d)
+{
+    return GuideOps{hints, valid, d.pl, d.pt, d.W, d.H};
+}
+int launch_cost_tile(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int H, int D, int n, const GuideOps &gd,
+                     cudaStream_t st);
 int launch_cost_tile_band(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int Hfull, int D, int row0, int rows, int n,
-                          cudaStream_t st);
+                          const GuideOps &gd, cudaStream_t st);
 long sweep_state_words(int W, int D);
 int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full, const uint32_t *cen_r_full, uint8_t *cost8, uint16_t *S16,
                           void *halo_ws, int W, int Hfull, int D, int row0, int rows, int n, int phases, const uint32_t *state_in,
                           uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &p,
-                          cudaStream_t st);
-int launch_guided_tile(uint8_t *cost, const float *hints, const float *valid, const RsgmDims &d, int n, cudaStream_t st);
+                          const GuideOps &gd, cudaStream_t st);
 struct StageHook { void (*fn)(void *, int); void *ctx; };   // called with VPPB200_STAGE_* when that stage has been queued
 size_t sweep_halo_bytes(int W, int H, int D, int n);       // workspace of the v-sweep: inter-CTA halo lines, abort flag, P2 table
 // plain_costs: the costs are plain Hamming distances (<= 24, no guided modulation): un-normalised path state in the v-sweeps

@@ -73,9 +73,32 @@ __device__ __forceinline__ uint32_t pack4(uint32_t a, uint32_t b, uint32_t c, ui
     return a | (b << 8) | (c << 16) | (d << 24);
 }
 
-template <bool CHECK>
+// _guided_dsi (models/rsgm/rsgm.py:115-127) of one cost: numba's float64 weight 10 * (1 - exp(-(h - d)^2 / 2)) rounded to float32
+// once, cost = (uint16)((double)cost * (double)w); the arithmetic of guided_u8_kernel (rsgm_ops.cu).  Costs <= 24: the result
+// (<= 240) still fits a byte.
+__device__ __forceinline__ uint32_t guided_cost(uint32_t c, float h, int d)
+{
+    const double tt = __dsub_rn((double)h, (double)d);
+    const float w = (float)__dmul_rn(10.0, __dsub_rn(1.0, exp(__ddiv_rn(-__dmul_rn(tt, tt), 2.0))));
+    return (uint32_t)(uint8_t)(uint16_t)__dmul_rn((double)c, (double)w);
+}
+
+// the costs c[2j] (disparity k) and c[2j+1] (disparity k + K2) of the columns j whose bit is set in vm (a valid hint hv[j])
+__device__ __forceinline__ void guided_pairs(uint32_t (&c)[16], const float (&hv)[8], uint32_t vm, int k, int K2)
+{
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+        if (vm & (1u << j)) {
+            c[2 * j] = guided_cost(c[2 * j], hv[j], k);
+            c[2 * j + 1] = guided_cost(c[2 * j + 1], hv[j], k + K2);
+        }
+    }
+}
+
+// GUIDED: the costs of the columns with a valid hint (bit j of vm, hint hv[j]) are modulated before they are packed
+template <bool CHECK, bool GUIDED>
 __device__ __forceinline__ void cost_pairs(const uint32_t (&L)[8], const uint32_t *__restrict__ rp, int x, int W, int K2, int k0, int k1,
-                                           uint4 *__restrict__ out)
+                                           uint4 *__restrict__ out, const float (&hv)[8], uint32_t vm)
 {
     // word k of column x+j holds the costs of disparities k (low byte) and k + K2 (high byte):
     // wl[j] = R[x + j - k], wh[j] = R[x + j - k - K2]; both windows slide by one code per word
@@ -95,6 +118,7 @@ __device__ __forceinline__ void cost_pairs(const uint32_t (&L)[8], const uint32_
             }
             c[2 * j] = lo; c[2 * j + 1] = hi;
         }
+        if (GUIDED && vm) guided_pairs(c, hv, vm, k, K2);
         out[k * 4] = make_uint4(pack4(c[0], c[1], c[2], c[3]), pack4(c[4], c[5], c[6], c[7]), pack4(c[8], c[9], c[10], c[11]),
                                 pack4(c[12], c[13], c[14], c[15]));
 #pragma unroll
@@ -106,9 +130,13 @@ __device__ __forceinline__ void cost_pairs(const uint32_t (&L)[8], const uint32_
 
 // Row bands: cl / cr / cost point at the band's first row, t.H = rows of the band, row0 / Hfull place it in the frame (the
 // constant-12 rows are the first and last two rows of the FRAME).
+// GUIDED (_guided_dsi, models/rsgm/rsgm.py:115-127, fused: the costs are modulated in registers before the stores): every
+// padded pixel that maps into the user frame with valid > 0 -- the constant-12 rows included where they lie inside it, the tile
+// padding columns (x >= t.W) never.  A thread reads valid (and, where it is set, the hint) of its 8 columns once.
+template <bool GUIDED>
 __global__ void __launch_bounds__(256) cost_tile_kernel(const uint32_t *__restrict__ cl, const uint32_t *__restrict__ cr,
                                                         uint16_t *__restrict__ cost, TL t, long total_tiles, int row0, int Hfull,
-                                                        long census_frame_stride)
+                                                        long census_frame_stride, GuideOps gd)
 {
     const long tile = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (tile >= total_tiles) return;
@@ -126,7 +154,35 @@ __global__ void __launch_bounds__(256) cost_tile_kernel(const uint32_t *__restri
         for (int k = k0; k < k1; k++) out[k * 4] = make_uint4(0, 0, 0, 0);
         return;
     }
+    float hv[8];
+    uint32_t vm = 0;                               // bit j: column x + j has a valid hint hv[j]
+    if (GUIDED) {
+        const int yf = y - gd.pt;
+        if (yf >= 0 && yf < gd.H) {
+            const long s0 = ((row / t.H) * gd.H + yf) * (long)gd.W + (x - gd.pl);
+#pragma unroll
+            for (int j = 0; j < 8; j++) {
+                hv[j] = 0.0f;
+                const int xf = x + j - gd.pl;
+                if (xf >= 0 && xf < gd.W && gd.valid[s0 + j] > 0) {
+                    vm |= 1u << j;
+                    hv[j] = gd.hints[s0 + j];
+                }
+            }
+        }
+    }
     if (y < 2 || y >= Hfull - 2) {
+        if (GUIDED && vm) {
+            for (int k = k0; k < k1; k++) {
+                uint32_t c[16];
+#pragma unroll
+                for (int j = 0; j < 16; j++) c[j] = 12u;
+                guided_pairs(c, hv, vm, k, t.K2);
+                out[k * 4] = make_uint4(pack4(c[0], c[1], c[2], c[3]), pack4(c[4], c[5], c[6], c[7]), pack4(c[8], c[9], c[10], c[11]),
+                                        pack4(c[12], c[13], c[14], c[15]));
+            }
+            return;
+        }
         for (int k = k0; k < k1; k++) out[k * 4] = make_uint4(0x0C0C0C0Cu, 0x0C0C0C0Cu, 0x0C0C0C0Cu, 0x0C0C0C0Cu);
         return;
     }
@@ -136,52 +192,31 @@ __global__ void __launch_bounds__(256) cost_tile_kernel(const uint32_t *__restri
         L[0] = a.x; L[1] = a.y; L[2] = a.z; L[3] = a.w; L[4] = b.x; L[5] = b.y; L[6] = b.z; L[7] = b.w;
     }
     const uint32_t *rp = cr + crow;
-    if (g * 32 >= t.D + 2) cost_pairs<false>(L, rp, x, t.W, t.K2, k0, k1, out);       // every d <= x and every read inside the row
-    else cost_pairs<true>(L, rp, x, t.W, t.K2, k0, k1, out);
+    if (g * 32 >= t.D + 2) cost_pairs<false, GUIDED>(L, rp, x, t.W, t.K2, k0, k1, out, hv, vm);   // every d <= x and every read inside the row
+    else cost_pairs<true, GUIDED>(L, rp, x, t.W, t.K2, k0, k1, out, hv, vm);
 }
 
-int launch_cost_tile(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int H, int D, int n, cudaStream_t st)
+int launch_cost_tile(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int H, int D, int n, const GuideOps &gd,
+                     cudaStream_t st)
 {
-    return launch_cost_tile_band(cl, cr, cost, W, H, D, 0, H, n, st);
+    return launch_cost_tile_band(cl, cr, cost, W, H, D, 0, H, n, gd, st);
 }
-// rows [row0, row0 + rows) of frames of Hfull rows: cl / cr are the FULL census images, cost holds the band only
+// rows [row0, row0 + rows) of frames of Hfull rows: cl / cr are the FULL census images, cost holds the band only.  gd.hints ==
+// NULL: plain Hamming costs; otherwise gd.hints / gd.valid are the whole user frames (band row r is hint row row0 + r - gd.pt).
 int launch_cost_tile_band(const uint32_t *cl, const uint32_t *cr, uint8_t *cost, int W, int Hfull, int D, int row0, int rows, int n,
-                          cudaStream_t st)
+                          const GuideOps &gd, cudaStream_t st)
 {
     const TL t = make_tl(W, rows, D);
     const long tiles = (long)n * rows * t.G;
-    cost_tile_kernel<<<cdiv(tiles * 32, 256), 256, 0, st>>>(cl + (long)row0 * W, cr + (long)row0 * W, reinterpret_cast<uint16_t *>(cost), t,
-                                                            tiles, row0, Hfull, (long)W * Hfull);
+    if (gd.hints)
+        cost_tile_kernel<true><<<cdiv(tiles * 32, 256), 256, 0, st>>>(cl + (long)row0 * W, cr + (long)row0 * W,
+                                                                      reinterpret_cast<uint16_t *>(cost), t, tiles, row0, Hfull,
+                                                                      (long)W * Hfull, gd);
+    else
+        cost_tile_kernel<false><<<cdiv(tiles * 32, 256), 256, 0, st>>>(cl + (long)row0 * W, cr + (long)row0 * W,
+                                                                       reinterpret_cast<uint16_t *>(cost), t, tiles, row0, Hfull,
+                                                                       (long)W * Hfull, gd);
     VPP_LAUNCH_CHECK("cost_tile_kernel");
-    return VPPB200_OK;
-}
-
-// _guided_dsi (models/rsgm/rsgm.py:115-127) on the layout-T u8 volume; arithmetic as guided_u8_kernel (rsgm_ops.cu)
-__global__ void guided_tile_kernel(uint8_t *__restrict__ cost, const float *__restrict__ hints, const float *__restrict__ valid,
-                                   RsgmDims d, TL t, long total)
-{
-    long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= total) return;
-    const int dd = (int)(i % d.D);
-    const long px = i / d.D;
-    const int xp = (int)(px % d.Wp), yp = (int)((px / d.Wp) % d.Hp);
-    const int x = xp - d.pl, y = yp - d.pt;
-    const long f = px / ((long)d.Wp * d.Hp);
-    if (x < 0 || x >= d.W || y < 0 || y >= d.H) return;
-    const long s = (f * d.H + y) * d.W + x;
-    if (!(valid[s] > 0)) return;
-    const double tt = __dsub_rn((double)hints[s], (double)dd);
-    const float w = (float)__dmul_rn(10.0, __dsub_rn(1.0, exp(__ddiv_rn(-__dmul_rn(tt, tt), 2.0))));
-    const long word = f * t.frame + (((long)yp * t.G + xp / 32) * t.K2 + dd % t.K2) * 32 + xp % 32;
-    uint8_t *p = cost + word * 2 + (dd >= t.K2 ? 1 : 0);
-    *p = (uint8_t)(uint16_t)__dmul_rn((double)*p, (double)w);
-}
-int launch_guided_tile(uint8_t *cost, const float *hints, const float *valid, const RsgmDims &d, int n, cudaStream_t st)
-{
-    const TL t = make_tl(d.Wp, d.Hp, d.D);
-    long total = (long)n * d.Hp * d.Wp * d.D;
-    guided_tile_kernel<<<cdiv(total, 256), 256, 0, st>>>(cost, hints, valid, d, t, total);
-    VPP_LAUNCH_CHECK("guided_tile_kernel");
     return VPPB200_OK;
 }
 
@@ -1392,11 +1427,12 @@ int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S1
 // steps to queue: COST (Hamming volume of the band from the full census images) | H_FWD | V_DOWN | V_UP | H_BWD (fused with WTA).
 // The vertical sweeps continue across bands through the exported row state: V_DOWN of a band that does not start at row 0 reads
 // state_in (= state_out of the band above), V_UP of a band that does not end at the last row reads state_in (= state_out of the
-// band below); state_out == NULL: nothing is exported.  cost8 / S16 / dl / dr hold the band's rows only.
+// band below); state_out == NULL: nothing is exported.  cost8 / S16 / dl / dr hold the band's rows only.  gd: guided modulation
+// of the band's volume in COST (gd.hints == NULL: none); plain_costs must be gd.hints == NULL in every phase of the frame.
 int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full, const uint32_t *cen_r_full, uint8_t *cost8, uint16_t *S16,
                           void *halo_ws, int W, int Hfull, int D, int row0, int rows, int n, int phases, const uint32_t *state_in,
                           uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &prm,
-                          cudaStream_t st)
+                          const GuideOps &gd, cudaStream_t st)
 {
     const TL t = make_tl(W, rows, D);
     if (row0 < 0 || rows < 3 || row0 + rows > Hfull) return VPPB200_ERR_ARG;
@@ -1412,7 +1448,7 @@ int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full,
         // frames are Hfull * W apart in the guide but rows * W apart in an h-sweep's row numbering: one frame per call when banded
         return VPPB200_ERR_ARG;
     }
-    if (phases & 1) if ((rc = launch_cost_tile_band(cen_l_full, cen_r_full, cost8, W, Hfull, D, row0, rows, n, st))) return rc;
+    if (phases & 1) if ((rc = launch_cost_tile_band(cen_l_full, cen_r_full, cost8, W, Hfull, D, row0, rows, n, gd, st))) return rc;
     if (phases & 2) if ((rc = run_h(guide_band, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, st))) return rc;
     if (phases & 4) {
         const VBand b{Hfull, row0, row0 == 0 ? 1 : 0, row0 == 0 ? nullptr : state_in, state_out};

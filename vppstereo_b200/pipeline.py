@@ -5,6 +5,9 @@ batch of frames, with the images staying on the device between the two (test.py:
     disp = pipe.run_device(left_u8, right_u8, hints_f32)        # CUDA tensors in, CUDA float32 [N,H,W] out
     disp = pipe.run_host(left_pinned, right_pinned, hints_pinned)  # host tensors in, pinned host float32 out
 
+    pipe = VppRsgmPipeline(H, W, guided=True)                   # guided matching (rsgm.py:115-127) on the same hints:
+    disp = pipe.run_device(left_u8, right_u8, hints_f32, validhints=valid_f32)    # compute_rsgm(left, lv, rv, hints, validhints)
+
 Three phases of neighbouring batches run concurrently on three internal streams (software pipeline across calls):
   front(k+1) = VPP + pad/gray/census/cost volume   |   main(k) = 8-path SGM sweeps + WTA   |   tail(k-1) = median ... fills
 with two buffer sets for everything that crosses a phase boundary; the SGM sweeps alone keep the critical stream busy
@@ -21,10 +24,15 @@ from . import vpp_core_opt as _core
 
 
 class VppRsgmPipeline:
+    guided = False                                    # set per object by __init__(guided=...)
+
     def __init__(self, H, W, channels=3, batch=64, dmax=192, wsize=3, blending=0.4, c_occ=0.0, left2right=True,
-                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None):
+                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None, guided=False):
         # sgm_params: (p1, p2min, alpha, gamma) honoured by the matcher; None = the reference's effective values (7, 17, 0.25, 50)
+        # guided: the matcher is compute_rsgm(left, lv, rv, hints, validhints) -- every entry point then takes `validhints`
+        # (float32 [N,H,W], placed like `hints`).  Parameters outside the guided sweep domain run on the per-path kernels.
         self.sgm_params = None if sgm_params is None else _lib.sgm_params(*sgm_params)
+        self.guided = bool(guided)
         torch = _lib.require_cuda()
         self.torch = torch
         self.H, self.W, self.C, self.N, self.D = int(H), int(W), int(channels), int(batch), int(dmax)
@@ -58,11 +66,13 @@ class VppRsgmPipeline:
             self.front_done = [torch.cuda.Event(), torch.cuda.Event()]
             self.main_done = [None, None]
             self.tail_done = [None, None]
+            self.last_n = None                        # batch size of the latest run_device call
             self.disp = torch.empty((self.N, self.H, self.W), dtype=torch.float32, device=self.device)
             # staging for run_host
             self.d_left = torch.empty_like(self.lv)
             self.d_right = torch.empty_like(self.lv)
             self.d_hints = torch.empty((self.N, self.H, self.W), dtype=torch.float32, device=self.device)
+            self.d_valid = torch.empty_like(self.d_hints) if self.guided else None
             self.h_disp = torch.empty((self.N, self.H, self.W), dtype=torch.float32).pin_memory()
             self._stream_sets = None                  # created by the first submit_host
             self.host_depth = 3                       # staging sets of the streaming host API
@@ -99,11 +109,16 @@ class VppRsgmPipeline:
     def workspace_bytes(self):
         return self.ws_rsgm.numel() + self.ws_vpp.numel()
 
-    def _check(self, left, right, hints, out=None, host=False):
+    def _check(self, left, right, hints, out=None, host=False, validhints=None):
         """Operand validation shared by every entry point: the kernels receive raw pointers, so a wrong dtype, shape, device
         or a non-contiguous view would be read as garbage or out of bounds.  Returns the batch size."""
         torch = self.torch
-        for name, t in (("left", left), ("right", right), ("hints", hints)):
+        if self.guided and validhints is None:
+            raise ValueError("validhints: required by a guided pipeline (guided=True)")
+        if not self.guided and validhints is not None:
+            raise ValueError("validhints: given to an unguided pipeline (construct it with guided=True)")
+        ops = (("left", left), ("right", right), ("hints", hints)) + ((("validhints", validhints),) if self.guided else ())
+        for name, t in ops:
             if not isinstance(t, torch.Tensor):
                 raise TypeError(f"{name}: expected a torch tensor, got {type(t).__name__}")
         if left.dim() != 4 or tuple(left.shape[1:]) != (self.H, self.W, self.C):
@@ -113,6 +128,8 @@ class VppRsgmPipeline:
             raise ValueError(f"batch of {N} frames does not fit this pipeline (batch={self.N})")
         want = (("left", left, torch.uint8, (N, self.H, self.W, self.C)), ("right", right, torch.uint8, (N, self.H, self.W, self.C)),
                 ("hints", hints, torch.float32, (N, self.H, self.W)))
+        if self.guided:
+            want += (("validhints", validhints, torch.float32, (N, self.H, self.W)),)
         if out is not None:
             if not isinstance(out, torch.Tensor):
                 raise TypeError("out: expected a torch tensor")
@@ -144,16 +161,19 @@ class VppRsgmPipeline:
         replays the projected pattern of any frame on the host."""
         return (self.seed * 0x9E3779B97F4A7C15 + int(step)) & (2**64 - 1)
 
-    def _phase(self, phases, b, left, lv, rv, out, N, stream):
+    def _phase(self, phases, b, left, lv, rv, out, N, stream, hints, validhints):
+        # hints / validhints go to every phase of a guided batch (their nullness selects the sweeps' state); FRONT reads them
         L = self.lib
         prm = None if self.sgm_params is None else C.byref(self.sgm_params)
-        rc = L.vppb200_compute_rsgm_ex(_lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), None, None, _lib.ptr(out), self.H, self.W,
+        h, v = (_lib.ptr(hints), _lib.ptr(validhints)) if self.guided else (None, None)
+        rc = L.vppb200_compute_rsgm_ex(_lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W,
                                        self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm),
                                        C.c_size_t(self.ws_rsgm.numel()), N, C.c_void_p(stream.cuda_stream), phases, 2, b, None, prm)
         _lib.check(rc, "compute_rsgm_phases")
 
-    def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None):
+    def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None, validhints=None):
         """VPP (in copies) + compute_rsgm; all operands CUDA tensors [N,H,W,C] uint8 / [N,H,W] float32.
+        `validhints` (guided pipelines only, required there): compute_rsgm(left, lv, rv, hints, validhints).
 
         The work is queued on the pipeline's three streams (front / main / tail, see the module docstring) and the caller's
         current stream is made to wait for the result, so `out` is valid in current-stream order like the output of any
@@ -164,11 +184,11 @@ class VppRsgmPipeline:
         (`self.front_done[k & 1]` of call k).
         `step`: explicit call number for the pattern seed (default: the pipeline's own counter, 1, 2, ...)."""
         torch = self.torch
-        N = self._check(left, right, hints, out)
+        N = self._check(left, right, hints, out, validhints=validhints)
         with torch.cuda.device(self.device):
-            return self._run_device(left, right, hints, out, inputs_ready, step, N)
+            return self._run_device(left, right, hints, validhints, out, inputs_ready, step, N)
 
-    def _run_device(self, left, right, hints, out, inputs_ready, step, N):
+    def _run_device(self, left, right, hints, validhints, out, inputs_ready, step, N):
         torch, L = self.torch, self.lib
         out = self.disp[:N] if out is None else out
         caller = torch.cuda.current_stream(self.device)
@@ -184,6 +204,13 @@ class VppRsgmPipeline:
             front.wait_event(inputs_ready)
         if self.main_done[b] is not None:
             front.wait_event(self.main_done[b])          # set b (guide, cost volume) was last read by the sweeps two calls ago
+        if N != self.last_n:
+            # the matcher's workspace is laid out for the call's batch size: the buffers of a call with another N overlap both
+            # sets of the calls before it, so it starts when they have finished (no overlap across a change of N)
+            for ev in self.main_done + self.tail_done:
+                if ev is not None:
+                    front.wait_event(ev)
+        self.last_n = N
         with torch.cuda.stream(front):
             lv.copy_(left); rv.copy_(right)              # vpp() returns copies (vpp_standalone.py:397)
             rc = L.vppb200_vpp_scan_rnd(_lib.ptr(lv), _lib.ptr(rv), _lib.ptr(hints), self.W, self.H, self.C, 0, self.wsize,
@@ -191,36 +218,36 @@ class VppRsgmPipeline:
                                         0, int(self.interpolate), 1, None, None, C.c_uint64(seed), None, _lib.ptr(self.ws_vpp),
                                         C.c_size_t(self.ws_vpp.numel()), N, C.c_void_p(front.cuda_stream))
             _lib.check(rc, "vpp_scan_rnd")
-            self._phase(1, b, left, lv, rv, out, N, front)
+            self._phase(1, b, left, lv, rv, out, N, front, hints, validhints)
             self.front_done[b].record(front)
         # ---- main: the four SGM sweeps + WTA (the critical stream)
         main.wait_event(self.front_done[b])
         if self.tail_done[b] is not None:
             main.wait_event(self.tail_done[b])           # raw disparities of set b were last read by the tail two calls ago
         with torch.cuda.stream(main):
-            self._phase(2, b, left, lv, rv, out, N, main)
+            self._phase(2, b, left, lv, rv, out, N, main, hints, validhints)
             ev = torch.cuda.Event(); ev.record(main)
             self.main_done[b] = ev
         # ---- tail: everything after WTA; `out` may still be read by work the caller queued before this call
         tail.wait_stream(caller)
         tail.wait_event(self.main_done[b])
         with torch.cuda.stream(tail):
-            self._phase(4, b, left, lv, rv, out, N, tail)
+            self._phase(4, b, left, lv, rv, out, N, tail, hints, validhints)
             ev = torch.cuda.Event(); ev.record(tail)
             self.tail_done[b] = ev
         caller.wait_event(ev)
         self.lv, self.rv = self.lv2[b], self.rv2[b]     # the projected pair of the latest call
         return out
 
-    def run_device_serial(self, left, right, hints, out=None, step=None):
+    def run_device_serial(self, left, right, hints, out=None, step=None, validhints=None):
         """The same computation, everything in order on the current stream (no overlap between calls, no internal streams
         except the right-image branches): what bench.py times stage by stage."""
         torch = self.torch
-        N = self._check(left, right, hints, out)
+        N = self._check(left, right, hints, out, validhints=validhints)
         with torch.cuda.device(self.device):
-            return self._run_device_serial(left, right, hints, out, step, N)
+            return self._run_device_serial(left, right, hints, validhints, out, step, N)
 
-    def _run_device_serial(self, left, right, hints, out, step, N):
+    def _run_device_serial(self, left, right, hints, validhints, out, step, N):
         torch, L = self.torch, self.lib
         out = self.disp[:N] if out is None else out
         st = torch.cuda.current_stream(self.device)
@@ -236,21 +263,25 @@ class VppRsgmPipeline:
                                     0, int(self.interpolate), 1, None, None, C.c_uint64(seed), None, _lib.ptr(self.ws_vpp),
                                     C.c_size_t(self.ws_vpp.numel()), N, C.c_void_p(st.cuda_stream))
         _lib.check(rc, "vpp_scan_rnd")
-        self._phase(7, b, left, lv, rv, out, N, st)
+        self._phase(7, b, left, lv, rv, out, N, st, hints, validhints)
         for s in (self.vpp_stream, self.main_stream, self.tail_stream):
             s.wait_stream(st)
         self.lv, self.rv = self.lv2[b], self.rv2[b]
         return out
 
-    def run_host(self, left, right, hints):
+    def run_host(self, left, right, hints, validhints=None):
         """Host tensors (ideally pinned) in, pinned host float32 [N,H,W] out; the copies are part of the call."""
         torch = self.torch
-        N = self._check(left, right, hints, host=True)
+        N = self._check(left, right, hints, host=True, validhints=validhints)
         with torch.cuda.device(self.device):
             self.d_left[:N].copy_(left, non_blocking=True)
             self.d_right[:N].copy_(right, non_blocking=True)
             self.d_hints[:N].copy_(hints, non_blocking=True)
-            out = self.run_device(self.d_left[:N], self.d_right[:N], self.d_hints[:N])
+            dv = None
+            if self.guided:
+                dv = self.d_valid[:N]
+                dv.copy_(validhints, non_blocking=True)
+            out = self.run_device(self.d_left[:N], self.d_right[:N], self.d_hints[:N], validhints=dv)
             self.h_disp[:N].copy_(out, non_blocking=True)
             torch.cuda.current_stream(self.device).synchronize()
         return self.h_disp[:N]
@@ -264,13 +295,14 @@ class VppRsgmPipeline:
                 for _ in range(self.host_depth):
                     sets.append(dict(left=torch.empty_like(self.lv), right=torch.empty_like(self.lv),
                                      hints=torch.empty_like(self.d_hints), disp=torch.empty_like(self.disp),
+                                     valid=torch.empty_like(self.d_hints) if self.guided else None,
                                      h_disp=torch.empty((self.N, self.H, self.W), dtype=torch.float32).pin_memory(),
                                      copied_in=torch.cuda.Event(), computed=torch.cuda.Event(), copied_out=torch.cuda.Event(),
                                      busy=False))
                 self._stream_sets = dict(sets=sets, h2d=torch.cuda.Stream(self.device), d2h=torch.cuda.Stream(self.device), turn=0)
         return self._stream_sets
 
-    def submit_host(self, left, right, hints, on_computed=None):
+    def submit_host(self, left, right, hints, on_computed=None, validhints=None):
         """Queue one batch of host tensors (pinned for real overlap); returns a ticket for collect().  At most `host_depth`
         (3) batches are in flight: submitting one more first requires collecting the oldest.  Keeping two batches queued
         behind the running one lets the next batch's inputs arrive, and its front phase start, while the current sweeps run.
@@ -282,7 +314,7 @@ class VppRsgmPipeline:
         st = ss["sets"][slot]
         if st["busy"]:
             raise RuntimeError(f"submit_host: collect() the batch submitted {self.host_depth} calls ago first")
-        N = self._check(left, right, hints, host=True)
+        N = self._check(left, right, hints, host=True, validhints=validhints)
         compute = torch.cuda.current_stream(self.device)
         with torch.cuda.device(self.device):
             with torch.cuda.stream(ss["h2d"]):
@@ -290,9 +322,12 @@ class VppRsgmPipeline:
                 st["left"][:N].copy_(left, non_blocking=True)
                 st["right"][:N].copy_(right, non_blocking=True)
                 st["hints"][:N].copy_(hints, non_blocking=True)
+                if self.guided:
+                    st["valid"][:N].copy_(validhints, non_blocking=True)
                 st["copied_in"].record(ss["h2d"])
             compute.wait_event(st["copied_in"])
-            self.run_device(st["left"][:N], st["right"][:N], st["hints"][:N], out=st["disp"][:N], inputs_ready=st["copied_in"])
+            self.run_device(st["left"][:N], st["right"][:N], st["hints"][:N], out=st["disp"][:N], inputs_ready=st["copied_in"],
+                            validhints=st["valid"][:N] if self.guided else None)
             st["computed"].record(compute)
             if on_computed is not None:
                 on_computed(st["disp"][:N])
