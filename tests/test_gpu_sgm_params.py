@@ -124,8 +124,6 @@ def _params_struct(p):
 def test_ex_entry_points_refuse_bad_params(bad):
     from vppstereo_b200 import _lib
     L = _lib.lib()
-    L.vppb200_rsgm_workspace_bytes.restype = ctypes.c_size_t
-    L.vppb200_banded_workspace_bytes.restype = ctypes.c_size_t
     rsgm_args, band_args = _abi_args(L, bad)
     assert L.vppb200_compute_rsgm_ex(*rsgm_args) == _lib.ERR_ARG
     assert L.vppb200_sgm_band_ex(*band_args) == _lib.ERR_ARG

@@ -11,7 +11,6 @@ def _band_args(L, prm, hints, valid):
     buf = (ctypes.c_uint8 * 64)()
     one = ctypes.cast(buf, ctypes.c_void_p)
     H, W, C, D = 16, 32, 3, 16
-    L.vppb200_banded_workspace_bytes.restype = ctypes.c_size_t
     bws = L.vppb200_banded_workspace_bytes(H, W, C, D)
     p = None if prm is None else ctypes.byref(prm)
     h = one if hints else None

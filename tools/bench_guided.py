@@ -107,9 +107,7 @@ def main():
     if "b" not in skip:
         libs = {"this": _lib.lib()}
         if args.parent_lib:
-            libs["parent"] = ctypes.CDLL(os.path.abspath(args.parent_lib))
-        for L in libs.values():
-            L.vppb200_rsgm_workspace_bytes.restype = ctypes.c_size_t
+            libs["parent"] = _lib.bind(ctypes.CDLL(os.path.abspath(args.parent_lib)))
         need = max(L.vppb200_rsgm_workspace_bytes(H, W, C, D, B) for L in libs.values())
         ws = torch.empty(need, dtype=torch.uint8, device=dev)
         outs = {k: torch.empty((B, H, W), dtype=torch.float32, device=dev) for k in libs}

@@ -15,22 +15,6 @@ LIB_PATH = os.path.join(HERE, "libvppstereo_b200.so")
 OK = 0
 ERR_WIDTH, ERR_DISP, ERR_THREADS, ERR_UNIQUENESS, ERR_METHOD, ERR_WORKSPACE, ERR_ARG, ERR_CUDA = -1, -2, -3, -4, -5, -6, -7, -100
 
-# every symbol include/vppstereo_b200.h declares (tests check the library exports all of them)
-SYMBOLS = [
-    "vppb200_version", "vppb200_last_cuda_error", "vppb200_launch_count", "vppb200_rcp_lut_host", "vppb200_async_error",
-    "vppb200_glibc_srand", "vppb200_glibc_rand_fill", "vppb200_stage_timing", "vppb200_stage_times",
-    "vppb200_census5x5", "vppb200_cost_census5x5_xyd", "vppb200_aggregate", "vppb200_match_wta",
-    "vppb200_match_wta_right", "vppb200_subpixel_refine", "vppb200_median3x3",
-    "vppb200_rsgm_workspace_bytes", "vppb200_compute_rsgm", "vppb200_compute_rsgm_tapped",
-    "vppb200_rsgm_workspace_bytes_sets", "vppb200_compute_rsgm_phases",
-    "vppb200_vpp_workspace_bytes", "vppb200_vpp_max_dist_workspace_bytes", "vppb200_vpp_scan_rnd", "vppb200_vpp_scan_max_dist", "vppb200_vpp_scan_rnd_adaptive", "vppb200_vpp_scan_rnd_rows",
-    "vppb200_vpp_scan_max_dist_adaptive", "vppb200_bilateral_filling", "vppb200_f32chw_to_u8hwc", "vppb200_gt_reshape",
-    "vppb200_u8hwc_to_f32chw", "vppb200_set_tuning",
-    "vppb200_occlusion_workspace_bytes", "vppb200_occlusion_heuristic",
-    "vppb200_banded_workspace_bytes", "vppb200_banded_dims", "vppb200_rsgm_front_census", "vppb200_sgm_band", "vppb200_rsgm_tail",
-    "vppb200_compute_rsgm_ex", "vppb200_sgm_band_ex", "vppb200_sgm_params_fast", "vppb200_sgm_band_guided",
-]
-
 _lib = None
 
 
@@ -42,6 +26,73 @@ class RsgmTaps(C.Structure):
 class VppSgmParams(C.Structure):
     """vppb200_sgm_params: the SGM penalties a caller asks compute_rsgm to honour"""
     _fields_ = [("p1", C.c_int), ("p2min", C.c_int), ("alpha", C.c_float), ("gamma", C.c_int)]
+
+
+# The prototype of every function include/vppstereo_b200.h declares, in the header's order: name -> (restype, argtypes).
+# tests/test_abi_prototypes.py checks it against the header under this rule:
+#   int, float, double, size_t, int64_t, uint64_t, uint32_t -> their ctypes types; a const char * return -> c_char_p;
+#   const vppb200_sgm_params * -> POINTER(VppSgmParams), const vppb200_rsgm_taps * -> POINTER(RsgmTaps) (pass the struct or
+#   None: ctypes takes the reference); every other pointer -> c_void_p (device and host buffers are opaque addresses: an int,
+#   None, a c_void_p, a ctypes array or a byref(...)).
+# ctypes then converts every argument as C expects it (a Python float becomes a C float where the header says float) and
+# refuses a value of the wrong kind (a float for an int) with ctypes.ArgumentError.
+_i, _f, _d, _sz, _i64, _u64, _u32, _p = C.c_int, C.c_float, C.c_double, C.c_size_t, C.c_int64, C.c_uint64, C.c_uint32, C.c_void_p
+_taps, _prm = C.POINTER(RsgmTaps), C.POINTER(VppSgmParams)
+PROTOTYPES = {
+    # library
+    "vppb200_version": (C.c_char_p, ()),
+    "vppb200_last_cuda_error": (C.c_char_p, ()),
+    "vppb200_async_error": (_i, ()),
+    "vppb200_launch_count": (_u64, ()),
+    "vppb200_rcp_lut_host": (_i, (_p,)),
+    "vppb200_glibc_srand": (_i, (_p, _u32)),
+    "vppb200_glibc_rand_fill": (_i, (_p, _p, _i64)),
+    "vppb200_stage_timing": (_i, (_i,)),
+    "vppb200_stage_times": (_i, (_p, _p)),
+    "vppb200_set_tuning": (_i, (_i, _i)),
+    # pyrSGM operators
+    "vppb200_census5x5": (_i, (_p, _p, _i, _i, _i, _p)),
+    "vppb200_cost_census5x5_xyd": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _p)),
+    "vppb200_aggregate": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p)),
+    "vppb200_match_wta": (_i, (_p, _p, _i, _i, _i, _f, _i, _p)),
+    "vppb200_match_wta_right": (_i, (_p, _p, _i, _i, _i, _f, _i, _p)),
+    "vppb200_subpixel_refine": (_i, (_p, _p, _i, _i, _i, _i, _p, _i, _p)),
+    "vppb200_median3x3": (_i, (_p, _p, _i, _i, _i, _p)),
+    # compute_rsgm
+    "vppb200_rsgm_workspace_bytes": (_sz, (_i, _i, _i, _i, _i)),
+    "vppb200_compute_rsgm": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p)),
+    "vppb200_rsgm_workspace_bytes_sets": (_sz, (_i, _i, _i, _i, _i, _i)),
+    "vppb200_compute_rsgm_phases": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _i, _i, _i)),
+    "vppb200_compute_rsgm_tapped": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _taps)),
+    # honoured SGM parameters
+    "vppb200_compute_rsgm_ex": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _i, _i, _i, _taps, _prm)),
+    "vppb200_sgm_params_fast": (_i, (_prm, _i)),
+    # row bands
+    "vppb200_banded_workspace_bytes": (_sz, (_i, _i, _i, _i)),
+    "vppb200_banded_dims": (_i, (_i, _i, _i, _i, _p, _p, _p, _p)),
+    "vppb200_rsgm_front_census": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _sz, _p)),
+    "vppb200_sgm_band": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p)),
+    "vppb200_sgm_band_ex": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p, _prm)),
+    "vppb200_sgm_band_guided": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p, _prm, _p, _p)),
+    "vppb200_rsgm_tail": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _p, _sz, _p)),
+    # vpp_core_opt operators
+    "vppb200_vpp_workspace_bytes": (_sz, (_i, _i, _i, _i)),
+    "vppb200_vpp_scan_rnd": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _u64, _p, _p, _sz, _i, _p)),
+    "vppb200_vpp_scan_rnd_rows": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _u64, _i, _i, _p, _p, _sz, _i, _p)),
+    "vppb200_vpp_max_dist_workspace_bytes": (_sz, (_i, _i, _i, _i, _i, _i)),
+    "vppb200_vpp_scan_max_dist": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _sz, _i, _p)),
+    "vppb200_bilateral_filling": (_i, (_p, _p, _p, _i, _i, _i, _p, _d, _i, _p)),
+    "vppb200_vpp_scan_rnd_adaptive": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _u64, _p, _p, _i, _p, _p, _sz, _i, _p)),
+    "vppb200_vpp_scan_max_dist_adaptive": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _i, _p, _p, _sz, _i, _p)),
+    "vppb200_gt_reshape": (_i, (_p, _i, _i, _p, _p, _p, _sz, _p)),
+    # occlusion mask
+    "vppb200_occlusion_workspace_bytes": (_sz, (_i, _i, _i)),
+    "vppb200_occlusion_heuristic": (_i, (_p, _p, _p, _i, _i, _i, _i, _d, _d, _d, _d, _p, _sz, _i, _p)),
+    # hand-off to the networks
+    "vppb200_u8hwc_to_f32chw": (_i, (_p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p)),
+    "vppb200_f32chw_to_u8hwc": (_i, (_p, _p, _i, _i, _i, _i, _p)),
+}
+SYMBOLS = tuple(PROTOTYPES)
 
 
 def sgm_params(p1, p2min, alpha, gamma):
@@ -63,14 +114,14 @@ def sgm_params(p1, p2min, alpha, gamma):
     if not (np.isfinite(a) and a >= 0.0) or not np.isfinite(np.float32(a)):
         raise ValueError(f"alpha must be a finite number >= 0, got {alpha!r}")
     prm = VppSgmParams(vals["p1"], vals["p2min"], a, vals["gamma"])
-    if lib().vppb200_sgm_params_fast(C.byref(prm), 0) < 0:           # the library's own validation (same rules)
+    if lib().vppb200_sgm_params_fast(prm, 0) < 0:                    # the library's own validation (same rules)
         raise ValueError(f"invalid SGM parameters {(p1, p2min, alpha, gamma)}")
     return prm
 
 
 def sgm_params_fast(prm, guided=False):
     """True if the four sweeps compute these parameters (otherwise compute_rsgm falls back to the per-path kernels)."""
-    return lib().vppb200_sgm_params_fast(C.byref(prm), int(bool(guided))) == 1
+    return lib().vppb200_sgm_params_fast(prm, int(bool(guided))) == 1
 
 
 def lib():
@@ -79,18 +130,27 @@ def lib():
     if _lib is None:
         if not os.path.exists(LIB_PATH):
             raise RuntimeError(f"{LIB_PATH} not built: run `python -m vppstereo_b200.build` (there is no CPU fallback)")
-        l = C.CDLL(LIB_PATH)
-        l.vppb200_version.restype = C.c_char_p
-        l.vppb200_last_cuda_error.restype = C.c_char_p
-        l.vppb200_launch_count.restype = C.c_uint64
-        l.vppb200_rsgm_workspace_bytes.restype = C.c_size_t
-        l.vppb200_vpp_workspace_bytes.restype = C.c_size_t
-        l.vppb200_vpp_max_dist_workspace_bytes.restype = C.c_size_t
-        l.vppb200_rsgm_workspace_bytes_sets.restype = C.c_size_t
-        l.vppb200_occlusion_workspace_bytes.restype = C.c_size_t
-        l.vppb200_banded_workspace_bytes.restype = C.c_size_t
-        _lib = l
+        _lib = bind(C.CDLL(LIB_PATH))
     return _lib
+
+
+def bind(cdll):
+    """Give every PROTOTYPES entry that `cdll` exports its restype and argtypes (also for another build of the library)."""
+    for name, (restype, argtypes) in PROTOTYPES.items():
+        if hasattr(cdll, name):
+            fn = getattr(cdll, name)
+            fn.restype, fn.argtypes = restype, argtypes
+    return cdll
+
+
+def call(name, *args, what=None):
+    """Call the status-returning entry point `name` and raise through check() (message tagged `what`, default `name`) unless
+    it returns VPPB200_OK.  A wrong number of arguments raises TypeError before anything reaches C: ctypes itself only refuses
+    too few."""
+    fn = getattr(lib(), name)
+    if len(args) != len(fn.argtypes):
+        raise TypeError(f"{name} takes {len(fn.argtypes)} arguments ({len(args)} given)")
+    check(fn(*args), name if what is None else what)
 
 
 TUNE_SGM_MAX_STRIP, TUNE_SGM_SWEEP, TUNE_SGM_CLUSTERS, TUNE_VPP_ROWS, TUNE_SGM_BYTE_SUMS, TUNE_VPP_MD_WAVE, TUNE_SGM_FUSE_COST, TUNE_RCP_HOST, TUNE_SGM_V_RED = 0, 1, 2, 3, 4, 5, 6, 7, 8
@@ -102,7 +162,7 @@ _tuning = {}
 
 def set_tuning(key, value):
     """Process-wide tuning / test hook (include/vppstereo_b200.h: vppb200_set_tuning)."""
-    check(lib().vppb200_set_tuning(int(key), int(value)), "set_tuning")
+    call("vppb200_set_tuning", int(key), int(value), what="set_tuning")
     _tuning[int(key)] = int(value)
 
 
@@ -115,7 +175,7 @@ def check_async(device=None):
     """Raise if a cooperative sweep on `device` reported a timed-out hand-off since the last check (synchronises the device)."""
     torch = torch_mod()
     with torch.cuda.device(device if device is not None else torch.cuda.current_device()):
-        check(lib().vppb200_async_error(), "async_error")
+        call("vppb200_async_error", what="async_error")
 
 
 def launch_count():

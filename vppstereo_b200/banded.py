@@ -45,9 +45,10 @@ class BandedRsgm:
             raise Exception(f"Invalid dmax ({dmax}): dmax > 256")               # models/rsgm/rsgm.py:34-35
         self.subpixel = bool(subpixel)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        L = self.lib = _lib.lib()
+        L = _lib.lib()
         hp, wp, sw, vb = C.c_int(0), C.c_int(0), C.c_int64(0), C.c_int64(0)
-        _lib.check(L.vppb200_banded_dims(self.H, self.W, self.C, self.D, C.byref(hp), C.byref(wp), C.byref(sw), C.byref(vb)), "banded_dims")
+        _lib.call("vppb200_banded_dims", self.H, self.W, self.C, self.D, C.byref(hp), C.byref(wp), C.byref(sw), C.byref(vb),
+                  what="banded_dims")
         self.Hp, self.Wp, self.state_words, self.vol_row_bytes = hp.value, wp.value, sw.value, vb.value
         self.bands = self._split(int(n_bands))
         with torch.cuda.device(self.device):
@@ -94,10 +95,9 @@ class BandedRsgm:
         """pad + gray + census of the whole frame (rsgm.py:254-262, :8-28)"""
         l, lv, rv = self._images(left, left_vpp, right_vpp)
         with self.torch.cuda.device(self.device):
-            rc = self.lib.vppb200_rsgm_front_census(_lib.ptr(l), _lib.ptr(lv), _lib.ptr(rv), _lib.ptr(self.guide), _lib.ptr(self.cl),
-                                                    _lib.ptr(self.cr), self.H, self.W, self.C, self.D, _lib.ptr(self.ws),
-                                                    C.c_size_t(self.ws.numel()), _lib.stream_ptr(self.device))
-        _lib.check(rc, "rsgm_front_census")
+            _lib.call("vppb200_rsgm_front_census", _lib.ptr(l), _lib.ptr(lv), _lib.ptr(rv), _lib.ptr(self.guide), _lib.ptr(self.cl),
+                      _lib.ptr(self.cr), self.H, self.W, self.C, self.D, _lib.ptr(self.ws), self.ws.numel(),
+                      _lib.stream_ptr(self.device), what="rsgm_front_census")
 
     def run_band(self, band, phases, cost, S, state_in=None, state_out=None, stream=None, hints=None, validhints=None):
         """phases of one band (vppb200_sgm_band_guided); hints / validhints: float32 [H,W] CUDA tensors of the whole frame or both
@@ -107,14 +107,11 @@ class BandedRsgm:
         dl = self.dl[row0:row0 + rows]
         dr = self.dr[row0:row0 + rows]
         with torch.cuda.device(self.device):
-            st = _lib.stream_ptr(self.device) if stream is None else C.c_void_p(stream.cuda_stream)
-            prm = None if self.sgm_params is None else C.byref(self.sgm_params)
-            rc = self.lib.vppb200_sgm_band_guided(_lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost),
-                                                  _lib.ptr(S), self.H, self.W, self.C, self.D, row0, rows, int(phases),
-                                                  _lib.ptr(state_in), _lib.ptr(state_out), _lib.ptr(dl), _lib.ptr(dr), None,
-                                                  _lib.ptr(self.ws), C.c_size_t(self.ws.numel()), st, prm, _lib.ptr(hints),
-                                                  _lib.ptr(validhints))
-        _lib.check(rc, "sgm_band")
+            st = _lib.stream_ptr(self.device) if stream is None else stream.cuda_stream
+            _lib.call("vppb200_sgm_band_guided", _lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost),
+                      _lib.ptr(S), self.H, self.W, self.C, self.D, row0, rows, int(phases), _lib.ptr(state_in), _lib.ptr(state_out),
+                      _lib.ptr(dl), _lib.ptr(dr), None, _lib.ptr(self.ws), self.ws.numel(), st, self.sgm_params, _lib.ptr(hints),
+                      _lib.ptr(validhints), what="sgm_band")
 
     def _hints(self, hints, validhints):
         """guided matching operands (rsgm.py:115-127) as compute_rsgm takes them -> (hints, validhints) float32 [H,W] CUDA tensors,
@@ -141,10 +138,8 @@ class BandedRsgm:
         torch = self.torch
         with torch.cuda.device(self.device):
             out = torch.empty((self.H, self.W), dtype=torch.float32, device=self.device) if out is None else out
-            rc = self.lib.vppb200_rsgm_tail(_lib.ptr(self.dl), _lib.ptr(self.dr), _lib.ptr(out), self.H, self.W, self.C, self.D,
-                                            1 if self.subpixel else 0, _lib.ptr(self.ws), C.c_size_t(self.ws.numel()),
-                                            _lib.stream_ptr(self.device))
-        _lib.check(rc, "rsgm_tail")
+            _lib.call("vppb200_rsgm_tail", _lib.ptr(self.dl), _lib.ptr(self.dr), _lib.ptr(out), self.H, self.W, self.C, self.D,
+                      1 if self.subpixel else 0, _lib.ptr(self.ws), self.ws.numel(), _lib.stream_ptr(self.device), what="rsgm_tail")
         return out
 
     def compute(self, left, left_vpp, right_vpp, hints=None, validhints=None):

@@ -8,8 +8,6 @@ window / un-warp round trip (gaps of one pixel linearly filled) and the binary m
 numpy in -> numpy out; CUDA tensors ([H,W] or a batch [N,H,W]) in -> CUDA tensors out, so the mask can go straight into
 `vpp(..., g_occ=mask)` without a host hop.  Maps are float32 (what test.py passes); other dtypes are converted.
 """
-import ctypes as C
-
 from . import _lib
 
 __all__ = ["occlusion_heuristic"]
@@ -25,13 +23,11 @@ def occlusion_heuristic(dmap, rx=9, ry=7, l=2, g=0.4375, th_conf=1, th_filter=0.
     n = d.shape[0] if d.dim() == 3 else 1
     out = torch.empty_like(d)
     conf = torch.empty(d.shape, dtype=torch.uint8, device=d.device)
-    L = _lib.lib()
     with torch.cuda.device(d.device):
-        ws = _lib.workspace(L.vppb200_occlusion_workspace_bytes(H, W, n), d.device, tag="occ")
-        rc = L.vppb200_occlusion_heuristic(_lib.ptr(d), _lib.ptr(out), _lib.ptr(conf), W, H, int(rx), int(ry), C.c_double(l),
-                                           C.c_double(g), C.c_double(th_conf), C.c_double(th_filter), _lib.ptr(ws),
-                                           C.c_size_t(ws.numel()), n, _lib.stream_ptr(d.device))
-    _lib.check(rc, "occlusion_heuristic")
+        ws = _lib.workspace(_lib.lib().vppb200_occlusion_workspace_bytes(H, W, n), d.device, tag="occ")
+        _lib.call("vppb200_occlusion_heuristic", _lib.ptr(d), _lib.ptr(out), _lib.ptr(conf), W, H, int(rx), int(ry), float(l),
+                  float(g), float(th_conf), float(th_filter), _lib.ptr(ws), ws.numel(), n, _lib.stream_ptr(d.device),
+                  what="occlusion_heuristic")
     if host:
         return out.cpu().numpy(), conf.cpu().numpy()
     return out, conf

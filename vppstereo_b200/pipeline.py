@@ -17,8 +17,6 @@ run_host is the end-to-end path: host->device copies of the three inputs and the
 are part of the call.  submit_host / collect is the same path for streams of batches: the copies of batch k+1 and of
 batch k-1 ride their own CUDA streams while batch k computes (two staging sets, events between the streams).
 """
-import ctypes as C
-
 from . import _lib
 from . import vpp_core_opt as _core
 
@@ -48,7 +46,6 @@ class VppRsgmPipeline:
         self.step = 0                                 # pattern-seed counter
         self.calls = 0                                # buffer-set parity
         L = _lib.lib()
-        self.lib = L
         with torch.cuda.device(self.device):
             self.ws_rsgm = torch.empty(L.vppb200_rsgm_workspace_bytes_sets(self.H, self.W, self.C, self.D, self.N, 2),
                                        dtype=torch.uint8, device=self.device)
@@ -161,15 +158,18 @@ class VppRsgmPipeline:
         replays the projected pattern of any frame on the host."""
         return (self.seed * 0x9E3779B97F4A7C15 + int(step)) & (2**64 - 1)
 
+    def _vpp(self, lv, rv, hints, seed, N, stream):
+        # VPP of the projected-image pair lv / rv in place: rnd pattern drawn on the device from `seed`, numba arithmetic
+        _lib.call("vppb200_vpp_scan_rnd", _lib.ptr(lv), _lib.ptr(rv), _lib.ptr(hints), self.W, self.H, self.C, 0, self.wsize,
+                  self.direction, self.blending, self.c_occ, _lib.ptr(self.occ), 0, int(self.interpolate), 1, None, None, seed,
+                  None, _lib.ptr(self.ws_vpp), self.ws_vpp.numel(), N, stream.cuda_stream, what="vpp_scan_rnd")
+
     def _phase(self, phases, b, left, lv, rv, out, N, stream, hints, validhints):
         # hints / validhints go to every phase of a guided batch (their nullness selects the sweeps' state); FRONT reads them
-        L = self.lib
-        prm = None if self.sgm_params is None else C.byref(self.sgm_params)
         h, v = (_lib.ptr(hints), _lib.ptr(validhints)) if self.guided else (None, None)
-        rc = L.vppb200_compute_rsgm_ex(_lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W,
-                                       self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm),
-                                       C.c_size_t(self.ws_rsgm.numel()), N, C.c_void_p(stream.cuda_stream), phases, 2, b, None, prm)
-        _lib.check(rc, "compute_rsgm_phases")
+        _lib.call("vppb200_compute_rsgm_ex", _lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W,
+                  self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm), self.ws_rsgm.numel(), N,
+                  stream.cuda_stream, phases, 2, b, None, self.sgm_params, what="compute_rsgm_phases")
 
     def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None, validhints=None):
         """VPP (in copies) + compute_rsgm; all operands CUDA tensors [N,H,W,C] uint8 / [N,H,W] float32.
@@ -189,7 +189,7 @@ class VppRsgmPipeline:
             return self._run_device(left, right, hints, validhints, out, inputs_ready, step, N)
 
     def _run_device(self, left, right, hints, validhints, out, inputs_ready, step, N):
-        torch, L = self.torch, self.lib
+        torch = self.torch
         out = self.disp[:N] if out is None else out
         caller = torch.cuda.current_stream(self.device)
         front, main, tail = self.vpp_stream, self.main_stream, self.tail_stream
@@ -213,11 +213,7 @@ class VppRsgmPipeline:
         self.last_n = N
         with torch.cuda.stream(front):
             lv.copy_(left); rv.copy_(right)              # vpp() returns copies (vpp_standalone.py:397)
-            rc = L.vppb200_vpp_scan_rnd(_lib.ptr(lv), _lib.ptr(rv), _lib.ptr(hints), self.W, self.H, self.C, 0, self.wsize,
-                                        self.direction, C.c_double(self.blending), C.c_double(self.c_occ), _lib.ptr(self.occ),
-                                        0, int(self.interpolate), 1, None, None, C.c_uint64(seed), None, _lib.ptr(self.ws_vpp),
-                                        C.c_size_t(self.ws_vpp.numel()), N, C.c_void_p(front.cuda_stream))
-            _lib.check(rc, "vpp_scan_rnd")
+            self._vpp(lv, rv, hints, seed, N, front)
             self._phase(1, b, left, lv, rv, out, N, front, hints, validhints)
             self.front_done[b].record(front)
         # ---- main: the four SGM sweeps + WTA (the critical stream)
@@ -248,7 +244,7 @@ class VppRsgmPipeline:
             return self._run_device_serial(left, right, hints, validhints, out, step, N)
 
     def _run_device_serial(self, left, right, hints, validhints, out, step, N):
-        torch, L = self.torch, self.lib
+        torch = self.torch
         out = self.disp[:N] if out is None else out
         st = torch.cuda.current_stream(self.device)
         for s in (self.vpp_stream, self.main_stream, self.tail_stream):
@@ -258,11 +254,7 @@ class VppRsgmPipeline:
         lv, rv = self.lv2[b][:N], self.rv2[b][:N]
         seed = self._next_seed(step)
         lv.copy_(left); rv.copy_(right)
-        rc = L.vppb200_vpp_scan_rnd(_lib.ptr(lv), _lib.ptr(rv), _lib.ptr(hints), self.W, self.H, self.C, 0, self.wsize,
-                                    self.direction, C.c_double(self.blending), C.c_double(self.c_occ), _lib.ptr(self.occ),
-                                    0, int(self.interpolate), 1, None, None, C.c_uint64(seed), None, _lib.ptr(self.ws_vpp),
-                                    C.c_size_t(self.ws_vpp.numel()), N, C.c_void_p(st.cuda_stream))
-        _lib.check(rc, "vpp_scan_rnd")
+        self._vpp(lv, rv, hints, seed, N, st)
         self._phase(7, b, left, lv, rv, out, N, st, hints, validhints)
         for s in (self.vpp_stream, self.main_stream, self.tail_stream):
             s.wait_stream(st)

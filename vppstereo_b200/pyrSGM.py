@@ -6,8 +6,6 @@ Operands may be numpy arrays (copied to the device and back, so `models/rsgm/rsg
 `import vppstereo_b200.pyrSGM as pyrSGM`) or CUDA tensors (updated in place on the device, no host round-trip;
 uint16/uint32 volumes are carried as int16/int32 storage).  A leading batch dimension is accepted on every operand.
 """
-import ctypes as C
-
 import numpy as np
 
 from . import _lib
@@ -77,7 +75,7 @@ def census5x5_SSE(src, dst, width, height):
     s, _ = _lib.operand(src, np.uint8, None)
     n = _frames(s.numel(), width * height)
     d = _out_operand(dst, np.uint32, False)
-    _lib.check(_lib.lib().vppb200_census5x5(_lib.ptr(s), _lib.ptr(d), width, height, n, _lib.stream_ptr()), "census5x5_SSE")
+    _lib.call("vppb200_census5x5", _lib.ptr(s), _lib.ptr(d), width, height, n, _lib.stream_ptr(), what="census5x5_SSE")
     _writeback(dst, d, np.uint32)
 
 
@@ -90,7 +88,7 @@ def median3x3_SSE(src, dst, width, height):
     s, _ = _lib.operand(src, np.float32, None)
     n = _frames(s.numel(), width * height)
     d = _out_operand(dst, np.float32, False)
-    _lib.check(_lib.lib().vppb200_median3x3(_lib.ptr(s), _lib.ptr(d), width, height, n, _lib.stream_ptr()), "median3x3_SSE")
+    _lib.call("vppb200_median3x3", _lib.ptr(s), _lib.ptr(d), width, height, n, _lib.stream_ptr(), what="median3x3_SSE")
     _writeback(dst, d, np.float32)
 
 
@@ -108,8 +106,8 @@ def costMeasureCensus5x5_xyd_SSE(leftCensus, rightCensus, dsi, width, height, di
     cr, _ = _lib.operand(rightCensus, np.uint32, None)
     n = _frames(cl.numel(), width * height)
     d = _out_operand(dsi, np.uint16, False)
-    _lib.check(_lib.lib().vppb200_cost_census5x5_xyd(_lib.ptr(cl), _lib.ptr(cr), _lib.ptr(d), width, height, dispCount,
-                                                      numThreads, n, _lib.stream_ptr()), "costMeasureCensus5x5_xyd_SSE")
+    _lib.call("vppb200_cost_census5x5_xyd", _lib.ptr(cl), _lib.ptr(cr), _lib.ptr(d), width, height, dispCount, numThreads, n,
+              _lib.stream_ptr(), what="costMeasureCensus5x5_xyd_SSE")
     _writeback(dsi, d, np.uint16)
 
 
@@ -139,9 +137,8 @@ def aggregate_SSE(img, dsi, dsiAgg, width, height, dispCount, P1, P2min, Alpha, 
     if per != width * height:                      # colour buffer: keep the first W*H bytes of each frame
         g = g.view(n, per)[:, : width * height].contiguous()
     d = _out_operand(dsiAgg, np.uint16, False)
-    _lib.check(_lib.lib().vppb200_aggregate(_lib.ptr(g), _lib.ptr(s), _lib.ptr(d), width, height, dispCount, P1, P2min,
-                                             C.c_float(Alpha), Gamma, int(bool(honor_params)), n, _lib.stream_ptr()),
-               "aggregate_SSE")
+    _lib.call("vppb200_aggregate", _lib.ptr(g), _lib.ptr(s), _lib.ptr(d), width, height, dispCount, P1, P2min, Alpha, Gamma,
+              int(bool(honor_params)), n, _lib.stream_ptr(), what="aggregate_SSE")
     _writeback(dsiAgg, d, np.uint16)
 
 
@@ -156,8 +153,7 @@ def _wta(sym, name, dsiAgg, dispImg, width, height, dispCount, uniqueness):
     s, _ = _lib.operand(dsiAgg, np.uint16, None)
     n = _frames(s.numel(), width * height * dispCount)
     d = _out_operand(dispImg, np.float32, False)
-    fn = getattr(_lib.lib(), sym)
-    _lib.check(fn(_lib.ptr(s), _lib.ptr(d), width, height, dispCount, C.c_float(uniqueness), n, _lib.stream_ptr()), name)
+    _lib.call(sym, _lib.ptr(s), _lib.ptr(d), width, height, dispCount, uniqueness, n, _lib.stream_ptr(), what=name)
     _writeback(dispImg, d, np.float32)
 
 
@@ -188,6 +184,6 @@ def subPixelRefine(dsi, dispImg, width, height, dispCount, method, rcp_lut=None)
     n = _frames(s.numel(), width * height * dispCount)
     d = _out_operand(dispImg, np.float32, True)
     lut = _lib.np_to_dev(rcp_lut, np.float32) if rcp_lut is not None and not _lib.is_tensor(rcp_lut) else rcp_lut
-    _lib.check(_lib.lib().vppb200_subpixel_refine(_lib.ptr(s), _lib.ptr(d), width, height, dispCount, method, _lib.ptr(lut), n,
-                                                   _lib.stream_ptr()), "subPixelRefine")
+    _lib.call("vppb200_subpixel_refine", _lib.ptr(s), _lib.ptr(d), width, height, dispCount, method, _lib.ptr(lut), n,
+              _lib.stream_ptr(), what="subPixelRefine")
     _writeback(dispImg, d, np.float32)

@@ -53,8 +53,22 @@ def _prep(left, left_vpp, right_vpp, hints, validhints, dmax):
 
 
 def _params(honor_params, p1, p2min, alpha, gamma):
-    """ctypes pointer to the validated parameters (ValueError before any device work), or None = the reference's effective ones"""
-    return _lib.C.byref(_lib.sgm_params(p1, p2min, alpha, gamma)) if honor_params else None
+    """the validated parameters (ValueError before any device work), or None = the reference's effective ones"""
+    return _lib.sgm_params(p1, p2min, alpha, gamma) if honor_params else None
+
+
+def _compute(what, imgs, h, v, out, D, subpixel, rcp_lut, prm, taps):
+    """vppb200_compute_rsgm_ex, all three phases, on the images' device and its current stream; taps: None or an RsgmTaps"""
+    N, H, W, C = imgs[1].shape
+    dev = imgs[1].device
+    ws = _lib.workspace(_lib.lib().vppb200_rsgm_workspace_bytes(H, W, C, D, N), dev, "rsgm")
+    lut = None
+    if rcp_lut is not None:
+        lut = rcp_lut if _lib.is_tensor(rcp_lut) else _lib.np_to_dev(rcp_lut, np.float32)
+    with _lib.torch_mod().cuda.device(dev):
+        _lib.call("vppb200_compute_rsgm_ex", _lib.ptr(imgs[0]), _lib.ptr(imgs[1]), _lib.ptr(imgs[2]), _lib.ptr(h), _lib.ptr(v),
+                  _lib.ptr(out), H, W, C, D, 1 if subpixel else 0, _lib.ptr(lut), _lib.ptr(ws), ws.numel(), N,
+                  _lib.stream_ptr(dev), 7, 1, 0, taps, prm, what=what)
 
 
 def compute_rsgm(left, left_vpp, right_vpp, hints=None, validhints=None, dmax=192, p1=11, p2min=17, alpha=0.5, gamma=35,
@@ -69,19 +83,8 @@ def compute_rsgm(left, left_vpp, right_vpp, hints=None, validhints=None, dmax=19
     vectors recorded on another CPU)."""
     prm = _params(honor_params, p1, p2min, alpha, gamma)
     torch, was_numpy, batched, imgs, h, v, (N, H, W, C) = _prep(left, left_vpp, right_vpp, hints, validhints, int(dmax))
-    L = _lib.lib()
-    dev = imgs[1].device
-    out = torch.empty((N, H, W), dtype=torch.float32, device=dev)
-    need = L.vppb200_rsgm_workspace_bytes(H, W, C, int(dmax), N)
-    ws = _lib.workspace(need, dev, "rsgm")
-    lut = None
-    if rcp_lut is not None:
-        lut = rcp_lut if _lib.is_tensor(rcp_lut) else _lib.np_to_dev(rcp_lut, np.float32)
-    with torch.cuda.device(dev):
-        rc = L.vppb200_compute_rsgm_ex(_lib.ptr(imgs[0]), _lib.ptr(imgs[1]), _lib.ptr(imgs[2]), _lib.ptr(h), _lib.ptr(v),
-                                       _lib.ptr(out), H, W, C, int(dmax), 1 if subpixel else 0, _lib.ptr(lut), _lib.ptr(ws),
-                                       _lib.C.c_size_t(ws.numel()), N, _lib.stream_ptr(dev), 7, 1, 0, None, prm)
-    _lib.check(rc, "compute_rsgm")
+    out = torch.empty((N, H, W), dtype=torch.float32, device=imgs[1].device)
+    _compute("compute_rsgm", imgs, h, v, out, int(dmax), subpixel, rcp_lut, prm, None)
     res = out if batched else out[0]
     return res.cpu().numpy() if was_numpy else res
 
@@ -93,7 +96,6 @@ def compute_rsgm_stages(left, left_vpp, right_vpp, hints=None, validhints=None, 
     p1 .. honor_params as in compute_rsgm."""
     prm = _params(honor_params, p1, p2min, alpha, gamma)
     torch, was_numpy, batched, imgs, h, v, (N, H, W, C) = _prep(left, left_vpp, right_vpp, hints, validhints, int(dmax))
-    L = _lib.lib()
     dev = imgs[1].device
     D = int(dmax)
     pad_h, pad_w = (((H // 16) + 1) * 16 - H) % 16, (((W // 16) + 1) * 16 - W) % 16
@@ -105,16 +107,7 @@ def compute_rsgm_stages(left, left_vpp, right_vpp, hints=None, validhints=None, 
     dl = torch.empty((N, Hp, Wp), dtype=torch.float32, device=dev)
     dr = torch.empty_like(dl)
     taps = _lib.RsgmTaps(cl.data_ptr(), cr.data_ptr(), S.data_ptr(), dl.data_ptr(), dr.data_ptr())
-    need = L.vppb200_rsgm_workspace_bytes(H, W, C, D, N)
-    ws = _lib.workspace(need, dev, "rsgm")
-    lut = None
-    if rcp_lut is not None:
-        lut = rcp_lut if _lib.is_tensor(rcp_lut) else _lib.np_to_dev(rcp_lut, np.float32)
-    with torch.cuda.device(dev):
-        rc = L.vppb200_compute_rsgm_ex(_lib.ptr(imgs[0]), _lib.ptr(imgs[1]), _lib.ptr(imgs[2]), _lib.ptr(h), _lib.ptr(v),
-                                       _lib.ptr(out), H, W, C, D, 1 if subpixel else 0, _lib.ptr(lut), _lib.ptr(ws),
-                                       _lib.C.c_size_t(ws.numel()), N, _lib.stream_ptr(dev), 7, 1, 0, _lib.C.byref(taps), prm)
-    _lib.check(rc, "compute_rsgm_stages")
+    _compute("compute_rsgm_stages", imgs, h, v, out, D, subpixel, rcp_lut, prm, taps)
     torch.cuda.synchronize(dev)
     return dict(census_l=_lib.dev_to_np(cl, np.uint32), census_r=_lib.dev_to_np(cr, np.uint32),
                 dsi_agg=_lib.dev_to_np(S, np.uint16), disp_l=dl.cpu().numpy(), disp_r=dr.cpu().numpy(),

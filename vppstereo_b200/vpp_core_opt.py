@@ -31,7 +31,7 @@ def init_rand(_seed=0):
     global _state
     _state = (C.c_uint32 * 34)()
     seed = int(_seed) & 0xFFFFFFFF                # <int> cast of the Python number, then srand(unsigned)
-    _lib.check(_lib.lib().vppb200_glibc_srand(_state, C.c_uint32(seed)), "init_rand")
+    _lib.call("vppb200_glibc_srand", _state, seed, what="init_rand")
 
 
 def draw_pattern(n):
@@ -39,7 +39,7 @@ def draw_pattern(n):
     if _state is None:
         init_rand(1)
     out = np.empty(int(n), np.uint8)
-    _lib.check(_lib.lib().vppb200_glibc_rand_fill(_state, out.ctypes.data_as(C.c_void_p), C.c_int64(int(n))), "draw_pattern")
+    _lib.call("vppb200_glibc_rand_fill", _state, out.ctypes.data, int(n), what="draw_pattern")
     return out
 
 
@@ -129,7 +129,12 @@ def _scan(kind, l, r, g, width, height, channels, uniform_color, wsize, wagg, di
     filled, thr = adaptive if adaptive is not None else (None, None)
     adaptive_on = filled is not None or thr is not None
     n_thr = int(thr.shape[-1]) if thr is not None else 0
+    what = "virtual_projection_scan_" + kind
     with torch.cuda.device(dev):
+        # operands of the five scan entry points: the image / blend operands and the trailing five are the same for all of them
+        img = (_lib.ptr(lt), _lib.ptr(rt), _lib.ptr(gt), width, height, channels, int(bool(uniform_color)), wsize)
+        blend = (cc, co, _lib.ptr(ot), int(bool(discard_occluded)), int(bool(interpolate)), int(arith))
+        tail = (_lib.ptr(counts), _lib.ptr(ws), ws.numel(), n, _lib.stream_ptr(dev))
         if kind == "rnd":
             pt = ot_off = None
             if device_rng_seed is None:
@@ -148,43 +153,24 @@ def _scan(kind, l, r, g, width, height, channels, uniform_color, wsize, wagg, di
                 if pt.numel() == 0:
                     pt = torch.zeros(1, dtype=torch.uint8, device=dev)
                 ot_off = torch.from_numpy(offs).to(dev)
+            rnd = img + (direction,) + blend + (_lib.ptr(pt), _lib.ptr(ot_off), int(device_rng_seed or 0) & (2**64 - 1))
             if rows is not None:
                 if adaptive_on:
                     raise ValueError("row bands are implemented for the fixed-patch rnd scan")
-                rc = L.vppb200_vpp_scan_rnd_rows(_lib.ptr(lt), _lib.ptr(rt), _lib.ptr(gt), width, height, channels,
-                                                 int(bool(uniform_color)), wsize, direction, C.c_double(cc), C.c_double(co),
-                                                 _lib.ptr(ot), int(bool(discard_occluded)), int(bool(interpolate)), int(arith),
-                                                 _lib.ptr(pt), _lib.ptr(ot_off), C.c_uint64(int(device_rng_seed or 0) & (2**64 - 1)),
-                                                 int(rows[0]), int(rows[1]), _lib.ptr(counts), _lib.ptr(ws), C.c_size_t(ws.numel()),
-                                                 n, _lib.stream_ptr(dev))
+                _lib.call("vppb200_vpp_scan_rnd_rows", *rnd, int(rows[0]), int(rows[1]), *tail, what=what)
             elif adaptive_on:
-                rc = L.vppb200_vpp_scan_rnd_adaptive(_lib.ptr(lt), _lib.ptr(rt), _lib.ptr(gt), width, height, channels,
-                                                     int(bool(uniform_color)), wsize, direction, C.c_double(cc), C.c_double(co),
-                                                     _lib.ptr(ot), int(bool(discard_occluded)), int(bool(interpolate)), int(arith),
-                                                     _lib.ptr(pt), _lib.ptr(ot_off), C.c_uint64(int(device_rng_seed or 0) & (2**64 - 1)),
-                                                     _lib.ptr(filled), _lib.ptr(thr), n_thr, _lib.ptr(counts), _lib.ptr(ws),
-                                                     C.c_size_t(ws.numel()), n, _lib.stream_ptr(dev))
+                _lib.call("vppb200_vpp_scan_rnd_adaptive", *rnd, _lib.ptr(filled), _lib.ptr(thr), n_thr, *tail, what=what)
             else:
-                rc = L.vppb200_vpp_scan_rnd(_lib.ptr(lt), _lib.ptr(rt), _lib.ptr(gt), width, height, channels,
-                                            int(bool(uniform_color)), wsize, direction, C.c_double(cc), C.c_double(co),
-                                            _lib.ptr(ot), int(bool(discard_occluded)), int(bool(interpolate)), int(arith),
-                                            _lib.ptr(pt), _lib.ptr(ot_off), C.c_uint64(int(device_rng_seed or 0) & (2**64 - 1)),
-                                            _lib.ptr(counts), _lib.ptr(ws), C.c_size_t(ws.numel()), n, _lib.stream_ptr(dev))
-        elif adaptive_on:
-            rc = L.vppb200_vpp_scan_max_dist_adaptive(_lib.ptr(lt), _lib.ptr(rt), _lib.ptr(gt), width, height, channels,
-                                                      int(bool(uniform_color)), wsize, int(wagg[0]), int(wagg[1]), direction,
-                                                      C.c_double(cc), C.c_double(co), _lib.ptr(ot), int(bool(discard_occluded)),
-                                                      int(bool(interpolate)), int(arith), _lib.ptr(filled), _lib.ptr(thr), n_thr,
-                                                      _lib.ptr(counts), _lib.ptr(ws), C.c_size_t(ws.numel()), n, _lib.stream_ptr(dev))
-        elif rows is not None:
-            raise ValueError("maxDistance does not split into independent row bands (SURVEY.md 8e): its windows read the current images")
+                _lib.call("vppb200_vpp_scan_rnd", *rnd, *tail, what=what)
         else:
-            rc = L.vppb200_vpp_scan_max_dist(_lib.ptr(lt), _lib.ptr(rt), _lib.ptr(gt), width, height, channels,
-                                             int(bool(uniform_color)), wsize, int(wagg[0]), int(wagg[1]), direction,
-                                             C.c_double(cc), C.c_double(co), _lib.ptr(ot), int(bool(discard_occluded)),
-                                             int(bool(interpolate)), int(arith), _lib.ptr(counts), _lib.ptr(ws),
-                                             C.c_size_t(ws.numel()), n, _lib.stream_ptr(dev))
-    _lib.check(rc, "virtual_projection_scan_" + kind)
+            md = img + (int(wagg[0]), int(wagg[1]), direction) + blend
+            if adaptive_on:
+                _lib.call("vppb200_vpp_scan_max_dist_adaptive", *md, _lib.ptr(filled), _lib.ptr(thr), n_thr, *tail, what=what)
+            elif rows is not None:
+                raise ValueError("maxDistance does not split into independent row bands (SURVEY.md 8e): its windows read the current "
+                                 "images")
+            else:
+                _lib.call("vppb200_vpp_scan_max_dist", *md, *tail, what=what)
     if host:
         np.copyto(l, lt.cpu().numpy().reshape(l.shape))
         np.copyto(r, rt.cpu().numpy().reshape(r.shape))
@@ -216,14 +202,12 @@ def gt_reshape(_gt):
     if gt.dim() != 2:
         raise ValueError("Buffer has wrong number of dimensions (expected 2, got %d)" % gt.dim())
     H, W = gt.shape
-    L = _lib.lib()
     dev = gt.device
     out = torch.zeros((W * H, 4), dtype=torch.float32, device=dev)
     cnt = torch.zeros(1, dtype=torch.int32, device=dev)
-    ws = _lib.workspace(L.vppb200_vpp_workspace_bytes(H, W, 1, 1), dev, "vpp")
+    ws = _lib.workspace(_lib.lib().vppb200_vpp_workspace_bytes(H, W, 1, 1), dev, "vpp")
     with torch.cuda.device(dev):
-        rc = L.vppb200_gt_reshape(_lib.ptr(gt), W, H, _lib.ptr(out), _lib.ptr(cnt), _lib.ptr(ws), C.c_size_t(ws.numel()),
-                                  _lib.stream_ptr(dev))
-    _lib.check(rc, "gt_reshape")
+        _lib.call("vppb200_gt_reshape", _lib.ptr(gt), W, H, _lib.ptr(out), _lib.ptr(cnt), _lib.ptr(ws), ws.numel(),
+                  _lib.stream_ptr(dev), what="gt_reshape")
     res = out[: int(cnt.item())]
     return res.cpu().numpy() if host else res

@@ -8,7 +8,6 @@ reference's numba generator is never seeded by test.py (SURVEY.md 8c.5), so its 
 here the pattern comes from `pattern=` (extra keyword, uint8 stream in draw order) or from a torch generator.
 `vpp_to_network` adds the device hand-off of test.py:179-197 (uint8 HWC -> float32 CHW / 255, replicate pad).
 """
-import ctypes as C
 import functools
 import math
 
@@ -113,7 +112,6 @@ def _patch_thresholds(dmin, dmax, patch_size, gamma):
 def _adaptive_operands(lc, g, wsize, use_distance, use_bilateral, gamma, o_xy, o_i, th):
     """(filled_g or None, thresholds or None) as device tensors for the adaptive scans."""
     torch = _lib.torch_mod()
-    L = _lib.lib()
     batched = g.dim() == 3
     gg = g if batched else g[None]
     N, H, W = gg.shape
@@ -136,9 +134,8 @@ def _adaptive_operands(lc, g, wsize, use_distance, use_bilateral, gamma, o_xy, o
         wt = torch.from_numpy(_bilateral_weights(n, o_xy, o_i)).to(g.device)
         filled = torch.empty_like(gg)
         with torch.cuda.device(g.device):
-            rc = L.vppb200_bilateral_filling(_lib.ptr(gg.contiguous()), _lib.ptr(gray), _lib.ptr(filled), W, H, n, _lib.ptr(wt),
-                                             C.c_double(float(th)), N, _lib.stream_ptr(g.device))
-        _lib.check(rc, "bilateral_filling")
+            _lib.call("vppb200_bilateral_filling", _lib.ptr(gg.contiguous()), _lib.ptr(gray), _lib.ptr(filled), W, H, n, _lib.ptr(wt),
+                      float(th), N, _lib.stream_ptr(g.device), what="bilateral_filling")
     return filled, thr
 
 
@@ -158,9 +155,8 @@ def vpp_to_network(img_u8, pad_to=32):
     pl, pr, pt, pb = pad_w // 2, pad_w - pad_w // 2, pad_h // 2, pad_h - pad_h // 2
     out = torch.empty((N, Cn, H + pad_h, W + pad_w), dtype=torch.float32, device=t.device)
     with torch.cuda.device(t.device):
-        rc = _lib.lib().vppb200_u8hwc_to_f32chw(_lib.ptr(t), _lib.ptr(out), H, W, Cn, pt, pb, pl, pr, N,
-                                                 _lib.stream_ptr(t.device))
-    _lib.check(rc, "vpp_to_network")
+        _lib.call("vppb200_u8hwc_to_f32chw", _lib.ptr(t), _lib.ptr(out), H, W, Cn, pt, pb, pl, pr, N, _lib.stream_ptr(t.device),
+                  what="vpp_to_network")
     return out, (pl, pr, pt, pb)
 
 
@@ -176,8 +172,8 @@ def network_to_vpp(img_f32):
     N, Cn, H, W = t.shape
     out = torch.empty((N, H, W, Cn), dtype=torch.uint8, device=t.device)
     with torch.cuda.device(t.device):
-        rc = _lib.lib().vppb200_f32chw_to_u8hwc(_lib.ptr(t), _lib.ptr(out), H, W, Cn, N, _lib.stream_ptr(t.device))
-    _lib.check(rc, "network_to_vpp")
+        _lib.call("vppb200_f32chw_to_u8hwc", _lib.ptr(t), _lib.ptr(out), H, W, Cn, N, _lib.stream_ptr(t.device),
+                  what="network_to_vpp")
     return out[0] if single else out
 
 
