@@ -119,7 +119,8 @@ int vppb200_aggregate(const uint8_t *img, const uint16_t *dsi, uint16_t *dsi_agg
                       int P1, int P2min, float alpha, int gamma, int honor_params, int n, void *stream);
 
 /* matchWTA_SSE / matchWTARight_SSE(dsiAgg, disp f32[H,W], W, H, D, uniqueness)  RSGM/pyrSGM.cpp:296,:399,
- * StereoBMHelper.cpp:634-750,:893-1015.  First arg-min; uniqueness is validated and otherwise dead, as upstream. */
+ * StereoBMHelper.cpp:634-750,:893-1015.  First arg-min; uniqueness is validated and otherwise dead, as upstream (the _uniq
+ * variants below apply it). */
 int vppb200_match_wta(const uint16_t *dsi_agg, float *disp, int W, int H, int D, float uniqueness, int n, void *stream);
 int vppb200_match_wta_right(const uint16_t *dsi_agg, float *disp, int W, int H, int D, float uniqueness, int n, void *stream);
 
@@ -206,6 +207,29 @@ int vppb200_compute_rsgm_ex(const uint8_t *left, const uint8_t *left_vpp, const 
                             const vppb200_sgm_params *params);
 int vppb200_sgm_params_fast(const vppb200_sgm_params *params, int guided);
 
+/* ---- uniqueness ratio of the winner-takes-all (an opt-in: the reference computes its uniqueness test and then overwrites the
+ * result, RSGM/StereoBMHelper.cpp:717,:745,:981,:1009, so every other entry point keeps the plain first arg-min).
+ * Candidates of a pixel, from the final aggregated volume S: left view c[d] = S[y][x][d], end = min(D-1, x); right view
+ * c[k] = S[y][x+k][k], end = min(D-1, W-1-x).  b = the first arg-min (as without the test); c2 = min{c[d] : 0 <= d <= end,
+ * |d - b| >= 2} (the neighbours b +- 1 are part of the same minimum); f = (uint32)(1024.0f * uniqueness).  The pixel is accepted
+ * when no such d exists (end <= 1, or end == 2 with b == 1) or when 1024 * c[b] <= f * c2 (exact 32-bit arithmetic).  Accepted
+ * pixels are exactly what the plain WTA gives (left: including the sub-pixel step); a rejected pixel's raw disparity is -10.0f in
+ * both views at every column, which the rest of compute_rsgm treats as any other invalid pixel.
+ * uniqueness must be finite with 0 < uniqueness <= 1, otherwise VPPB200_ERR_UNIQUENESS before any CUDA call.  uniqueness == 1
+ * (f = 1024) accepts every pixel and runs exactly the kernels of the plain entry point.
+ *   vppb200_match_wta_uniq / vppb200_match_wta_right_uniq: vppb200_match_wta / _right with the test.
+ *   vppb200_compute_rsgm_uniq: vppb200_compute_rsgm_ex + uniqueness, read by MAIN (every phase of one batch must pass the same
+ *       value; it is validated on every call).  The work is booked on the SGM_H_BWD stage (WTA where the volume is materialised).
+ *   vppb200_sgm_band_uniq: vppb200_sgm_band_guided + uniqueness, read by phase 16. */
+int vppb200_match_wta_uniq(const uint16_t *dsi_agg, float *disp, int W, int H, int D, float uniqueness, int n, void *stream);
+int vppb200_match_wta_right_uniq(const uint16_t *dsi_agg, float *disp, int W, int H, int D, float uniqueness, int n, void *stream);
+int vppb200_compute_rsgm_uniq(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp,
+                              const float *hints, const float *validhints, float *disp_out,
+                              int H, int W, int C, int D, int flags, const float *rcp_lut,
+                              void *workspace, size_t workspace_bytes, int n, void *stream,
+                              int phases, int sets, int set, const vppb200_rsgm_taps *taps,
+                              const vppb200_sgm_params *params, float uniqueness);
+
 /* ---- one frame split into row bands over several GPUs (SURVEY.md 8e: an oversized frame) -------------------------------
  * compute_rsgm (models/rsgm/rsgm.py:250-294) as three calls so that the aggregation -- the 2.2 GB of volumes of a Middlebury
  * frame -- runs band by band on different GPUs, EXACTLY (unlike the reference's approximate StripedStereoSGM,
@@ -245,6 +269,12 @@ int vppb200_sgm_band_guided(const uint8_t *guide, const uint32_t *census_l, cons
                             uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
                             size_t workspace_bytes, void *stream, const vppb200_sgm_params *params, const float *hints,
                             const float *validhints);
+/*   vppb200_sgm_band_uniq: see the uniqueness block above. */
+int vppb200_sgm_band_uniq(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                          uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases, const uint32_t *state_in,
+                          uint32_t *state_out, float *dl_band, float *dr_band, const float *rcp_lut, void *workspace,
+                          size_t workspace_bytes, void *stream, const vppb200_sgm_params *params, const float *hints,
+                          const float *validhints, float uniqueness);
 int vppb200_rsgm_tail(float *dl, float *dr, float *disp_out, int H, int W, int C, int D, int flags, void *workspace,
                       size_t workspace_bytes, void *stream);
 

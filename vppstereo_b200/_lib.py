@@ -67,6 +67,10 @@ PROTOTYPES = {
     # honoured SGM parameters
     "vppb200_compute_rsgm_ex": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _i, _i, _i, _taps, _prm)),
     "vppb200_sgm_params_fast": (_i, (_prm, _i)),
+    # uniqueness ratio
+    "vppb200_match_wta_uniq": (_i, (_p, _p, _i, _i, _i, _f, _i, _p)),
+    "vppb200_match_wta_right_uniq": (_i, (_p, _p, _i, _i, _i, _f, _i, _p)),
+    "vppb200_compute_rsgm_uniq": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _i, _i, _i, _taps, _prm, _f)),
     # row bands
     "vppb200_banded_workspace_bytes": (_sz, (_i, _i, _i, _i)),
     "vppb200_banded_dims": (_i, (_i, _i, _i, _i, _p, _p, _p, _p)),
@@ -74,6 +78,7 @@ PROTOTYPES = {
     "vppb200_sgm_band": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p)),
     "vppb200_sgm_band_ex": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p, _prm)),
     "vppb200_sgm_band_guided": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p, _prm, _p, _p)),
+    "vppb200_sgm_band_uniq": (_i, (_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p, _prm, _p, _p, _f)),
     "vppb200_rsgm_tail": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _p, _sz, _p)),
     # vpp_core_opt operators
     "vppb200_vpp_workspace_bytes": (_sz, (_i, _i, _i, _i)),
@@ -117,6 +122,18 @@ def sgm_params(p1, p2min, alpha, gamma):
     if lib().vppb200_sgm_params_fast(prm, 0) < 0:                    # the library's own validation (same rules)
         raise ValueError(f"invalid SGM parameters {(p1, p2min, alpha, gamma)}")
     return prm
+
+
+def uniqueness(u, what="uniqueness"):
+    """The uniqueness ratio of an opt-in WTA test as float, validated on the host: TypeError (the reference's message) unless it is
+    a finite number with 0 < u <= 1 (include/vppstereo_b200.h)."""
+    try:
+        f = float(u)
+    except (TypeError, ValueError):
+        raise TypeError(f"Uniqueness must be inside ]0,1] ({u!r}, {what})") from None
+    if not (0.0 < f <= 1.0) or not (0.0 < float(np.float32(f)) <= 1.0):
+        raise TypeError(f"Uniqueness must be inside ]0,1] ({u!r}, {what})")
+    return f
 
 
 def sgm_params_fast(prm, guided=False):

@@ -27,9 +27,11 @@ PH_COST, PH_H_FWD, PH_V_DOWN, PH_V_UP, PH_H_BWD = 1, 2, 4, 8, 16
 
 
 class BandedRsgm:
-    def __init__(self, H, W, channels=3, dmax=192, n_bands=2, subpixel=True, device=None, sgm_params=None):
+    def __init__(self, H, W, channels=3, dmax=192, n_bands=2, subpixel=True, device=None, sgm_params=None, uniqueness=None):
         # sgm_params: (p1, p2min, alpha, gamma) honoured by the sweeps; None = the reference's effective values.  Bands exist on the
         # sweeps only, so parameters outside their domain (include/vppstereo_b200.h) are refused here.
+        # uniqueness: the WTA's uniqueness ratio (compute_rsgm(..., honor_uniqueness=True)); None = off
+        self.uniqueness = 1.0 if uniqueness is None else _lib.uniqueness(uniqueness, "BandedRsgm")
         self.sgm_params = None
         if sgm_params is not None:
             prm = _lib.sgm_params(*sgm_params)
@@ -108,10 +110,10 @@ class BandedRsgm:
         dr = self.dr[row0:row0 + rows]
         with torch.cuda.device(self.device):
             st = _lib.stream_ptr(self.device) if stream is None else stream.cuda_stream
-            _lib.call("vppb200_sgm_band_guided", _lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost),
+            _lib.call("vppb200_sgm_band_uniq", _lib.ptr(self.guide), _lib.ptr(self.cl), _lib.ptr(self.cr), _lib.ptr(cost),
                       _lib.ptr(S), self.H, self.W, self.C, self.D, row0, rows, int(phases), _lib.ptr(state_in), _lib.ptr(state_out),
                       _lib.ptr(dl), _lib.ptr(dr), None, _lib.ptr(self.ws), self.ws.numel(), st, self.sgm_params, _lib.ptr(hints),
-                      _lib.ptr(validhints), what="sgm_band")
+                      _lib.ptr(validhints), self.uniqueness, what="sgm_band")
 
     def _hints(self, hints, validhints):
         """guided matching operands (rsgm.py:115-127) as compute_rsgm takes them -> (hints, validhints) float32 [H,W] CUDA tensors,
@@ -168,13 +170,14 @@ class BandedRsgmDist(BandedRsgm):
     travels rank r -> r+1 (pass 0) and r -> r-1 (pass 1), the raw disparity bands go to every rank, every rank runs the (cheap,
     whole-frame) tail and returns the full disparity map.  Transfers: dist.PeerGather (peer-mapped buffers, DMA, flag words)."""
 
-    def __init__(self, H, W, channels=3, dmax=192, subpixel=True, device=None, group=None, sgm_params=None):
+    def __init__(self, H, W, channels=3, dmax=192, subpixel=True, device=None, group=None, sgm_params=None, uniqueness=None):
         import torch.distributed as dist
         from .dist import PeerGather
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
-        super().__init__(H, W, channels, dmax, n_bands=self.world, subpixel=subpixel, device=device, sgm_params=sgm_params)
+        super().__init__(H, W, channels, dmax, n_bands=self.world, subpixel=subpixel, device=device, sgm_params=sgm_params,
+                         uniqueness=uniqueness)
         if len(self.bands) != self.world:
             raise ValueError("frame too small for one band per rank")
         torch = self.torch

@@ -362,13 +362,21 @@ extern "C" int vppb200_aggregate(const uint8_t *img, const uint16_t *dsi, uint16
 
 static int check_uniq(float u) { return (u > 1.0f || u <= 0.0f) ? VPPB200_ERR_UNIQUENESS : VPPB200_OK; }
 
+// the uniqueness factor of the _uniq entry points: u finite, 0 < u <= 1 (NaN fails both comparisons); host only
+static int uniq_factor(float u, uint32_t *uf)
+{
+    if (!(u > 0.0f && u <= 1.0f)) return VPPB200_ERR_UNIQUENESS;
+    *uf = (uint32_t)(1024.0f * u);
+    return VPPB200_OK;
+}
+
 extern "C" int vppb200_match_wta(const uint16_t *S, float *disp, int W, int H, int D, float uniqueness, int n, void *stream)
 {
     int rc = check_wd(W, H, D, n);
     if (rc) return rc;
     if ((rc = check_uniq(uniqueness))) return rc;
     if (!S || !disp) return VPPB200_ERR_ARG;
-    return launch_wta_left(S, disp, W, H, D, n, (cudaStream_t)stream);
+    return launch_wta_left(S, disp, W, H, D, n, UNIQ_OFF, (cudaStream_t)stream);
 }
 
 extern "C" int vppb200_match_wta_right(const uint16_t *S, float *disp, int W, int H, int D, float uniqueness, int n, void *stream)
@@ -377,7 +385,28 @@ extern "C" int vppb200_match_wta_right(const uint16_t *S, float *disp, int W, in
     if (rc) return rc;
     if ((rc = check_uniq(uniqueness))) return rc;
     if (!S || !disp) return VPPB200_ERR_ARG;
-    return launch_wta_right(S, disp, W, H, D, n, (cudaStream_t)stream);
+    return launch_wta_right(S, disp, W, H, D, n, UNIQ_OFF, (cudaStream_t)stream);
+}
+
+extern "C" int vppb200_match_wta_uniq(const uint16_t *S, float *disp, int W, int H, int D, float uniqueness, int n, void *stream)
+{
+    uint32_t uf;
+    int rc = check_wd(W, H, D, n);
+    if (rc) return rc;
+    if ((rc = uniq_factor(uniqueness, &uf))) return rc;
+    if (!S || !disp) return VPPB200_ERR_ARG;
+    return launch_wta_left(S, disp, W, H, D, n, uf, (cudaStream_t)stream);
+}
+
+extern "C" int vppb200_match_wta_right_uniq(const uint16_t *S, float *disp, int W, int H, int D, float uniqueness, int n,
+                                            void *stream)
+{
+    uint32_t uf;
+    int rc = check_wd(W, H, D, n);
+    if (rc) return rc;
+    if ((rc = uniq_factor(uniqueness, &uf))) return rc;
+    if (!S || !disp) return VPPB200_ERR_ARG;
+    return launch_wta_right(S, disp, W, H, D, n, uf, (cudaStream_t)stream);
 }
 
 extern "C" int vppb200_subpixel_refine(const uint16_t *dsi, float *disp, int W, int H, int D, int method, const float *rcp_lut,
@@ -417,11 +446,12 @@ extern "C" size_t vppb200_rsgm_workspace_bytes_sets(int H, int W, int C, int D, 
 // and the cost volume of buffer set `set`), MAIN = 8-path aggregation + WTA (reads them, writes the raw disparities of the
 // set), TAIL = median/interpolation/LR check/speckles/fills (reads those, writes disp_out).  One call may run any subset
 // on `stream`; a caller that runs the phases of neighbouring batches on different streams orders them with events
-// (vppstereo_b200/pipeline.py).  workspace must have been sized for `sets` sets.
+// (vppstereo_b200/pipeline.py).  workspace must have been sized for `sets` sets.  uf: uniqueness factor of MAIN's WTA
+// (UNIQ_OFF = none).
 static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
                        const float *validhints, float *disp_out, int H, int W, int C, int D, int flags, const float *rcp_lut,
                        void *workspace, size_t workspace_bytes, int n, void *stream, const vppb200_rsgm_taps *taps, int phases,
-                       int sets, int set, const vppb200_sgm_params *params)
+                       int sets, int set, const vppb200_sgm_params *params, uint32_t uf)
 {
     SgmParams prm;
     if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
@@ -487,22 +517,22 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
             if (!want_volume) {
                 // the last sweep consumes the final S on the fly: WTA left (+ sub-pixel) and right come out of the aggregation
                 if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, w.dl, w.dr, rcp_lut, hints == nullptr, prm, &hook,
-                                                st)))
+                                                uf, st)))
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
             } else {
                 if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, nullptr, nullptr, nullptr, hints == nullptr, prm,
-                                                &hook, st)))
+                                                &hook, UNIQ_OFF, st)))
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
                 if ((rc = launch_s_tile_to_xyd(w.S, w.S_xyd, d.Wp, d.Hp, D, n, st))) return rc;
                 S_final = w.S_xyd;
-                if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, st))) return rc;
+                if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st))) return rc;
             }
         } else {
             if (fast_params) rc = launch_aggregate_fast(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
             else rc = launch_aggregate_generic_u8(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
             if (rc) return rc;
             tm.done(VPPB200_STAGE_SGM_H_BWD);                // the per-path fallback is booked on the last sweep's slot
-            if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, st))) return rc;
+            if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st))) return rc;
         }
         tm.done(VPPB200_STAGE_WTA);
     }
@@ -538,7 +568,7 @@ extern "C" int vppb200_compute_rsgm_tapped(const uint8_t *left, const uint8_t *l
                                            int n, void *stream, const vppb200_rsgm_taps *taps)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, taps, 7, 1, 0, nullptr);
+                       workspace_bytes, n, stream, taps, 7, 1, 0, nullptr, UNIQ_OFF);
 }
 
 extern "C" int vppb200_compute_rsgm(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
@@ -546,7 +576,7 @@ extern "C" int vppb200_compute_rsgm(const uint8_t *left, const uint8_t *left_vpp
                                     const float *rcp_lut, void *workspace, size_t workspace_bytes, int n, void *stream)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, nullptr, 7, 1, 0, nullptr);
+                       workspace_bytes, n, stream, nullptr, 7, 1, 0, nullptr, UNIQ_OFF);
 }
 
 extern "C" int vppb200_compute_rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp,
@@ -555,7 +585,7 @@ extern "C" int vppb200_compute_rsgm_phases(const uint8_t *left, const uint8_t *l
                                            int n, void *stream, int phases, int sets, int set)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, nullptr, phases, sets, set, nullptr);
+                       workspace_bytes, n, stream, nullptr, phases, sets, set, nullptr, UNIQ_OFF);
 }
 
 extern "C" int vppb200_compute_rsgm_ex(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
@@ -564,7 +594,20 @@ extern "C" int vppb200_compute_rsgm_ex(const uint8_t *left, const uint8_t *left_
                                        int sets, int set, const vppb200_rsgm_taps *taps, const vppb200_sgm_params *params)
 {
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
-                       workspace_bytes, n, stream, taps, phases, sets, set, params);
+                       workspace_bytes, n, stream, taps, phases, sets, set, params, UNIQ_OFF);
+}
+
+extern "C" int vppb200_compute_rsgm_uniq(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
+                                         const float *validhints, float *disp_out, int H, int W, int C, int D, int flags,
+                                         const float *rcp_lut, void *workspace, size_t workspace_bytes, int n, void *stream,
+                                         int phases, int sets, int set, const vppb200_rsgm_taps *taps,
+                                         const vppb200_sgm_params *params, float uniqueness)
+{
+    uint32_t uf;
+    const int rc = uniq_factor(uniqueness, &uf);
+    if (rc) return rc;
+    return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
+                       workspace_bytes, n, stream, taps, phases, sets, set, params, uf);
 }
 
 extern "C" int vppb200_sgm_params_fast(const vppb200_sgm_params *params, int guided)
@@ -635,12 +678,14 @@ extern "C" int vppb200_rsgm_front_census(const uint8_t *left, const uint8_t *lef
     return launch_census(w.gray_l, census_l, d.Wp, d.Hp, 1, st);
 }
 
-extern "C" int vppb200_sgm_band_guided(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
-                                       uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases,
-                                       const uint32_t *state_in, uint32_t *state_out, float *dl_band, float *dr_band,
-                                       const float *rcp_lut, void *workspace, size_t workspace_bytes, void *stream,
-                                       const vppb200_sgm_params *params, const float *hints, const float *validhints)
+extern "C" int vppb200_sgm_band_uniq(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                                     uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases,
+                                     const uint32_t *state_in, uint32_t *state_out, float *dl_band, float *dr_band,
+                                     const float *rcp_lut, void *workspace, size_t workspace_bytes, void *stream,
+                                     const vppb200_sgm_params *params, const float *hints, const float *validhints, float uniqueness)
 {
+    uint32_t uf;
+    if (uniq_factor(uniqueness, &uf)) return VPPB200_ERR_UNIQUENESS;
     SgmParams prm;
     if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
     if ((hints == nullptr) != (validhints == nullptr)) return VPPB200_ERR_ARG;
@@ -658,7 +703,17 @@ extern "C" int vppb200_sgm_band_guided(const uint8_t *guide, const uint32_t *cen
     if (!rcp_lut) rcp_lut = device_rcp_lut(st);
     if (!rcp_lut) return cuda_fail("device_rcp_lut", cudaGetLastError());
     return launch_aggregate_band(guide, census_l, census_r, cost_band, S_band, w.halo, d.Wp, d.Hp, D, row0, rows, 1, phases, state_in,
-                                 state_out, dl_band, dr_band, rcp_lut, plain, prm, guide_ops(hints, validhints, d), st);
+                                 state_out, dl_band, dr_band, rcp_lut, plain, prm, guide_ops(hints, validhints, d), uf, st);
+}
+
+extern "C" int vppb200_sgm_band_guided(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,
+                                       uint16_t *S_band, int H, int W, int C, int D, int row0, int rows, int phases,
+                                       const uint32_t *state_in, uint32_t *state_out, float *dl_band, float *dr_band,
+                                       const float *rcp_lut, void *workspace, size_t workspace_bytes, void *stream,
+                                       const vppb200_sgm_params *params, const float *hints, const float *validhints)
+{
+    return vppb200_sgm_band_uniq(guide, census_l, census_r, cost_band, S_band, H, W, C, D, row0, rows, phases, state_in, state_out,
+                                 dl_band, dr_band, rcp_lut, workspace, workspace_bytes, stream, params, hints, validhints, 1.0f);
 }
 
 extern "C" int vppb200_sgm_band_ex(const uint8_t *guide, const uint32_t *census_l, const uint32_t *census_r, uint8_t *cost_band,

@@ -58,6 +58,40 @@ __device__ __forceinline__ int adapt_p2(const SgmParams &p, int ip, int ipr)
     return r < p.P2min ? p.P2min : r;
 }
 
+// ---- uniqueness ratio of the winner-takes-all (opt-in; semantics in include/vppstereo_b200.h) ----------------------------
+// uf = (uint32)(1024.0f * u).  UNIQ_OFF (u = 1) accepts every pixel: the launchers then run the plain WTA instantiations.
+static constexpr uint32_t UNIQ_OFF = 1024u;
+
+// Accept the pixel whose first arg-min is key = (cost << 16 | b) over the candidates [0, end], c2 = the least cost of a rival
+// (|d - b| >= 2)?  Whether a rival exists at all is decided by b and end alone, so c2 may hold a genuine 65535 cost: 0xFFFF in
+// the callers' running minima is only the identity of min, never read as "no rival".
+__device__ __forceinline__ bool uniq_accept(uint32_t key, uint32_t c2, int end, uint32_t uf)
+{
+    const int b = (int)(key & 0xFFFFu);
+    const bool rival = end >= 3 || (end == 2 && b != 1);
+    return !rival || 1024u * (key >> 16) <= uf * c2;
+}
+
+// is candidate d a rival of the first arg-min b inside [0, end]?
+__device__ __forceinline__ bool uniq_rival(int d, int b, int end) { return d <= end && (unsigned)(d - b + 1) > 2u; }
+
+// One right-view target absorbs its candidate key = (c << 16 | k).  A target sees its candidates in descending k (it takes slot k
+// at column t + k of a sweep x = W-1 .. 0), so the least rival cost is kept online: best = the first arg-min so far (as the plain
+// WTA), fr = far | rest << 16 with far = min over absorbed k' with |k' - b| >= 2 and rest = min over the absorbed candidates but
+// the most recent, last = the most recent cost.  A new best k has only k + 1 (the most recent) as a neighbour among the absorbed
+// ones, so its far is the old rest.  Empty state: best = 0xFFFFFFFF, fr = 0xFFFFFFFF, last = 0xFFFF (absorbing the invalid key
+// 0xFFFFFFFF keeps it empty).
+__device__ __forceinline__ void uniq_absorb(uint32_t &best, uint32_t &fr, uint32_t &last, uint32_t key)
+{
+    const uint32_t c = key >> 16;
+    const bool better = key < best;
+    const bool rival = (best & 0xFFFFu) >= (key & 0xFFFFu) + 2u;
+    const uint32_t v = __vminu2(fr, (last << 16) | (rival ? c : 0xFFFFu));
+    fr = better ? ((v & 0xFFFF0000u) | (fr >> 16)) : v;
+    best = better ? key : best;
+    last = c;
+}
+
 // ---- stage launchers (defined in the .cu files, all asynchronous on `st`) -------------------------------
 int launch_pad_gray(const uint8_t *src, uint8_t *gray, const RsgmDims &d, int n, cudaStream_t st);
 int launch_pad_flatbytes(const uint8_t *src, uint8_t *guide, const RsgmDims &d, int n, cudaStream_t st);
@@ -97,13 +131,14 @@ long sweep_state_words(int W, int D);
 int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full, const uint32_t *cen_r_full, uint8_t *cost8, uint16_t *S16,
                           void *halo_ws, int W, int Hfull, int D, int row0, int rows, int n, int phases, const uint32_t *state_in,
                           uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &p,
-                          const GuideOps &gd, cudaStream_t st);
+                          const GuideOps &gd, uint32_t uf, cudaStream_t st);
 struct StageHook { void (*fn)(void *, int); void *ctx; };   // called with VPPB200_STAGE_* when that stage has been queued
 size_t sweep_halo_bytes(int W, int H, int D, int n);       // workspace of the v-sweep: inter-CTA halo lines, abort flag, P2 table
 // plain_costs: the costs are plain Hamming distances (<= 24, no guided modulation): un-normalised path state in the v-sweeps
 // p must satisfy sweep_params_supported(p, plain_costs)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost, uint16_t *S, void *halo_ws, int W, int H, int D, int n, float *dl,
-                          float *dr, const float *lut, bool plain_costs, const SgmParams &p, const StageHook *hook, cudaStream_t st);
+                          float *dr, const float *lut, bool plain_costs, const SgmParams &p, const StageHook *hook, uint32_t uf,
+                          cudaStream_t st);
 int sweep_take_abort_flag(int *out);
 int launch_s_tile_to_xyd(const uint16_t *St, uint16_t *Sx, int W, int H, int D, int n, cudaStream_t st);
 void sweep_set_max_strip(int cols);
@@ -112,9 +147,11 @@ void sweep_set_clusters(int c);
 void vpp_set_rows_kernel(int on);
 void vpp_set_md_wave(int on);
 int vpp_take_md_abort_flag(int *out);
-int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, cudaStream_t st);
-int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st);
-int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st);
+// uf: uniqueness factor (UNIQ_OFF = none)
+int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
+                           cudaStream_t st);
+int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, uint32_t uf, cudaStream_t st);
+int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, uint32_t uf, cudaStream_t st);
 int launch_subpixel(const uint16_t *S, float *disp, int W, int H, int D, int method, const float *lut, int n, cudaStream_t st);
 int launch_median(const float *src, float *dst, int W, int H, int n, cudaStream_t st);
 int launch_interp_clip(float *disp, int W, int H, int n, cudaStream_t st);   // _linear_interpolate(.,15,3) + clip>=0

@@ -441,13 +441,14 @@ int launch_guided_u8(uint8_t *dsi, const float *hints, const float *valid, const
 //          at column x' slot d holds target x'-d; after absorbing S[x'][d] every bucket moves one slot down, slot 0
 //          retires to disp_r[x'].  No atomics, no re-reads.
 //   sub-pixel (method 0, :1072-1102) optionally fused into the left result.
+//   UNIQ: the uniqueness ratio uf (common.cuh: uniq_accept; left: a second warp reduction over the rivals of the arg-min, right:
+//          the buckets carry uniq_absorb's state); a rejected pixel is -10 in both views.
 // ------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int s_at(const uint16_t *Srow, int x, int d, int D) { return Srow[(long)x * D + d]; }
 
-template <int NW, bool LEFT, bool RIGHT, bool SUBPIX>
-__global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restrict__ S, float *__restrict__ disp_l,
-                                                       float *__restrict__ disp_r, int W, int H, int D,
-                                                       const float *__restrict__ lut, long total_rows)
+template <int NW, bool LEFT, bool RIGHT, bool SUBPIX, bool UNIQ>
+__device__ __forceinline__ void wta_rows_body(const uint16_t *__restrict__ S, float *__restrict__ disp_l, float *__restrict__ disp_r,
+                                              int W, int H, int D, const float *__restrict__ lut, long total_rows, uint32_t uf)
 {
     const long row = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (row >= total_rows) return;
@@ -458,6 +459,11 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
     uint32_t bucket[2 * NW];
 #pragma unroll
     for (int k = 0; k < 2 * NW; k++) bucket[k] = 0xFFFFFFFFu;
+    uint32_t bfr[UNIQ ? 2 * NW : 1], blast[UNIQ ? 2 * NW : 1];       // UNIQ: far | rest << 16 and the most recent cost per bucket
+    if (UNIQ) {
+#pragma unroll
+        for (int k = 0; k < 2 * NW; k++) { bfr[k] = 0xFFFFFFFFu; blast[k] = 0xFFFFu; }
+    }
     const bool last_image_row = false;
     (void)last_image_row;
     for (int x = W - 1; x >= 0; x--) {
@@ -476,6 +482,13 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
 #pragma unroll
             for (int k = 0; k < 2 * NW; k++) m = min(m, (d0 + k <= end) ? key[k] : 0xFFFFFFFFu);
             m = __reduce_min_sync(0xFFFFFFFFu, m);
+            uint32_t c2 = 0xFFFFu;
+            if (UNIQ) {
+                const int b = (int)(m & 0xFFFFu);
+#pragma unroll
+                for (int k = 0; k < 2 * NW; k++) c2 = min(c2, uniq_rival(d0 + k, b, end) ? key[k] >> 16 : 0xFFFFu);
+                c2 = __reduce_min_sync(0xFFFFFFFFu, c2);
+            }
             if (lane == 0) {
                 const int best = (int)(m & 0xFFFFu);
                 float out = (float)best;
@@ -490,49 +503,95 @@ __global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restric
                         out = -10.0f;
                     }
                 }
+                if (UNIQ && !uniq_accept(m, c2, end, uf)) out = -10.0f;
                 disp_l[row * W + x] = out;
             }
         }
         if (RIGHT) {
+            if (UNIQ) {
 #pragma unroll
-            for (int k = 0; k < 2 * NW; k++) bucket[k] = min(bucket[k], key[k]);
-            if (lane == 0) disp_r[row * W + x] = (float)(bucket[0] & 0xFFFFu);
+                for (int k = 0; k < 2 * NW; k++) uniq_absorb(bucket[k], bfr[k], blast[k], key[k]);
+            } else {
+#pragma unroll
+                for (int k = 0; k < 2 * NW; k++) bucket[k] = min(bucket[k], key[k]);
+            }
+            if (lane == 0) {
+                float out = (float)(bucket[0] & 0xFFFFu);
+                if (UNIQ && !uniq_accept(bucket[0], bfr[0] & 0xFFFFu, min(D - 1, W - 1 - x), uf)) out = -10.0f;
+                disp_r[row * W + x] = out;
+            }
             // shift every bucket one disparity slot down; the top slot of the warp starts a new target
             uint32_t from_up = __shfl_down_sync(0xFFFFFFFFu, bucket[0], 1);
             if (lane == 31) from_up = 0xFFFFFFFFu;
 #pragma unroll
             for (int k = 0; k < 2 * NW - 1; k++) bucket[k] = bucket[k + 1];
             bucket[2 * NW - 1] = from_up;
+            if (UNIQ) {
+                uint32_t fr_up = __shfl_down_sync(0xFFFFFFFFu, bfr[0], 1), last_up = __shfl_down_sync(0xFFFFFFFFu, blast[0], 1);
+                if (lane == 31) { fr_up = 0xFFFFFFFFu; last_up = 0xFFFFu; }
+#pragma unroll
+                for (int k = 0; k < 2 * NW - 1; k++) { bfr[k] = bfr[k + 1]; blast[k] = blast[k + 1]; }
+                bfr[2 * NW - 1] = fr_up; blast[2 * NW - 1] = last_up;
+            }
         }
     }
 }
 
-template <bool LEFT, bool RIGHT, bool SUBPIX>
-static int launch_wta_t(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, cudaStream_t st)
+template <int NW, bool LEFT, bool RIGHT, bool SUBPIX>
+__global__ void __launch_bounds__(128) wta_rows_kernel(const uint16_t *__restrict__ S, float *__restrict__ disp_l,
+                                                       float *__restrict__ disp_r, int W, int H, int D,
+                                                       const float *__restrict__ lut, long total_rows)
+{
+    wta_rows_body<NW, LEFT, RIGHT, SUBPIX, false>(S, disp_l, disp_r, W, H, D, lut, total_rows, UNIQ_OFF);
+}
+template <int NW, bool LEFT, bool RIGHT, bool SUBPIX>
+__global__ void __launch_bounds__(128) wta_rows_uniq_kernel(const uint16_t *__restrict__ S, float *__restrict__ disp_l,
+                                                            float *__restrict__ disp_r, int W, int H, int D,
+                                                            const float *__restrict__ lut, long total_rows, uint32_t uf)
+{
+    wta_rows_body<NW, LEFT, RIGHT, SUBPIX, true>(S, disp_l, disp_r, W, H, D, lut, total_rows, uf);
+}
+
+template <bool LEFT, bool RIGHT, bool SUBPIX, bool UNIQ>
+static int launch_wta_u(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
+                        cudaStream_t st)
 {
     const long rows = (long)n * H;
     const int blocks = cdiv(rows * 32, 128);
     const int nw = (D + 63) / 64;
+#define VPP_WTA(NW)                                                                                                   \
+    if (UNIQ) wta_rows_uniq_kernel<NW, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows, uf);     \
+    else wta_rows_kernel<NW, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows);                 \
+    break
     switch (nw) {
-        case 1: wta_rows_kernel<1, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
-        case 2: wta_rows_kernel<2, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
-        case 3: wta_rows_kernel<3, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
-        default: wta_rows_kernel<4, LEFT, RIGHT, SUBPIX><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows); break;
+        case 1: VPP_WTA(1);
+        case 2: VPP_WTA(2);
+        case 3: VPP_WTA(3);
+        default: VPP_WTA(4);
     }
-    VPP_LAUNCH_CHECK("wta_rows_kernel");
+#undef VPP_WTA
+    VPP_LAUNCH_CHECK(UNIQ ? "wta_rows_uniq_kernel" : "wta_rows_kernel");
     return VPPB200_OK;
 }
-int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st)
+template <bool LEFT, bool RIGHT, bool SUBPIX>
+static int launch_wta_t(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
+                        cudaStream_t st)
 {
-    return launch_wta_t<true, false, false>(S, disp, nullptr, W, H, D, nullptr, n, st);
+    return uf < UNIQ_OFF ? launch_wta_u<LEFT, RIGHT, SUBPIX, true>(S, dl, dr, W, H, D, lut, n, uf, st)
+                         : launch_wta_u<LEFT, RIGHT, SUBPIX, false>(S, dl, dr, W, H, D, lut, n, UNIQ_OFF, st);
 }
-int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, cudaStream_t st)
+int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, uint32_t uf, cudaStream_t st)
 {
-    return launch_wta_t<false, true, false>(S, nullptr, disp, W, H, D, nullptr, n, st);
+    return launch_wta_t<true, false, false>(S, disp, nullptr, W, H, D, nullptr, n, uf, st);
 }
-int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, cudaStream_t st)
+int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, uint32_t uf, cudaStream_t st)
 {
-    return launch_wta_t<true, true, true>(S, dl, dr, W, H, D, lut, n, st);
+    return launch_wta_t<false, true, false>(S, nullptr, disp, W, H, D, nullptr, n, uf, st);
+}
+int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
+                           cudaStream_t st)
+{
+    return launch_wta_t<true, true, true>(S, dl, dr, W, H, D, lut, n, uf, st);
 }
 
 // subPixelRefine as a stand-alone operator (RSGM/StereoBMHelper.cpp:1065-1135), one thread per pixel

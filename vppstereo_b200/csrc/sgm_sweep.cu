@@ -341,21 +341,26 @@ __device__ __forceinline__ uint32_t &u4c(uint4 &v, int i) { return i == 0 ? v.x 
 // fly by the winner-takes-all step instead of being written (RSGM/StereoBMHelper.cpp:634-750 left, :893-1015 right,
 // :1072-1102 sub-pixel; same arithmetic as wta_rows_kernel in rsgm_ops.cu, which sweeps x = W-1 .. 0 like this pass).
 // FULLK: K2 == NW * 32, every lane's NW words are real disparities (no validity selects)
+// MODE 3 (opt-in): MODE 2 with the uniqueness ratio uf < UNIQ_OFF (common.cuh: uniq_accept); a rejected pixel is -10 in both
+// views.  The right conveyor carries three times the state.  uf rides in the upper half of `total_rows` (a launch has fewer than
+// 2^31 rows), so that the instantiations of MODE 0..2 keep the signature and the code they had before the opt-in existed.
 template <int NW, int MODE, int DIR, bool FULLK>
 __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__restrict__ img, const uint16_t *__restrict__ cost,
                                                             uint32_t *__restrict__ S, TL t, long total_rows,
                                                             float *__restrict__ disp_l, float *__restrict__ disp_r,
                                                             const float *__restrict__ lut, SgmParams prm)
 {
-    constexpr bool STORE = MODE == 0, WTA = MODE == 2;
+    constexpr bool STORE = MODE == 0, WTA = MODE >= 2, UNIQ = MODE == 3;
     static_assert(!WTA || DIR < 0, "the fused WTA rides the backward sweep");
     extern __shared__ __align__(16) uint8_t hsm[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const long row = (long)blockIdx.x * HWARPS + warp;
+    const uint32_t uf = UNIQ ? (uint32_t)((unsigned long)total_rows >> 32) : UNIQ_OFF;
+    if (UNIQ) total_rows &= 0xFFFFFFFFL;
     if (row >= total_rows) return;
     const int K2 = t.K2, W = t.W, D = t.D;
     // (MODE 2: dense 32-byte S rows -- two-way bank conflicts on the six 16-byte accesses per chunk, but five CTAs per SM instead of four)
-    constexpr int SROW = MODE == 2 ? HSROW_WTA : HSROW;
+    constexpr int SROW = WTA ? HSROW_WTA : HSROW;
     const int stage_b = K2 * (HCROW + SROW);
     uint8_t *base = hsm + (size_t)warp * 2 * stage_b;
     const uint8_t *irow = img + row * W;
@@ -416,6 +421,13 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
     for (int k = 0; k < NW; k++) { ba[k] = 0xFFFFFFFFu; bb[k] = 0xFFFFFFFFu; }
     int step = 0;
     uint32_t carry = 0;
+    // UNIQ: the rest of each target's state (uniq_absorb), riding the conveyor beside ba / bb: ua / ub = far | rest << 16,
+    // la / lb = the most recent cost
+    uint32_t ua[UNIQ ? NW : 1], ub[UNIQ ? NW : 1], la[UNIQ ? NW : 1], lb[UNIQ ? NW : 1];
+    if (UNIQ) {
+#pragma unroll
+        for (int k = 0; k < NW; k++) { ua[k] = 0xFFFFFFFFu; ub[k] = 0xFFFFFFFFu; la[k] = 0xFFFFu; lb[k] = 0xFFFFu; }
+    }
     for (int q = 0; q < nchunks; q++) {
         cp_async_wait<1>();
         __syncwarp();
@@ -438,8 +450,8 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
 
         // WTA: the chunk's 8 left minima (cost << 16 | d) and 8 retired right winners are parked in shared memory (uniform values,
         // one store each); the sub-pixel step is deferred to the end of the chunk, where the final S of all 8 pixels sits in the
-        // stage buffer and lanes 0..7 finish one pixel each
-        uint32_t *wout = reinterpret_cast<uint32_t *>(hsm + (size_t)HWARPS * 2 * stage_b) + warp * 16;
+        // stage buffer and lanes 0..7 finish one pixel each.  UNIQ: the least rival costs of both views follow at [16, 32).
+        uint32_t *wout = reinterpret_cast<uint32_t *>(hsm + (size_t)HWARPS * 2 * stage_b) + warp * (UNIQ ? 32 : 16);
         const bool nomask = xlo >= D - 1;             // every d <= x in this chunk: the left arg-min needs no range mask
 #pragma unroll
         for (int pp = 0; pp < 8; pp++, step++) {
@@ -492,29 +504,72 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
                 }
                 m = __reduce_min_sync(0xFFFFFFFFu, m);
                 wout[p] = m;
+                if (UNIQ) {
+                    // the least cost over the rivals of b = m & 0xFFFF: a second warp reduction
+                    const int b = (int)(m & 0xFFFFu);
+                    uint32_t r = 0xFFFFFFFFu;
+#pragma unroll
+                    for (int k = 0; k < NW; k++)
+                        if (wv[k])
+                            r = __vminu2(r, fin[k] | (uniq_rival(d0 + k, b, end) ? 0u : 0xFFFFu) |
+                                                (uniq_rival(K2 + d0 + k, b, end) ? 0u : 0xFFFF0000u));
+                    wout[16 + p] = __reduce_min_sync(0xFFFFFFFFu, min(r & 0xFFFFu, r >> 16));
+                }
                 // right: every in-flight target absorbs its disparity slot, slot d = 0 retires to disp_r[x], the conveyor moves
                 // one disparity down: within the halves by register moves, between lanes by a rotating shuffle (lane 31
                 // receives lane 0's slots: its low-half tail takes d = K2 from there, its high-half tail starts empty)
+                if (UNIQ) {
 #pragma unroll
-                for (int k = 0; k < NW; k++) { ba[k] = min(ba[k], ka[k]); bb[k] = min(bb[k], kb[k]); }
+                    for (int k = 0; k < NW; k++) { uniq_absorb(ba[k], ua[k], la[k], ka[k]); uniq_absorb(bb[k], ub[k], lb[k], kb[k]); }
+                    if (lane == 0) wout[24 + p] = ua[0] & 0xFFFFu;
+                } else {
+#pragma unroll
+                    for (int k = 0; k < NW; k++) { ba[k] = min(ba[k], ka[k]); bb[k] = min(bb[k], kb[k]); }
+                }
                 if (lane == 0) wout[8 + p] = ba[0];
                 const uint32_t fa = __shfl_sync(0xFFFFFFFFu, ba[0], (lane + 1) & 31);
                 const uint32_t fb = __shfl_sync(0xFFFFFFFFu, bb[0], (lane + 1) & 31);
+                uint32_t fua = 0, fub = 0, fla = 0, flb = 0;
+                if (UNIQ) {
+                    fua = __shfl_sync(0xFFFFFFFFu, ua[0], (lane + 1) & 31);
+                    fub = __shfl_sync(0xFFFFFFFFu, ub[0], (lane + 1) & 31);
+                    fla = __shfl_sync(0xFFFFFFFFu, la[0], (lane + 1) & 31);
+                    flb = __shfl_sync(0xFFFFFFFFu, lb[0], (lane + 1) & 31);
+#pragma unroll
+                    for (int k = 0; k < NW - 1; k++) { ua[k] = ua[k + 1]; ub[k] = ub[k + 1]; la[k] = la[k + 1]; lb[k] = lb[k + 1]; }
+                }
 #pragma unroll
                 for (int k = 0; k < NW - 1; k++) { ba[k] = ba[k + 1]; bb[k] = bb[k + 1]; }
                 if (FULLK) {
                     ba[NW - 1] = lane == 31 ? fb : fa;
                     bb[NW - 1] = lane == 31 ? 0xFFFFFFFFu : fb;
+                    if (UNIQ) {
+                        ua[NW - 1] = lane == 31 ? fub : fua;
+                        la[NW - 1] = lane == 31 ? flb : fla;
+                        ub[NW - 1] = lane == 31 ? 0xFFFFFFFFu : fub;
+                        lb[NW - 1] = lane == 31 ? 0xFFFFu : flb;
+                    }
                 } else {
                     // the lane that holds word K2-1: its low-half tail (disparity K2-1) takes over disparity K2 = lane 0's first
                     // high-half slot; slots past K2-1 stay empty
                     const uint32_t fb0 = __shfl_sync(0xFFFFFFFFu, fb, 31);          // = lane 0's bb[0] before the move
                     ba[NW - 1] = fa; bb[NW - 1] = fb;
+                    uint32_t fub0 = 0, flb0 = 0;
+                    if (UNIQ) {
+                        fub0 = __shfl_sync(0xFFFFFFFFu, fub, 31);
+                        flb0 = __shfl_sync(0xFFFFFFFFu, flb, 31);
+                        ua[NW - 1] = fua; ub[NW - 1] = fub; la[NW - 1] = fla; lb[NW - 1] = flb;
+                    }
                     if (lane >= lane_last) {
 #pragma unroll
                         for (int k = 0; k < NW; k++) {
-                            if (lane > lane_last || k > jl) { ba[k] = 0xFFFFFFFFu; bb[k] = 0xFFFFFFFFu; }
-                            else if (k == jl) { ba[k] = fb0; bb[k] = 0xFFFFFFFFu; }
+                            if (lane > lane_last || k > jl) {
+                                ba[k] = 0xFFFFFFFFu; bb[k] = 0xFFFFFFFFu;
+                                if (UNIQ) { ua[k] = 0xFFFFFFFFu; ub[k] = 0xFFFFFFFFu; la[k] = 0xFFFFu; lb[k] = 0xFFFFu; }
+                            } else if (k == jl) {
+                                ba[k] = fb0; bb[k] = 0xFFFFFFFFu;
+                                if (UNIQ) { ua[k] = fub0; la[k] = flb0; ub[k] = 0xFFFFFFFFu; lb[k] = 0xFFFFu; }
+                            }
                         }
                     }
                 }
@@ -551,8 +606,13 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
                         o = -10.0f;
                     }
                 }
+                float orr = (float)(wout[8 + lane] & 0xFFFFu);
+                if (UNIQ) {
+                    if (!uniq_accept(m, wout[16 + lane], min(D - 1, x), uf)) o = -10.0f;
+                    if (!uniq_accept(wout[8 + lane], wout[24 + lane], min(D - 1, W - 1 - x), uf)) orr = -10.0f;
+                }
                 disp_l[row * W + x] = o;
-                disp_r[row * W + x] = (float)(wout[8 + lane] & 0xFFFFu);
+                disp_r[row * W + x] = orr;
             }
             carry = __shfl_sync(0xFFFFFFFFu, s0[0].x, 0) & 0xFFFFu;         // S(d = 0) of the chunk's first column
         } else {
@@ -580,27 +640,30 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
 
 template <int NW, int MODE, int DIR>
 static int run_h_t(const uint8_t *img, const uint16_t *cost, uint32_t *S, const TL &t, int n, float *dl, float *dr,
-                   const float *lut, const SgmParams &prm, cudaStream_t st)
+                   const float *lut, const SgmParams &prm, uint32_t uf, cudaStream_t st)
 {
     const long rows = (long)n * t.H;
+    if (MODE == 3 && rows >= (1L << 31)) return VPPB200_ERR_ARG;      // uf rides in the upper half of total_rows
     const int blocks = cdiv(rows, HWARPS);
-    const size_t stage = MODE == 2 ? (size_t)t.K2 * (HCROW + HSROW_WTA) : h_stage_bytes(t.K2);
-    const size_t smem = (size_t)HWARPS * 2 * stage + (MODE == 2 ? (size_t)HWARPS * 16 * 4 : 0);
+    const size_t stage = MODE >= 2 ? (size_t)t.K2 * (HCROW + HSROW_WTA) : h_stage_bytes(t.K2);
+    const size_t smem = (size_t)HWARPS * 2 * stage + (MODE >= 2 ? (size_t)HWARPS * (MODE == 3 ? 32 : 16) * 4 : 0);
     auto kern = t.K2 == NW * 32 ? sgm_h_kernel<NW, MODE, DIR, true> : sgm_h_kernel<NW, MODE, DIR, false>;
     if (smem > 48 * 1024) VPP_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<blocks, HWARPS * 32, smem, st>>>(img, cost, S, t, rows, dl, dr, lut, prm);
+    kern<<<blocks, HWARPS * 32, smem, st>>>(img, cost, S, t, MODE == 3 ? rows | (long)uf << 32 : rows, dl, dr, lut, prm);
     VPP_LAUNCH_CHECK("sgm_h_kernel");
     return VPPB200_OK;
 }
 
-// mode 0: forward sweep, S = L;  mode 1: backward sweep, S += L;  mode 2: backward sweep fused with WTA (dl, dr, lut)
+// mode 0: forward sweep, S = L;  mode 1: backward sweep, S += L;  mode 2: backward sweep fused with WTA (dl, dr, lut), with the
+// uniqueness ratio (mode 3) when uf < UNIQ_OFF
 static int run_h(const uint8_t *img, const uint16_t *cost, uint32_t *S, const TL &t, int mode, int n, float *dl, float *dr,
-                 const float *lut, const SgmParams &prm, cudaStream_t st)
+                 const float *lut, const SgmParams &prm, uint32_t uf, cudaStream_t st)
 {
 #define VPP_RUN_H(NW)                                                                                                  \
-    return mode == 0 ? run_h_t<NW, 0, 1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, st)                       \
-         : mode == 1 ? run_h_t<NW, 1, -1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, st)                      \
-                     : run_h_t<NW, 2, -1>(img, cost, S, t, n, dl, dr, lut, prm, st)
+    return mode == 0 ? run_h_t<NW, 0, 1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, UNIQ_OFF, st)             \
+         : mode == 1 ? run_h_t<NW, 1, -1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, UNIQ_OFF, st)            \
+         : uf < UNIQ_OFF ? run_h_t<NW, 3, -1>(img, cost, S, t, n, dl, dr, lut, prm, uf, st)                            \
+                         : run_h_t<NW, 2, -1>(img, cost, S, t, n, dl, dr, lut, prm, UNIQ_OFF, st)
     switch ((t.K2 + 31) / 32) {
         case 1: VPP_RUN_H(1);
         case 2: VPP_RUN_H(2);
@@ -1393,7 +1456,7 @@ static bool v_norm(bool plain_costs, int H, const SgmParams &p)
 // 6.78 ms: step 22.3 vs 22.0 ms.)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S16, void *halo_ws, int W, int H, int D, int n,
                           float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &prm, const StageHook *hook,
-                          cudaStream_t st)
+                          uint32_t uf, cudaStream_t st)
 {
     if (!sweep_params_supported(prm, plain_costs)) return VPPB200_ERR_ARG;
     const TL t = make_tl(W, H, D);
@@ -1411,13 +1474,13 @@ int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S1
                       sp.p2, norm, prm, st);
         return r;
     };
-    if ((rc = run_h(img, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, st))) return rc;
+    if ((rc = run_h(img, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, UNIQ_OFF, st))) return rc;
     done(VPPB200_STAGE_SGM_H_FWD);
     if ((rc = sweep(0))) return rc;
     done(VPPB200_STAGE_SGM_V_DOWN);
     if ((rc = sweep(1))) return rc;
     done(VPPB200_STAGE_SGM_V_UP);
-    if ((rc = run_h(img, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, st))) return rc;
+    if ((rc = run_h(img, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, uf, st))) return rc;
     done(VPPB200_STAGE_SGM_H_BWD);
     return VPPB200_OK;
 }
@@ -1432,7 +1495,7 @@ int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S1
 int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full, const uint32_t *cen_r_full, uint8_t *cost8, uint16_t *S16,
                           void *halo_ws, int W, int Hfull, int D, int row0, int rows, int n, int phases, const uint32_t *state_in,
                           uint32_t *state_out, float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &prm,
-                          const GuideOps &gd, cudaStream_t st)
+                          const GuideOps &gd, uint32_t uf, cudaStream_t st)
 {
     const TL t = make_tl(W, rows, D);
     if (row0 < 0 || rows < 3 || row0 + rows > Hfull) return VPPB200_ERR_ARG;
@@ -1449,7 +1512,7 @@ int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full,
         return VPPB200_ERR_ARG;
     }
     if (phases & 1) if ((rc = launch_cost_tile_band(cen_l_full, cen_r_full, cost8, W, Hfull, D, row0, rows, n, gd, st))) return rc;
-    if (phases & 2) if ((rc = run_h(guide_band, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, st))) return rc;
+    if (phases & 2) if ((rc = run_h(guide_band, cost, S, t, 0, n, nullptr, nullptr, nullptr, prm, UNIQ_OFF, st))) return rc;
     if (phases & 4) {
         const VBand b{Hfull, row0, row0 == 0 ? 1 : 0, row0 == 0 ? nullptr : state_in, state_out};
         if (!b.pass_start && !state_in) return VPPB200_ERR_ARG;
@@ -1461,7 +1524,7 @@ int launch_aggregate_band(const uint8_t *guide_full, const uint32_t *cen_l_full,
         if (!b.pass_start && !state_in) return VPPB200_ERR_ARG;
         if ((rc = run_v(guide_full, cost, S, halo_ws, t, 1, n, plan, norm, prm, st, &b))) return rc;
     }
-    if (phases & 16) if ((rc = run_h(guide_band, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, st))) return rc;
+    if (phases & 16) if ((rc = run_h(guide_band, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, uf, st))) return rc;
     return VPPB200_OK;
 }
 

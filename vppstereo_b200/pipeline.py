@@ -25,11 +25,13 @@ class VppRsgmPipeline:
     guided = False                                    # set per object by __init__(guided=...)
 
     def __init__(self, H, W, channels=3, batch=64, dmax=192, wsize=3, blending=0.4, c_occ=0.0, left2right=True,
-                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None, guided=False):
+                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None, guided=False, uniqueness=None):
         # sgm_params: (p1, p2min, alpha, gamma) honoured by the matcher; None = the reference's effective values (7, 17, 0.25, 50)
         # guided: the matcher is compute_rsgm(left, lv, rv, hints, validhints) -- every entry point then takes `validhints`
         # (float32 [N,H,W], placed like `hints`).  Parameters outside the guided sweep domain run on the per-path kernels.
+        # uniqueness: the WTA's uniqueness ratio, compute_rsgm(..., uniqueness=u, honor_uniqueness=True); None = off
         self.sgm_params = None if sgm_params is None else _lib.sgm_params(*sgm_params)
+        self.uniqueness = 1.0 if uniqueness is None else _lib.uniqueness(uniqueness, "VppRsgmPipeline")
         self.guided = bool(guided)
         torch = _lib.require_cuda()
         self.torch = torch
@@ -167,9 +169,9 @@ class VppRsgmPipeline:
     def _phase(self, phases, b, left, lv, rv, out, N, stream, hints, validhints):
         # hints / validhints go to every phase of a guided batch (their nullness selects the sweeps' state); FRONT reads them
         h, v = (_lib.ptr(hints), _lib.ptr(validhints)) if self.guided else (None, None)
-        _lib.call("vppb200_compute_rsgm_ex", _lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W,
+        _lib.call("vppb200_compute_rsgm_uniq", _lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W,
                   self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm), self.ws_rsgm.numel(), N,
-                  stream.cuda_stream, phases, 2, b, None, self.sgm_params, what="compute_rsgm_phases")
+                  stream.cuda_stream, phases, 2, b, None, self.sgm_params, self.uniqueness, what="compute_rsgm_phases")
 
     def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None, validhints=None):
         """VPP (in copies) + compute_rsgm; all operands CUDA tensors [N,H,W,C] uint8 / [N,H,W] float32.

@@ -142,7 +142,10 @@ def aggregate_SSE(img, dsi, dsiAgg, width, height, dispCount, P1, P2min, Alpha, 
     _writeback(dsiAgg, d, np.uint16)
 
 
-def _wta(sym, name, dsiAgg, dispImg, width, height, dispCount, uniqueness):
+def _wta(sym, name, dsiAgg, dispImg, width, height, dispCount, uniqueness, honor_uniqueness):
+    if honor_uniqueness:
+        uniqueness = _lib.uniqueness(uniqueness, name)           # finite, 0 < u <= 1 (NaN included)
+        sym += "_uniq"
     width, height, dispCount, uniqueness = int(width), int(height), int(dispCount), float(uniqueness)
     if width % 16 != 0:
         raise TypeError(f"Width must be a multiple of 16 ({width}x{height})")
@@ -158,15 +161,18 @@ def _wta(sym, name, dsiAgg, dispImg, width, height, dispCount, uniqueness):
 
 
 @_on_operand_device
-def matchWTA_SSE(dsiAgg, dispImg, width, height, dispCount, uniqueness):
-    """matchWTA_SSE(dsiAgg u16, disp f32[H,W], W, H, D, uniqueness)  RSGM/pyrSGM.cpp:296-397"""
-    _wta("vppb200_match_wta", "matchWTA_SSE", dsiAgg, dispImg, width, height, dispCount, uniqueness)
+def matchWTA_SSE(dsiAgg, dispImg, width, height, dispCount, uniqueness, honor_uniqueness=False):
+    """matchWTA_SSE(dsiAgg u16, disp f32[H,W], W, H, D, uniqueness)  RSGM/pyrSGM.cpp:296-397.
+    As upstream, uniqueness is validated and then has no effect unless the extra keyword honor_uniqueness=True is given: then a
+    pixel whose best cost is not below uniqueness times its best rival's (include/vppstereo_b200.h) gets -10."""
+    _wta("vppb200_match_wta", "matchWTA_SSE", dsiAgg, dispImg, width, height, dispCount, uniqueness, honor_uniqueness)
 
 
 @_on_operand_device
-def matchWTARight_SSE(dsiAgg, dispImg, width, height, dispCount, uniqueness):
-    """matchWTARight_SSE(dsiAgg u16, disp f32[H,W], W, H, D, uniqueness)  RSGM/pyrSGM.cpp:399-502"""
-    _wta("vppb200_match_wta_right", "matchWTARight_SSE", dsiAgg, dispImg, width, height, dispCount, uniqueness)
+def matchWTARight_SSE(dsiAgg, dispImg, width, height, dispCount, uniqueness, honor_uniqueness=False):
+    """matchWTARight_SSE(dsiAgg u16, disp f32[H,W], W, H, D, uniqueness)  RSGM/pyrSGM.cpp:399-502; honor_uniqueness as in
+    matchWTA_SSE."""
+    _wta("vppb200_match_wta_right", "matchWTARight_SSE", dsiAgg, dispImg, width, height, dispCount, uniqueness, honor_uniqueness)
 
 
 @_on_operand_device

@@ -57,8 +57,9 @@ def _params(honor_params, p1, p2min, alpha, gamma):
     return _lib.sgm_params(p1, p2min, alpha, gamma) if honor_params else None
 
 
-def _compute(what, imgs, h, v, out, D, subpixel, rcp_lut, prm, taps):
-    """vppb200_compute_rsgm_ex, all three phases, on the images' device and its current stream; taps: None or an RsgmTaps"""
+def _compute(what, imgs, h, v, out, D, subpixel, rcp_lut, prm, taps, uniq):
+    """vppb200_compute_rsgm_uniq, all three phases, on the images' device and its current stream; taps: None or an RsgmTaps;
+    uniq: the validated uniqueness ratio, 1.0 = none"""
     N, H, W, C = imgs[1].shape
     dev = imgs[1].device
     ws = _lib.workspace(_lib.lib().vppb200_rsgm_workspace_bytes(H, W, C, D, N), dev, "rsgm")
@@ -66,35 +67,44 @@ def _compute(what, imgs, h, v, out, D, subpixel, rcp_lut, prm, taps):
     if rcp_lut is not None:
         lut = rcp_lut if _lib.is_tensor(rcp_lut) else _lib.np_to_dev(rcp_lut, np.float32)
     with _lib.torch_mod().cuda.device(dev):
-        _lib.call("vppb200_compute_rsgm_ex", _lib.ptr(imgs[0]), _lib.ptr(imgs[1]), _lib.ptr(imgs[2]), _lib.ptr(h), _lib.ptr(v),
+        _lib.call("vppb200_compute_rsgm_uniq", _lib.ptr(imgs[0]), _lib.ptr(imgs[1]), _lib.ptr(imgs[2]), _lib.ptr(h), _lib.ptr(v),
                   _lib.ptr(out), H, W, C, D, 1 if subpixel else 0, _lib.ptr(lut), _lib.ptr(ws), ws.numel(), N,
-                  _lib.stream_ptr(dev), 7, 1, 0, taps, prm, what=what)
+                  _lib.stream_ptr(dev), 7, 1, 0, taps, prm, uniq, what=what)
+
+
+def _uniq(honor_uniqueness, uniqueness, what):
+    """the validated uniqueness ratio (TypeError before any device work), or 1.0 = the reference's plain first arg-min"""
+    return _lib.uniqueness(uniqueness, what) if honor_uniqueness else 1.0
 
 
 def compute_rsgm(left, left_vpp, right_vpp, hints=None, validhints=None, dmax=192, p1=11, p2min=17, alpha=0.5, gamma=35,
-                 uniqueness=0.95, subpixel=True, rcp_lut=None, honor_params=False):
+                 uniqueness=0.95, subpixel=True, rcp_lut=None, honor_params=False, honor_uniqueness=False):
     """compute_rsgm(...) -> float32 [H,W] disparity  (models/rsgm/rsgm.py:250-294).
 
-    p1, p2min, alpha, gamma and uniqueness are accepted for signature compatibility and have no effect, exactly as in
+    p1, p2min, alpha, gamma and uniqueness are accepted for signature compatibility and have no effect by default, exactly as in
     the reference (RSGM/pyrSGM.cpp:519 vs :557-560; StereoBMHelper.cpp:717,:745).  `honor_params=True` (extra) makes p1, p2min,
     alpha and gamma take effect (the keyword of pyrSGM.aggregate_SSE; ValueError for values outside 0..65535 or a negative or
     non-finite alpha).  Parameters outside the sweeps' domain (include/vppstereo_b200.h) are computed exactly but by slower
-    per-path kernels.  `rcp_lut` (extra, optional) overrides the host-CPU RCPSS table used by the sub-pixel step (for golden
+    per-path kernels.  `honor_uniqueness=True` (extra, independent of honor_params) makes uniqueness take effect in both WTA views:
+    a pixel whose best cost is not within uniqueness of its best rival's is invalid (-10 before the tail; TypeError unless
+    0 < uniqueness <= 1).  `rcp_lut` (extra, optional) overrides the host-CPU RCPSS table used by the sub-pixel step (for golden
     vectors recorded on another CPU)."""
     prm = _params(honor_params, p1, p2min, alpha, gamma)
+    uq = _uniq(honor_uniqueness, uniqueness, "compute_rsgm")
     torch, was_numpy, batched, imgs, h, v, (N, H, W, C) = _prep(left, left_vpp, right_vpp, hints, validhints, int(dmax))
     out = torch.empty((N, H, W), dtype=torch.float32, device=imgs[1].device)
-    _compute("compute_rsgm", imgs, h, v, out, int(dmax), subpixel, rcp_lut, prm, None)
+    _compute("compute_rsgm", imgs, h, v, out, int(dmax), subpixel, rcp_lut, prm, None, uq)
     res = out if batched else out[0]
     return res.cpu().numpy() if was_numpy else res
 
 
 def compute_rsgm_stages(left, left_vpp, right_vpp, hints=None, validhints=None, dmax=192, subpixel=True, rcp_lut=None, p1=11,
-                        p2min=17, alpha=0.5, gamma=35, honor_params=False):
+                        p2min=17, alpha=0.5, gamma=35, honor_params=False, uniqueness=0.95, honor_uniqueness=False):
     """Same pipeline, also returning the stage taps used by the parity tests: dict with padded `census_l/r` (uint32),
     `dsi_agg` (uint16 [Hp,Wp,D]), `disp_l/r` (float32 [Hp,Wp] after median + interpolation + clip) and `out`.
-    p1 .. honor_params as in compute_rsgm."""
+    p1 .. honor_uniqueness as in compute_rsgm."""
     prm = _params(honor_params, p1, p2min, alpha, gamma)
+    uq = _uniq(honor_uniqueness, uniqueness, "compute_rsgm_stages")
     torch, was_numpy, batched, imgs, h, v, (N, H, W, C) = _prep(left, left_vpp, right_vpp, hints, validhints, int(dmax))
     dev = imgs[1].device
     D = int(dmax)
@@ -107,7 +117,7 @@ def compute_rsgm_stages(left, left_vpp, right_vpp, hints=None, validhints=None, 
     dl = torch.empty((N, Hp, Wp), dtype=torch.float32, device=dev)
     dr = torch.empty_like(dl)
     taps = _lib.RsgmTaps(cl.data_ptr(), cr.data_ptr(), S.data_ptr(), dl.data_ptr(), dr.data_ptr())
-    _compute("compute_rsgm_stages", imgs, h, v, out, D, subpixel, rcp_lut, prm, taps)
+    _compute("compute_rsgm_stages", imgs, h, v, out, D, subpixel, rcp_lut, prm, taps, uq)
     torch.cuda.synchronize(dev)
     return dict(census_l=_lib.dev_to_np(cl, np.uint32), census_r=_lib.dev_to_np(cr, np.uint32),
                 dsi_agg=_lib.dev_to_np(S, np.uint16), disp_l=dl.cpu().numpy(), disp_r=dr.cpu().numpy(),
