@@ -224,7 +224,7 @@ def test_compute_rsgm_params_vs_oracle(mods, orc, prm, shape, D, channels, sub):
 @pytest.mark.parametrize("prm", [(11, 17, 0.5, 35), (3, 30, 0.3, 80), (10, 10, 0.5, 265)])
 def test_aggregated_volume_vs_oracle(mods, orc, tuning, prm, sweep):
     """the dsi_agg stage tap against the oracle's aggregate_SSE(honor_params=True) on the same census volume, with the sweeps and
-    with the fast per-path kernels"""
+    with the sweeps turned off (the per-path kernel)"""
     rsgm, synth, _lib = mods
     tuning(_lib.TUNE_SGM_SWEEP, sweep)
     p = synth.make_pair(17, shape=(45, 100), hints="random")
@@ -265,9 +265,9 @@ def _kernel_names(fn):
 
 
 @pytest.mark.gpu
-def test_sweeps_run_for_in_domain_params(mods):
+def test_sweeps_run_for_in_domain_params(mods, tuning):
     """a silent fallback would pass every exactness test: the kernels that run are checked too"""
-    rsgm, synth = mods[0], mods[1]
+    rsgm, synth, _lib = mods
     p = synth.make_pair(9, shape=(40, 96), hints="random")
     run = lambda prm: rsgm.compute_rsgm(p["left"], p["left"], p["right"], dmax=32, **_honoured(prm))
     run((11, 17, 0.5, 35)); run((30, 10, 0.5, 20))                      # warm-up (module load, workspace)
@@ -277,6 +277,11 @@ def test_sweeps_run_for_in_domain_params(mods):
     names = _kernel_names(lambda: run((30, 10, 0.5, 20)))
     assert any("sgm_path_generic_kernel" in n for n in names), sorted(names)
     assert not any("sgm_v2_kernel" in n or "sgm_h_kernel" in n for n in names), sorted(names)
+    # in-domain parameters without the sweeps: the same per-path kernel as outside the domain
+    tuning(_lib.TUNE_SGM_SWEEP, 0)
+    names = _kernel_names(lambda: run((11, 17, 0.5, 35)))
+    assert any("sgm_path_generic_kernel" in n for n in names), sorted(names)
+    assert not any("sgm_path_fast" in n for n in names), sorted(names)
 
 
 @pytest.mark.gpu

@@ -356,8 +356,8 @@ extern "C" int vppb200_aggregate(const uint8_t *img, const uint16_t *dsi, uint16
     int rc = check_wd(W, H, D, n);
     if (rc) return rc;
     if (!img || !dsi || !dsi_agg || H < 3) return VPPB200_ERR_ARG;
-    if (!honor_params) { P1 = 7; P2min = 17; alpha = 0.25f; gamma = 50; }    // RSGM/pyrSGM.cpp:519 vs :557-560
-    return launch_aggregate_generic(img, dsi, dsi_agg, W, H, D, P1, P2min, alpha, gamma, n, (cudaStream_t)stream);
+    const SgmParams prm = honor_params ? SgmParams{P1, P2min, gamma, alpha} : default_sgm_params();   // RSGM/pyrSGM.cpp:519 vs :557-560
+    return launch_aggregate_generic(img, dsi, dsi_agg, W, H, D, prm, n, (cudaStream_t)stream);
 }
 
 static int check_uniq(float u) { return (u > 1.0f || u <= 0.0f) ? VPPB200_ERR_UNIQUENESS : VPPB200_OK; }
@@ -474,10 +474,9 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
     int rc;
     StageMarks tm;
     if (phases == 7) tm.begin(st);                           // per-stage timing covers whole-pipeline calls only
-    // the sweeps for parameters of their domain (the layout of the cost volume follows: every phase of a batch must see the same
-    // parameters and hints); otherwise the per-path kernels, saturating where the parameters make that reachable
-    const bool fast_params = sweep_params_supported(prm, hints == nullptr);
-    const bool tiled = fast_params && aggregate_tile_supported(d.Wp, d.Hp, D, n);
+    // the sweeps for parameters of their domain and shapes they hold (the layout of the cost volume follows: every phase of a batch
+    // must see the same parameters and hints); otherwise the saturating per-path kernel, exact for any parameters
+    const bool tiled = sweep_params_supported(prm, hints == nullptr) && aggregate_tile_supported(d.Wp, d.Hp, D, n);
     const bool want_volume = taps && taps->dsi_agg;          // only the test tap needs the aggregated volume itself
     const uint16_t *S_final = w.S;
     if (front) {
@@ -528,9 +527,7 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
                 if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st))) return rc;
             }
         } else {
-            if (fast_params) rc = launch_aggregate_fast(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
-            else rc = launch_aggregate_generic_u8(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st);
-            if (rc) return rc;
+            if ((rc = launch_aggregate_generic(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st))) return rc;
             tm.done(VPPB200_STAGE_SGM_H_BWD);                // the per-path fallback is booked on the last sweep's slot
             if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st))) return rc;
         }

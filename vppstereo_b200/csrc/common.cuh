@@ -100,17 +100,13 @@ int launch_census_fused(const uint8_t *src, uint32_t *dst, const RsgmDims &d, in
 int launch_cost_u16(const uint32_t *cl, const uint32_t *cr, uint16_t *dsi, int W, int H, int D, int n, cudaStream_t st);
 int launch_cost_u8(const uint32_t *cl, const uint32_t *cr, uint8_t *dsi, int W, int H, int D, int n, cudaStream_t st);
 int launch_guided_u8(uint8_t *dsi, const float *hints, const float *valid, const RsgmDims &d, int n, cudaStream_t st);
-// generic (saturating, u16 or u8 costs, any parameters) and fast (u8 costs, parameters of the sweep domain) 8-path aggregation
-int launch_aggregate_generic(const uint8_t *img, const uint16_t *dsi, uint16_t *S, int W, int H, int D, int P1, int P2min,
-                             float alpha, int gamma, int n, cudaStream_t st);
-int launch_aggregate_generic_u8(const uint8_t *img, const uint8_t *dsi, uint16_t *S, int W, int H, int D, const SgmParams &p, int n,
-                                cudaStream_t st);
-int launch_aggregate_fast(const uint8_t *img, const uint8_t *dsi, uint16_t *S, int W, int H, int D, const SgmParams &p, int n,
-                          cudaStream_t st);
+// saturating 8-path aggregation, any parameters: CT = uint16_t (aggregate_SSE) or uint8_t (compute_rsgm without the sweeps)
+template <typename CT>
+int launch_aggregate_generic(const uint8_t *img, const CT *dsi, uint16_t *S, int W, int H, int D, const SgmParams &p, int n,
+                             cudaStream_t st);
 // sgm_sweep.cu: layout-T cost volume + 4-sweep aggregation with on-chip path state (cluster per frame)
 bool aggregate_tile_supported(int W, int H, int D, int n);
-// do the sweeps (and the fast per-path kernels) compute these parameters exactly?  plain_costs: Hamming costs (<= 24), otherwise
-// guided costs (<= 240)
+// do the sweeps compute these parameters exactly?  plain_costs: Hamming costs (<= 24), otherwise guided costs (<= 240)
 bool sweep_params_supported(const SgmParams &p, bool plain_costs);
 size_t tile_volume_elems(int W, int H, int D, int n);
 // guided modulation of the tiled cost volume (models/rsgm/rsgm.py:115-127), fused into the cost kernel: hints / valid float32

@@ -1425,9 +1425,9 @@ bool aggregate_tile_supported(int W, int H, int D, int n)
     return plan_v(t, n, &plan) == VPPB200_OK;
 }
 
-// The parameter domain of the sweeps (file header): with these the packed u16 arithmetic of the sweeps and of the fast per-path
-// kernels never saturates, the P2 table's bytes hold P2 - P1, and the hand-off words keep their tag bits.  Outside it,
-// compute_rsgm aggregates with the saturating generic kernels of sgm.cu.  Expects 0 <= P1, P2min, gamma <= 65535, alpha >= 0.
+// The parameter domain of the sweeps (file header): with these the packed u16 arithmetic of the sweeps never saturates, the P2
+// table's bytes hold P2 - P1, and the hand-off words keep their tag bits.  Outside it, compute_rsgm aggregates with the
+// saturating per-path kernel of sgm.cu.  Expects 0 <= P1, P2min, gamma <= 65535, alpha >= 0.
 bool sweep_params_supported(const SgmParams &p, bool plain_costs)
 {
     const int cmax = plain_costs ? 24 : 240;
