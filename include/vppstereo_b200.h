@@ -339,6 +339,27 @@ int vppb200_vpp_scan_max_dist_adaptive(uint8_t *l, uint8_t *r, const float *g, i
                                        const float *filled_g, const float *patch_thresholds, int n_thresholds,
                                        int32_t *n_hints_out, void *workspace, size_t workspace_bytes, int n, void *stream);
 
+/* The gray context image of vppb200_bilateral_filling from the un-projected left image (vpp_standalone.py:414-417):
+ * src uint8 [n][H][W][C] -> gray uint8 [n][H][W]; C = 3: cv2.cvtColor(BGR2GRAY) in OpenCV's 15-bit fixed point
+ * (B*3735 + G*19235 + R*9798 + 16384) >> 15; any other C: the first channel. */
+int vppb200_bgr2gray(const uint8_t *src, uint8_t *gray, int W, int H, int C, int n, void *stream);
+
+/* The patch_thresholds operand of the adaptive scans, computed on the device (no host round trip).  The reference's size is
+ *   size(d) = round(float64(ratio) ** (1/gamma) * (wsize-1) + 1)  (round half to even),
+ *   ratio   = float32(float32(d) - dmin) / float32(dmax - dmin),  dmin / dmax = min / max of the frame's hints (g > 0).
+ * It splits exactly in two:
+ *   host   -- size is a non-decreasing function of the float32 ratio alone, so for k = 2..wsize there is a smallest float32
+ *             ratio R_k in [0, 1] with size >= k; the caller tabulates ratio_steps = {R_2 .. R_wsize} (float32 [wsize-1], DEVICE)
+ *             once per (wsize, gamma) with the host's libm -- the only evaluation of pow();
+ *   device -- per frame (one CTA), dmin / dmax over g > 0, then thr[k-2] = the smallest float32 d in [dmin, dmax] with
+ *             ratio(d) >= R_k (ratio with float32 round-to-nearest subtraction and division), by bisection on the bit patterns.
+ * patch_thresholds float32 [n][wsize-1]: +inf for a frame without hints (never read) and for a frame whose hints all have one
+ * value (dmin == dmax, where the reference raises ZeroDivisionError: patch size 1, a defined result); the latter also sets
+ * status[f] = 1 (int32 [n] device, entries of other frames untouched: the caller clears it; may be NULL).  wsize == 1: no
+ * thresholds (ratio_steps / patch_thresholds may be NULL), only the status. */
+int vppb200_distance_patch_thresholds(const float *g, int W, int H, const float *ratio_steps, int wsize, float *patch_thresholds,
+                                      int32_t *status, int n, void *stream);
+
 /* gt_reshape(gt f32[H,W]) -> f32[N,4] = (x, y, d, 1) in raster order           vpp_core_opt.pyx:352-371.
  * out must hold W*H rows; count_out int32 [1] device. */
 int vppb200_gt_reshape(const float *gt, int W, int H, float *out, int32_t *count_out, void *workspace,

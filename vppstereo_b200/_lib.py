@@ -89,6 +89,8 @@ PROTOTYPES = {
     "vppb200_bilateral_filling": (_i, (_p, _p, _p, _i, _i, _i, _p, _d, _i, _p)),
     "vppb200_vpp_scan_rnd_adaptive": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _u64, _p, _p, _i, _p, _p, _sz, _i, _p)),
     "vppb200_vpp_scan_max_dist_adaptive": (_i, (_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _d, _d, _p, _i, _i, _i, _p, _p, _i, _p, _p, _sz, _i, _p)),
+    "vppb200_bgr2gray": (_i, (_p, _p, _i, _i, _i, _i, _p)),
+    "vppb200_distance_patch_thresholds": (_i, (_p, _i, _i, _p, _i, _p, _p, _i, _p)),
     "vppb200_gt_reshape": (_i, (_p, _i, _i, _p, _p, _p, _sz, _p)),
     # occlusion mask
     "vppb200_occlusion_workspace_bytes": (_sz, (_i, _i, _i)),

@@ -701,6 +701,78 @@ __global__ void __launch_bounds__(256) bilateral_filling_kernel(const float *__r
     out[t] = ((double)cmap > th) ? aug : 0.0f;
 }
 
+// ---- gray context of _bilateral_filling (vpp_standalone.py:415-417): cv2.cvtColor(BGR2GRAY) in OpenCV's 15-bit fixed point,
+// otherwise the first channel (np.squeeze of a one-channel image).  One thread = one pixel.
+__global__ void __launch_bounds__(256) bgr2gray_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ gray, int C, long total)
+{
+    const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= total) return;
+    const uint8_t *p = src + t * C;
+    gray[t] = C == 3 ? (uint8_t)((p[0] * 3735u + p[1] * 19235u + p[2] * 9798u + 16384u) >> 15) : p[0];
+}
+
+// ---- distance-based patch size (vpp_standalone.py:6-9) without a host round trip ----------------------------------------
+// size(d) = round(float64(ratio32(d)) ** (1/gamma) * (wsize-1) + 1) is non-decreasing in the float32 ratio, and ratio32 is
+// non-decreasing in d, so size(d) >= k  <=>  ratio32(d) >= R_k, R_k = the smallest float32 ratio in [0, 1] of size >= k (host
+// table, the only pow()).  One CTA per frame: dmin / dmax over the hints (float min / max: exact in any order), then one thread
+// per step bisects the float32 bit patterns of [dmin, dmax] as _patch_thresholds does.
+__device__ __forceinline__ float patch_ratio32(float d, float dmin, float span) { return __fdiv_rn(__fsub_rn(d, dmin), span); }
+
+__global__ void __launch_bounds__(1024) distance_patch_thresholds_kernel(const float *__restrict__ g, long hw,
+                                                                         const float *__restrict__ ratio_steps, int nthr,
+                                                                         float *__restrict__ thr, int32_t *__restrict__ status)
+{
+    const float *gf = g + (long)blockIdx.x * hw;
+    float lo = INFINITY, hi = -INFINITY;
+    // scalar head up to 16-byte alignment, float4 body (4 loads in flight per thread), scalar tail
+    const long head = min(hw, (long)((16 - ((uintptr_t)gf & 15)) & 15) / 4);
+    const long n4 = (hw - head) / 4;
+    auto take = [&](float v) { if (v > 0.0f) { lo = fminf(lo, v); hi = fmaxf(hi, v); } };
+    for (long i = threadIdx.x; i < head; i += blockDim.x) take(gf[i]);
+    const float4 *g4 = reinterpret_cast<const float4 *>(gf + head);
+    for (long i = threadIdx.x; i < n4; i += 4L * blockDim.x) {
+        float4 v[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const long q = i + (long)j * blockDim.x;
+            v[j] = q < n4 ? __ldg(g4 + q) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++) { take(v[j].x); take(v[j].y); take(v[j].z); take(v[j].w); }
+    }
+    for (long i = head + 4 * n4 + threadIdx.x; i < hw; i += blockDim.x) take(gf[i]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = fminf(lo, __shfl_xor_sync(0xFFFFFFFFu, lo, o));
+        hi = fmaxf(hi, __shfl_xor_sync(0xFFFFFFFFu, hi, o));
+    }
+    __shared__ float s_lo[32], s_hi[32];
+    const int warp = threadIdx.x >> 5, nwarps = (blockDim.x + 31) >> 5;
+    if ((threadIdx.x & 31) == 0) { s_lo[warp] = lo; s_hi[warp] = hi; }
+    __syncthreads();
+    lo = s_lo[0]; hi = s_hi[0];
+    for (int w = 1; w < nwarps; w++) { lo = fminf(lo, s_lo[w]); hi = fmaxf(hi, s_hi[w]); }
+    // no hints: the steps are never read; dmin == dmax: the reference raises ZeroDivisionError -- patch size 1 and status set
+    const bool degenerate = lo == hi;
+    if (degenerate && threadIdx.x == 0 && status) status[blockIdx.x] = 1;
+    const float span = __fsub_rn(hi, lo);
+    for (int k = threadIdx.x; k < nthr; k += blockDim.x) {
+        const float R = ratio_steps[k];
+        float out = INFINITY;
+        if (!(lo > hi) && !degenerate && patch_ratio32(hi, lo, span) >= R) {
+            uint32_t a = __float_as_uint(lo), b = __float_as_uint(hi);      // positive floats: bit order = value order
+            if (patch_ratio32(lo, lo, span) >= R) b = a;
+            while (a < b) {                                                  // invariant: ratio32(b) >= R
+                const uint32_t mid = a + (b - a) / 2;
+                if (patch_ratio32(__uint_as_float(mid), lo, span) >= R) b = mid;
+                else a = mid + 1;
+            }
+            out = __uint_as_float(b);
+        }
+        thr[(long)blockIdx.x * nthr + k] = out;
+    }
+}
+
 // ---- maxDistance: one warp per (frame, channel), sequential over hints ------------------------------------------
 // fold of the ordered window samples into (pa, pb)  (pyx:216-313): lane p of a chunk holds window position
 // chunk*32+p with up to two samples (left first, then right).
@@ -1305,6 +1377,26 @@ extern "C" int vppb200_bilateral_filling(const float *dmap, const uint8_t *gray,
     const long total = (long)n * H * W;
     bilateral_filling_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(dmap, gray, out, W, H, n_patch, weights, th, total);
     VPP_LAUNCH_CHECK("bilateral_filling_kernel");
+    return VPPB200_OK;
+}
+
+extern "C" int vppb200_bgr2gray(const uint8_t *src, uint8_t *gray, int W, int H, int C, int n, void *stream)
+{
+    if (!src || !gray || W <= 0 || H <= 0 || C <= 0 || n <= 0) return VPPB200_ERR_ARG;
+    const long total = (long)n * H * W;
+    bgr2gray_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(src, gray, C, total);
+    VPP_LAUNCH_CHECK("bgr2gray_kernel");
+    return VPPB200_OK;
+}
+
+extern "C" int vppb200_distance_patch_thresholds(const float *g, int W, int H, const float *ratio_steps, int wsize,
+                                                 float *patch_thresholds, int32_t *status, int n, void *stream)
+{
+    if (!g || W <= 0 || H <= 0 || wsize < 1 || n <= 0 || (wsize > 1 && (!ratio_steps || !patch_thresholds)))
+        return VPPB200_ERR_ARG;
+    distance_patch_thresholds_kernel<<<n, 1024, 0, (cudaStream_t)stream>>>(g, (long)W * H, ratio_steps, wsize - 1,
+                                                                           patch_thresholds, status);
+    VPP_LAUNCH_CHECK("distance_patch_thresholds_kernel");
     return VPPB200_OK;
 }
 

@@ -1,5 +1,5 @@
-"""The whole hot path as one object: VPP (rnd pattern, numba arithmetic as test.py uses it) followed by compute_rsgm on a
-batch of frames, with the images staying on the device between the two (test.py:158-225 without the host round-trips).
+"""The whole hot path as one object: VPP (numba arithmetic as test.py uses it) followed by compute_rsgm on a batch of frames,
+with the images staying on the device between the two (test.py:154-225 without the host round-trips).
 
     pipe = VppRsgmPipeline(H, W, batch=64, dmax=192)
     disp = pipe.run_device(left_u8, right_u8, hints_f32)        # CUDA tensors in, CUDA float32 [N,H,W] out
@@ -8,8 +8,19 @@ batch of frames, with the images staying on the device between the two (test.py:
     pipe = VppRsgmPipeline(H, W, guided=True)                   # guided matching (rsgm.py:115-127) on the same hints:
     disp = pipe.run_device(left_u8, right_u8, hints_f32, validhints=valid_f32)    # compute_rsgm(left, lv, rv, hints, validhints)
 
+The projection covers test.py's options with vpp()'s keyword names (default: rnd pattern, fixed patch, no occlusion mask):
+
+    pipe = VppRsgmPipeline(H, W, maskocc=True)                           # the paper's default: --maskocc
+    pipe = VppRsgmPipeline(H, W, maskocc=True, method="maxDistance")     # --colormethod maxDistance
+    pipe = VppRsgmPipeline(H, W, maskocc=True, wsize=7, use_bilateral_patch=True, use_distance_patch=True)   # the journal's
+
+maskocc: g_occ = occlusion_heuristic(hints)[1] with the reference's default parameters (test.py:154), computed per call on the
+device; the adaptive patches' operands (bilateral filling, distance-based patch thresholds) are computed on the device too, so
+no option adds a host round trip to run_device.
+
 Three phases of neighbouring batches run concurrently on three internal streams (software pipeline across calls):
-  front(k+1) = VPP + pad/gray/census/cost volume   |   main(k) = 8-path SGM sweeps + WTA   |   tail(k-1) = median ... fills
+  front(k+1) = [occlusion mask, adaptive-patch operands] + VPP + pad/gray/census/cost volume
+  main(k) = 8-path SGM sweeps + WTA   |   tail(k-1) = median ... fills
 with two buffer sets for everything that crosses a phase boundary; the SGM sweeps alone keep the critical stream busy
 and the small, latency-bound front and tail kernels fill the idle issue slots beside them.
 
@@ -17,19 +28,44 @@ run_host is the end-to-end path: host->device copies of the three inputs and the
 are part of the call.  submit_host / collect is the same path for streams of batches: the copies of batch k+1 and of
 batch k-1 ride their own CUDA streams while batch k computes (two staging sets, events between the streams).
 """
+import numpy as np
+
 from . import _lib
 from . import vpp_core_opt as _core
+from . import vpp_standalone as _vs
 
 
 class VppRsgmPipeline:
     guided = False                                    # set per object by __init__(guided=...)
+    _stage_marks = None   # bench-only hook (tools/bench_pipeline_modes.py): a list to which the front phase appends
+                          # (step name, timing CUDA event) after each of its steps; None (the default) records nothing
 
     def __init__(self, H, W, channels=3, batch=64, dmax=192, wsize=3, blending=0.4, c_occ=0.0, left2right=True,
-                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None, guided=False, uniqueness=None):
+                 interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None, guided=False, uniqueness=None,
+                 method="rnd", wsizeAgg_x=64, wsizeAgg_y=3, discard_occ=False, uniform_color=False, use_distance_patch=False,
+                 distance_gamma=0.3, use_bilateral_patch=False, bilateral_o_xy=2, bilateral_o_i=1, bilateral_th=.001,
+                 maskocc=False):
         # sgm_params: (p1, p2min, alpha, gamma) honoured by the matcher; None = the reference's effective values (7, 17, 0.25, 50)
         # guided: the matcher is compute_rsgm(left, lv, rv, hints, validhints) -- every entry point then takes `validhints`
         # (float32 [N,H,W], placed like `hints`).  Parameters outside the guided sweep domain run on the per-path kernels.
         # uniqueness: the WTA's uniqueness ratio, compute_rsgm(..., uniqueness=u, honor_uniqueness=True); None = off
+        # method ... bilateral_th: vpp()'s keywords of the same names (vpp_standalone.py:396), numba arithmetic
+        # maskocc: g_occ = occlusion_heuristic(hints)[1] (test.py:154, --maskocc); without it the mask is all zero and c_occ
+        # has no effect
+        # use_distance_patch: a batch with a frame whose hints all have one value has no reference output (the reference raises
+        # ZeroDivisionError); that frame is projected with patch size 1 and check() / run_host() / collect() raise
+        # ZeroDivisionError for it (see _raise_degenerate)
+        if method not in ("rnd", "maxDistance"):
+            raise ValueError(f"method: expected 'rnd' or 'maxDistance', got {method!r}")
+        for name, v in (("wsize", wsize), ("wsizeAgg_x", wsizeAgg_x), ("wsizeAgg_y", wsizeAgg_y)):
+            if int(v) != v or int(v) < 1:
+                raise ValueError(f"{name}: expected a window size >= 1, got {v!r}")
+        self.method = method
+        self.wsize_agg = (int(wsizeAgg_x), int(wsizeAgg_y))
+        self.discard_occ, self.uniform_color, self.maskocc = bool(discard_occ), bool(uniform_color), bool(maskocc)
+        self.use_distance_patch, self.use_bilateral_patch = bool(use_distance_patch), bool(use_bilateral_patch)
+        self.distance_gamma = distance_gamma
+        self.bilateral = (bilateral_o_xy, bilateral_o_i, float(bilateral_th))
         self.sgm_params = None if sgm_params is None else _lib.sgm_params(*sgm_params)
         self.uniqueness = 1.0 if uniqueness is None else _lib.uniqueness(uniqueness, "VppRsgmPipeline")
         self.guided = bool(guided)
@@ -51,9 +87,33 @@ class VppRsgmPipeline:
         with torch.cuda.device(self.device):
             self.ws_rsgm = torch.empty(L.vppb200_rsgm_workspace_bytes_sets(self.H, self.W, self.C, self.D, self.N, 2),
                                        dtype=torch.uint8, device=self.device)
-            self.ws_vpp = torch.empty(L.vppb200_vpp_workspace_bytes(self.H, self.W, self.C, self.N), dtype=torch.uint8,
-                                      device=self.device)
+            ws_vpp = L.vppb200_vpp_workspace_bytes(self.H, self.W, self.C, self.N)
+            if self.method == "maxDistance":     # + the row wavefront's dependency table
+                ws_vpp = max(ws_vpp, L.vppb200_vpp_max_dist_workspace_bytes(self.H, self.W, self.C, self.wsize, self.wsize_agg[1],
+                                                                            self.N))
+            self.ws_vpp = torch.empty(ws_vpp, dtype=torch.uint8, device=self.device)
             self.occ = torch.zeros((self.N, self.H, self.W), dtype=torch.uint8, device=self.device)
+            # buffers of the optional front-phase steps: produced and consumed inside one front phase, and front phases are
+            # ordered on one stream, so a single copy of each serves both buffer sets
+            self.ws_occ = self.gray = self.filled = self.bl_weights = self.ratio_steps = self.thr = None
+            self.status = self.status_host = None
+            if self.maskocc:
+                self.ws_occ = torch.empty(L.vppb200_occlusion_workspace_bytes(self.H, self.W, self.N), dtype=torch.uint8,
+                                          device=self.device)
+            if self.use_bilateral_patch:
+                self.gray = torch.empty((self.N, self.H, self.W), dtype=torch.uint8, device=self.device)
+                self.filled = torch.empty((self.N, self.H, self.W), dtype=torch.float32, device=self.device)
+                wt = _vs._bilateral_weights((self.wsize - 1) // 2, self.bilateral[0], self.bilateral[1])
+                self.bl_weights = torch.from_numpy(wt).to(self.device)
+            if self.use_distance_patch:
+                self.ratio_steps = torch.from_numpy(_vs._ratio_steps(self.wsize, distance_gamma).copy()).to(self.device)
+                if self.wsize > 1:
+                    self.thr = torch.empty((self.N, self.wsize - 1), dtype=torch.float32, device=self.device)
+                # degenerate-frame status words (see _raise_degenerate): one per way of calling, so that each is read only
+                # by the call that owns it -- run_device / run_device_serial (reported by check()), run_host; submit_host
+                # gives every staging set its own
+                self.status = torch.zeros(self.N, dtype=torch.int32, device=self.device)
+                self.status_host = torch.zeros(self.N, dtype=torch.int32, device=self.device)
             self.lv = torch.empty((self.N, self.H, self.W, self.C), dtype=torch.uint8, device=self.device)
             self.rv = torch.empty_like(self.lv)
             # two projected-image sets + VPP stream: see run_device
@@ -75,8 +135,9 @@ class VppRsgmPipeline:
             self.h_disp = torch.empty((self.N, self.H, self.W), dtype=torch.float32).pin_memory()
             self._stream_sets = None                  # created by the first submit_host
             self.host_depth = 3                       # staging sets of the streaming host API
-            # the zero-filled occlusion mask above was queued on the constructing stream, while the first call's front phase
-            # runs on this object's own streams (which do not wait for it when inputs_ready=True): finish it here
+            # the zero-filled occlusion mask / status and the tables above were queued on the constructing stream, while the
+            # first call's front phase runs on this object's own streams (which do not wait for it when inputs_ready=True):
+            # finish them here
             torch.cuda.current_stream(self.device).synchronize()
 
     def close(self):
@@ -102,11 +163,35 @@ class VppRsgmPipeline:
             pass
 
     def check(self):
-        """Wait for the device and raise if a sweep reported a timed-out hand-off between its CTAs (vppb200_async_error)."""
+        """Wait for the device and raise if a sweep reported a timed-out hand-off between its CTAs (vppb200_async_error), or
+        ZeroDivisionError for a degenerate frame (use_distance_patch, see _raise_degenerate) of a run_device /
+        run_device_serial call since the last check()."""
         _lib.check_async(self.device)
+        if self.status is None:
+            return
+        torch = self.torch
+        with torch.cuda.device(self.device):
+            self.vpp_stream.synchronize()
+            bad = self.status.cpu().numpy()
+            if bad.any():
+                with torch.cuda.stream(self.vpp_stream):      # ordered before every later front phase (serial ones wait for it)
+                    self.status.zero_()
+                self._raise_degenerate(bad, "a run_device / run_device_serial call since the last check()")
+
+    @staticmethod
+    def _raise_degenerate(status, which):
+        """use_distance_patch: the reference divides by (dmax - dmin) (vpp_standalone.py:7) and raises ZeroDivisionError for a
+        frame whose hints all have one value.  run_device does not synchronise, so the thresholds kernel only records such a
+        frame in a device status word of the call (the frame is projected with patch size 1: defined and deterministic, but
+        not a reference output, since the reference has none).  The calls that synchronise anyway raise for it: run_host()
+        and collect() for their own batch, check() for the run_device / run_device_serial calls since the previous check();
+        each status is cleared once read, so the pipeline stays usable for the next batch."""
+        f = int(np.flatnonzero(status)[0])
+        raise ZeroDivisionError(f"division by zero: every hint of frame {f} of {which} has the same disparity "
+                                "(use_distance_patch); that batch's output is not the reference's")
 
     def workspace_bytes(self):
-        return self.ws_rsgm.numel() + self.ws_vpp.numel()
+        return self.ws_rsgm.numel() + self.ws_vpp.numel() + (self.ws_occ.numel() if self.ws_occ is not None else 0)
 
     def _check(self, left, right, hints, out=None, host=False, validhints=None):
         """Operand validation shared by every entry point: the kernels receive raw pointers, so a wrong dtype, shape, device
@@ -160,11 +245,43 @@ class VppRsgmPipeline:
         replays the projected pattern of any frame on the host."""
         return (self.seed * 0x9E3779B97F4A7C15 + int(step)) & (2**64 - 1)
 
-    def _vpp(self, lv, rv, hints, seed, N, stream):
-        # VPP of the projected-image pair lv / rv in place: rnd pattern drawn on the device from `seed`, numba arithmetic
-        _lib.call("vppb200_vpp_scan_rnd", _lib.ptr(lv), _lib.ptr(rv), _lib.ptr(hints), self.W, self.H, self.C, 0, self.wsize,
-                  self.direction, self.blending, self.c_occ, _lib.ptr(self.occ), 0, int(self.interpolate), 1, None, None, seed,
-                  None, _lib.ptr(self.ws_vpp), self.ws_vpp.numel(), N, stream.cuda_stream, what="vpp_scan_rnd")
+    def _vpp(self, left, lv, rv, hints, seed, N, stream, status):
+        # VPP of the projected-image pair lv / rv in place (vpp_standalone.py:396-432), numba arithmetic; `left` = the
+        # un-projected left image, `status` = the call's degenerate-frame status words (use_distance_patch).  Every step is queued on `stream`, in the reference's order: occlusion mask, adaptive-patch
+        # operands, scan (rnd: pattern drawn on the device from `seed`).
+        s = stream.cuda_stream
+        self._mark("copy", stream)
+        if self.maskocc:                              # occlusion_heuristic(hints)[1] straight into the mask the scan reads
+            _lib.call("vppb200_occlusion_heuristic", _lib.ptr(hints), None, _lib.ptr(self.occ), self.W, self.H, 9, 7, 2.0, 0.4375,
+                      1.0, 0.1, _lib.ptr(self.ws_occ), self.ws_occ.numel(), N, s, what="occlusion_heuristic")
+        self._mark("occlusion", stream)
+        filled = thr = None
+        if self.use_bilateral_patch:
+            filled = self.filled[:N]
+            _vs.bilateral_filling(hints, left, (self.wsize - 1) // 2, self.bl_weights, self.bilateral[2], self.gray[:N], filled, s)
+        if self.use_distance_patch:
+            thr = self.thr[:N] if self.thr is not None else None
+            _vs.distance_patch_thresholds(hints, self.wsize, self.ratio_steps, thr, status, s)
+        self._mark("patch_operands", stream)
+        img = (_lib.ptr(lv), _lib.ptr(rv), _lib.ptr(hints), self.W, self.H, self.C, int(self.uniform_color), self.wsize)
+        blend = (self.blending, self.c_occ, _lib.ptr(self.occ), int(self.discard_occ), int(self.interpolate), 1)
+        tail = (None, _lib.ptr(self.ws_vpp), self.ws_vpp.numel(), N, s)
+        adaptive = () if filled is None and thr is None else (_lib.ptr(filled), _lib.ptr(thr), 0 if thr is None else self.wsize - 1)
+        if self.method == "maxDistance":
+            md = img + self.wsize_agg + (self.direction,) + blend
+            _lib.call("vppb200_vpp_scan_max_dist_adaptive" if adaptive else "vppb200_vpp_scan_max_dist", *md, *adaptive, *tail,
+                      what="vpp_scan_max_dist")
+        else:
+            rnd = img + (self.direction,) + blend + (None, None, seed)
+            _lib.call("vppb200_vpp_scan_rnd_adaptive" if adaptive else "vppb200_vpp_scan_rnd", *rnd, *adaptive, *tail,
+                      what="vpp_scan_rnd")
+        self._mark("scan", stream)
+
+    def _mark(self, name, stream):
+        if self._stage_marks is not None:
+            ev = self.torch.cuda.Event(enable_timing=True)
+            ev.record(stream)
+            self._stage_marks.append((name, ev))
 
     def _phase(self, phases, b, left, lv, rv, out, N, stream, hints, validhints):
         # hints / validhints go to every phase of a guided batch (their nullness selects the sweeps' state); FRONT reads them
@@ -188,9 +305,9 @@ class VppRsgmPipeline:
         torch = self.torch
         N = self._check(left, right, hints, out, validhints=validhints)
         with torch.cuda.device(self.device):
-            return self._run_device(left, right, hints, validhints, out, inputs_ready, step, N)
+            return self._run_device(left, right, hints, validhints, out, inputs_ready, step, N, self.status)
 
-    def _run_device(self, left, right, hints, validhints, out, inputs_ready, step, N):
+    def _run_device(self, left, right, hints, validhints, out, inputs_ready, step, N, status):
         torch = self.torch
         out = self.disp[:N] if out is None else out
         caller = torch.cuda.current_stream(self.device)
@@ -215,7 +332,7 @@ class VppRsgmPipeline:
         self.last_n = N
         with torch.cuda.stream(front):
             lv.copy_(left); rv.copy_(right)              # vpp() returns copies (vpp_standalone.py:397)
-            self._vpp(lv, rv, hints, seed, N, front)
+            self._vpp(left, lv, rv, hints, seed, N, front, status)
             self._phase(1, b, left, lv, rv, out, N, front, hints, validhints)
             self.front_done[b].record(front)
         # ---- main: the four SGM sweeps + WTA (the critical stream)
@@ -256,7 +373,7 @@ class VppRsgmPipeline:
         lv, rv = self.lv2[b][:N], self.rv2[b][:N]
         seed = self._next_seed(step)
         lv.copy_(left); rv.copy_(right)
-        self._vpp(lv, rv, hints, seed, N, st)
+        self._vpp(left, lv, rv, hints, seed, N, st, self.status)
         self._phase(7, b, left, lv, rv, out, N, st, hints, validhints)
         for s in (self.vpp_stream, self.main_stream, self.tail_stream):
             s.wait_stream(st)
@@ -275,9 +392,15 @@ class VppRsgmPipeline:
             if self.guided:
                 dv = self.d_valid[:N]
                 dv.copy_(validhints, non_blocking=True)
-            out = self.run_device(self.d_left[:N], self.d_right[:N], self.d_hints[:N], validhints=dv)
+            if self.status_host is not None:
+                self.status_host.zero_()          # current stream: the front phase below waits for it (inputs_ready=None)
+            out = self._run_device(self.d_left[:N], self.d_right[:N], self.d_hints[:N], dv, None, None, None, N, self.status_host)
             self.h_disp[:N].copy_(out, non_blocking=True)
             torch.cuda.current_stream(self.device).synchronize()
+            if self.status_host is not None:
+                bad = self.status_host[:N].cpu().numpy()     # the current stream is idle: this reads this call's words
+                if bad.any():
+                    self._raise_degenerate(bad, "this run_host batch")
         return self.h_disp[:N]
 
     # ---- streaming front-end: overlapped host<->device copies ---------------------------------------------------
@@ -291,6 +414,8 @@ class VppRsgmPipeline:
                                      hints=torch.empty_like(self.d_hints), disp=torch.empty_like(self.disp),
                                      valid=torch.empty_like(self.d_hints) if self.guided else None,
                                      h_disp=torch.empty((self.N, self.H, self.W), dtype=torch.float32).pin_memory(),
+                                     status=torch.empty_like(self.status) if self.status is not None else None,
+                                     h_status=torch.zeros(self.N, dtype=torch.int32).pin_memory(),
                                      copied_in=torch.cuda.Event(), computed=torch.cuda.Event(), copied_out=torch.cuda.Event(),
                                      busy=False))
                 self._stream_sets = dict(sets=sets, h2d=torch.cuda.Stream(self.device), d2h=torch.cuda.Stream(self.device), turn=0)
@@ -318,16 +443,20 @@ class VppRsgmPipeline:
                 st["hints"][:N].copy_(hints, non_blocking=True)
                 if self.guided:
                     st["valid"][:N].copy_(validhints, non_blocking=True)
+                if st["status"] is not None:
+                    st["status"].zero_()                 # this batch's own status words (read back with its disparities)
                 st["copied_in"].record(ss["h2d"])
             compute.wait_event(st["copied_in"])
-            self.run_device(st["left"][:N], st["right"][:N], st["hints"][:N], out=st["disp"][:N], inputs_ready=st["copied_in"],
-                            validhints=st["valid"][:N] if self.guided else None)
+            self._run_device(st["left"][:N], st["right"][:N], st["hints"][:N], st["valid"][:N] if self.guided else None,
+                             st["disp"][:N], st["copied_in"], None, N, st["status"])
             st["computed"].record(compute)
             if on_computed is not None:
                 on_computed(st["disp"][:N])
             with torch.cuda.stream(ss["d2h"]):
                 ss["d2h"].wait_event(st["computed"])
                 st["h_disp"][:N].copy_(st["disp"][:N], non_blocking=True)
+                if st["status"] is not None:
+                    st["h_status"][:N].copy_(st["status"][:N], non_blocking=True)
                 st["copied_out"].record(ss["d2h"])
         st["busy"], st["n"] = True, N
         ss["turn"] += 1
@@ -335,10 +464,13 @@ class VppRsgmPipeline:
 
     def collect(self, ticket):
         """Wait for a submitted batch; returns its pinned host float32 [N,H,W] disparities (valid until that staging set is
-        reused by the `host_depth`-th submit_host after it was submitted)."""
+        reused by the `host_depth`-th submit_host after it was submitted).  use_distance_patch: ZeroDivisionError if this
+        batch has a frame whose hints all have one value (see _raise_degenerate); the batches around it are unaffected."""
         st = self._streaming()["sets"][ticket]
         if not st["busy"]:
             raise RuntimeError("collect: nothing in flight for this ticket")
         st["copied_out"].synchronize()
         st["busy"] = False
+        if st["status"] is not None and st["h_status"][:st["n"]].any():
+            self._raise_degenerate(st["h_status"][:st["n"]].numpy(), f"the batch of ticket {ticket}")
         return st["h_disp"][:st["n"]]

@@ -109,33 +109,60 @@ def _patch_thresholds(dmin, dmax, patch_size, gamma):
     return thr
 
 
+@functools.lru_cache(maxsize=16)
+def _ratio_steps(patch_size, gamma):
+    """R_k for k = 2..patch_size: the smallest float32 ratio in [0, 1] whose patch size is >= k (vpp_standalone.py:6-9), float32
+    [patch_size-1].  With dmin = 0 and dmax = 1 the ratio of _patch_size is d itself, so these are _patch_thresholds(0, 1): the
+    only evaluation of pow(), with the host's libm.  vppb200_distance_patch_thresholds turns them into each frame's disparity
+    thresholds on the device.  (Read-only: the array is shared by every caller.)"""
+    steps = _patch_thresholds(np.float32(0.0), np.float32(1.0), int(patch_size), gamma)
+    steps.setflags(write=False)
+    return steps
+
+
+def distance_patch_thresholds(g, patch_size, ratio_steps, thr_out, status_out, stream):
+    """Queue vppb200_distance_patch_thresholds on `stream` (a raw stream handle): g float32 [N,H,W] CUDA, ratio_steps the device
+    copy of _ratio_steps(patch_size, gamma), thr_out float32 [N, patch_size-1] (None when patch_size == 1), status_out int32 [N]
+    (set to 1 for a frame whose hints all have one value)."""
+    N, H, W = g.shape
+    _lib.call("vppb200_distance_patch_thresholds", _lib.ptr(g), W, H, _lib.ptr(ratio_steps), int(patch_size), _lib.ptr(thr_out),
+              _lib.ptr(status_out), N, stream, what="distance_patch_thresholds")
+
+
+def bilateral_filling(g, left, n_patch, weights, th, gray_out, filled_out, stream):
+    """Queue the bilateral filling of the hints g float32 [N,H,W] (vpp_standalone.py:371-394) with the gray context of the
+    un-projected left image uint8 [N,H,W,C] (:414-417) on `stream`: gray_out uint8 [N,H,W], filled_out float32 [N,H,W];
+    weights = the device copy of _bilateral_weights(n_patch, o_xy, o_i)."""
+    N, H, W = g.shape
+    _lib.call("vppb200_bgr2gray", _lib.ptr(left), _lib.ptr(gray_out), W, H, int(left.shape[-1]), N, stream, what="bgr2gray")
+    _lib.call("vppb200_bilateral_filling", _lib.ptr(g), _lib.ptr(gray_out), _lib.ptr(filled_out), W, H, int(n_patch),
+              _lib.ptr(weights), float(th), N, stream, what="bilateral_filling")
+
+
 def _adaptive_operands(lc, g, wsize, use_distance, use_bilateral, gamma, o_xy, o_i, th):
     """(filled_g or None, thresholds or None) as device tensors for the adaptive scans."""
     torch = _lib.torch_mod()
     batched = g.dim() == 3
-    gg = g if batched else g[None]
+    gg = (g if batched else g[None]).contiguous()
     N, H, W = gg.shape
     n = (int(wsize) - 1) // 2
     filled = thr = None
-    if use_distance:
-        pos = gg > 0
-        dmin = torch.where(pos, gg, torch.full_like(gg, float("inf"))).amin(dim=(1, 2)).cpu().numpy()     # gt[gt>0].min() (:410)
-        dmax = torch.where(pos, gg, torch.full_like(gg, float("-inf"))).amax(dim=(1, 2)).cpu().numpy()
-        rows = [np.full(max(int(wsize) - 1, 0), np.inf, np.float32) if not np.isfinite(lo) else
-                _patch_thresholds(lo, hi, int(wsize), gamma) for lo, hi in zip(dmin, dmax)]               # frames without hints: unused
-        thr = torch.from_numpy(np.stack(rows)).to(g.device) if int(wsize) > 1 else None
-    if use_bilateral:
-        ll = lc if batched else lc[None]
-        if ll.shape[-1] == 3:      # cv2.cvtColor(lc, COLOR_BGR2GRAY) (:415): OpenCV's 15-bit fixed point
-            c = ll.to(torch.int32)
-            gray = ((c[..., 0] * 3735 + c[..., 1] * 19235 + c[..., 2] * 9798 + 16384) >> 15).to(torch.uint8).contiguous()
-        else:
-            gray = ll[..., 0].contiguous()                   # np.squeeze(lc) (:417)
-        wt = torch.from_numpy(_bilateral_weights(n, o_xy, o_i)).to(g.device)
-        filled = torch.empty_like(gg)
-        with torch.cuda.device(g.device):
-            _lib.call("vppb200_bilateral_filling", _lib.ptr(gg.contiguous()), _lib.ptr(gray), _lib.ptr(filled), W, H, n, _lib.ptr(wt),
-                      float(th), N, _lib.stream_ptr(g.device), what="bilateral_filling")
+    with torch.cuda.device(g.device):
+        st = _lib.stream_ptr(g.device)
+        if use_distance:
+            steps = torch.from_numpy(_ratio_steps(int(wsize), gamma).copy()).to(g.device)
+            thr = torch.empty((N, max(int(wsize) - 1, 0)), dtype=torch.float32, device=g.device) if int(wsize) > 1 else None
+            status = torch.zeros(N, dtype=torch.int32, device=g.device)
+            distance_patch_thresholds(gg, int(wsize), steps, thr, status, st)
+            bad = np.flatnonzero(status.cpu().numpy())
+            if bad.size:      # numba's python error model on (d_max - d_min) == 0 (:7), before any scan work
+                raise ZeroDivisionError(f"division by zero (frame {int(bad[0])}: every hint has the same disparity)")
+        if use_bilateral:
+            ll = (lc if batched else lc[None]).contiguous()
+            wt = torch.from_numpy(_bilateral_weights(n, o_xy, o_i)).to(g.device)
+            gray = torch.empty((N, H, W), dtype=torch.uint8, device=g.device)
+            filled = torch.empty_like(gg)
+            bilateral_filling(gg, ll, n, wt, th, gray, filled, st)
     return filled, thr
 
 
