@@ -230,6 +230,46 @@ int vppb200_compute_rsgm_uniq(const uint8_t *left, const uint8_t *left_vpp, cons
                               int phases, int sets, int set, const vppb200_rsgm_taps *taps,
                               const vppb200_sgm_params *params, float uniqueness);
 
+/* ---- per-pixel match info of the left view (an opt-in the reference does not have: its compute_rsgm returns a dense map in which
+ * a measured disparity and a hole filled by _interpolate_background, models/rsgm/rsgm.py:184-227, look the same).  Maps are cropped
+ * [n][H][W] like disp_out.  With the stages of compute_rsgm (rsgm.py:250-294) named
+ *   m    = the left map after WTA (with the uniqueness test where it is honoured), sub-pixel step and median3x3, padded frame;
+ *   c    = max(_linear_interpolate(m), 0), cropped;  mask = _left_right_check(c, c_right);  u = uint8(c with mask == 128 set to 0);
+ *   s    = filterSpeckles(u),
+ * state uint8 is the code of the first rule that applies, in this order:
+ *   VPPB200_STATE_NO_MATCH     c == 0 (no positive WTA winner, uniqueness-rejected, or not positive after the median, and not filled
+ *                              by the gap interpolation)
+ *   VPPB200_STATE_LR_REJECTED  mask == 128 (includes a match that points outside the right image)
+ *   VPPB200_STATE_BELOW_ONE    u == 0 (0 < c < 1, truncated by astype(uint8))
+ *   VPPB200_STATE_SPECKLE      s == 0
+ *   VPPB200_STATE_INTERPOLATED m <= 0 (the value came from _linear_interpolate)
+ *   VPPB200_STATE_MATCHED      otherwise (s > 0 and m > 0).
+ * Codes 2..5 are exactly the pixels whose disparity comes from the background fill (or stays 0 where the fill finds nothing).
+ * cost, rival uint16, from the final aggregated volume S at the padded pixel (y + pad_top, x + pad_left): with end = min(D-1, x +
+ * pad_left) and b = the first arg-min over 0..end, cost = S[b] and rival = min{S[d] : 0 <= d <= end, |d - b| >= 2}, 65535 when no
+ * such d exists -- the c[b] and c2 of the uniqueness block above, reported whether or not the test is honoured (and equal either
+ * way).  Turning the info on changes no disparity.
+ *   vppb200_rsgm_info_workspace_bytes: vppb200_rsgm_workspace_bytes_sets + per-set padded cost / rival maps (they cross the
+ *       MAIN -> TAIL boundary like the raw disparities).
+ *   vppb200_compute_rsgm_info: vppb200_compute_rsgm_uniq (same arguments, taps included) + the three outputs, all required
+ *       (VPPB200_ERR_ARG otherwise); every phase of one batch must pass the same pointers.  MAIN fills the set's cost / rival
+ *       maps, TAIL writes state_out, cost_out and rival_out (ordered like disp_out).  A workspace smaller than the info layout:
+ *       VPPB200_ERR_WORKSPACE. */
+#define VPPB200_STATE_MATCHED 0
+#define VPPB200_STATE_INTERPOLATED 1
+#define VPPB200_STATE_NO_MATCH 2
+#define VPPB200_STATE_LR_REJECTED 3
+#define VPPB200_STATE_BELOW_ONE 4
+#define VPPB200_STATE_SPECKLE 5
+size_t vppb200_rsgm_info_workspace_bytes(int H, int W, int C, int D, int n, int sets);
+int vppb200_compute_rsgm_info(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp,
+                              const float *hints, const float *validhints, float *disp_out,
+                              int H, int W, int C, int D, int flags, const float *rcp_lut,
+                              void *workspace, size_t workspace_bytes, int n, void *stream,
+                              int phases, int sets, int set, const vppb200_rsgm_taps *taps,
+                              const vppb200_sgm_params *params, float uniqueness,
+                              uint8_t *state_out, uint16_t *cost_out, uint16_t *rival_out);
+
 /* ---- one frame split into row bands over several GPUs (SURVEY.md 8e: an oversized frame) -------------------------------
  * compute_rsgm (models/rsgm/rsgm.py:250-294) as three calls so that the aggregation -- the 2.2 GB of volumes of a Middlebury
  * frame -- runs band by band on different GPUs, EXACTLY (unlike the reference's approximate StripedStereoSGM,

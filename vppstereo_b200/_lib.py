@@ -14,6 +14,8 @@ LIB_PATH = os.path.join(HERE, "libvppstereo_b200.so")
 
 OK = 0
 ERR_WIDTH, ERR_DISP, ERR_THREADS, ERR_UNIQUENESS, ERR_METHOD, ERR_WORKSPACE, ERR_ARG, ERR_CUDA = -1, -2, -3, -4, -5, -6, -7, -100
+# codes of the per-pixel match state (include/vppstereo_b200.h: VPPB200_STATE_*)
+STATE_MATCHED, STATE_INTERPOLATED, STATE_NO_MATCH, STATE_LR_REJECTED, STATE_BELOW_ONE, STATE_SPECKLE = 0, 1, 2, 3, 4, 5
 
 _lib = None
 
@@ -71,6 +73,10 @@ PROTOTYPES = {
     "vppb200_match_wta_uniq": (_i, (_p, _p, _i, _i, _i, _f, _i, _p)),
     "vppb200_match_wta_right_uniq": (_i, (_p, _p, _i, _i, _i, _f, _i, _p)),
     "vppb200_compute_rsgm_uniq": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _i, _i, _i, _taps, _prm, _f)),
+    # per-pixel match info
+    "vppb200_rsgm_info_workspace_bytes": (_sz, (_i, _i, _i, _i, _i, _i)),
+    "vppb200_compute_rsgm_info": (_i, (_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _sz, _i, _p, _i, _i, _i, _taps, _prm, _f,
+                                       _p, _p, _p)),
     # row bands
     "vppb200_banded_workspace_bytes": (_sz, (_i, _i, _i, _i)),
     "vppb200_banded_dims": (_i, (_i, _i, _i, _i, _p, _p, _p, _p)),

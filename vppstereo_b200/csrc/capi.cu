@@ -163,13 +163,15 @@ struct RsgmWs {
     uint16_t *S, *S_xyd;
     void *halo;
     float *dl, *dlf, *dr, *drf;
+    uint16_t *cost, *rival;                                   // the match info's padded maps (info layout only)
     TailBufs tail;
 };
 
 // `sets` buffer sets of everything that crosses a phase boundary (front -> main: guide, cost volume; main -> tail: raw
 // left/right disparities), so that the phases of neighbouring batches can run concurrently on different streams; `set`
-// selects the one this call uses.  Everything else is private to one phase and exists once.
-static size_t rsgm_ws_layout(const RsgmDims &d, int n, int sets, int set, void *base, RsgmWs *ws)
+// selects the one this call uses.  Everything else is private to one phase and exists once.  info: every set also holds the
+// padded cost / rival maps of the match info (main -> tail, like dl / dr); without it the layout is the one it always was.
+static size_t rsgm_ws_layout(const RsgmDims &d, int n, int sets, int set, void *base, RsgmWs *ws, bool info = false)
 {
     size_t off = 0;
     char *b = (char *)base;
@@ -180,12 +182,14 @@ static size_t rsgm_ws_layout(const RsgmDims &d, int n, int sets, int set, void *
     const size_t tv = tile_volume_elems(d.Wp, d.Hp, d.D, n);  // layout T pads the width to 32-column groups
     const size_t vol = tv > np * d.D ? tv : np * d.D;
     w.guide = nullptr; w.dsi = nullptr; w.dl = nullptr; w.dr = nullptr; w.census_l = nullptr; w.census_r = nullptr;
+    w.cost = nullptr; w.rival = nullptr;
     for (int k = 0; k < sets; k++) {
         uint8_t *guide = (uint8_t *)take(np), *dsi = (uint8_t *)take(vol);
         float *dl = (float *)take(np * 4), *dr = (float *)take(np * 4);
         // (the census images cross the front -> main boundary too: the forward sweep turns them into the cost volume)
         uint32_t *cl = (uint32_t *)take(np * 4), *cr = (uint32_t *)take(np * 4);
-        if (k == set) { w.guide = guide; w.dsi = dsi; w.dl = dl; w.dr = dr; w.census_l = cl; w.census_r = cr; }
+        uint16_t *cost = info ? (uint16_t *)take(np * 2) : nullptr, *rival = info ? (uint16_t *)take(np * 2) : nullptr;
+        if (k == set) { w.guide = guide; w.dsi = dsi; w.dl = dl; w.dr = dr; w.census_l = cl; w.census_r = cr; w.cost = cost; w.rival = rival; }
     }
     w.S = (uint16_t *)take(vol * 2);                          // the uint16 S (layout T)
     w.S_xyd = (uint16_t *)take(np * d.D * 2);                 // the reference's xyd order (WTA input, test tap)
@@ -447,11 +451,13 @@ extern "C" size_t vppb200_rsgm_workspace_bytes_sets(int H, int W, int C, int D, 
 // set), TAIL = median/interpolation/LR check/speckles/fills (reads those, writes disp_out).  One call may run any subset
 // on `stream`; a caller that runs the phases of neighbouring batches on different streams orders them with events
 // (vppstereo_b200/pipeline.py).  workspace must have been sized for `sets` sets.  uf: uniqueness factor of MAIN's WTA
-// (UNIQ_OFF = none).
+// (UNIQ_OFF = none).  state_out != NULL: the match info (all three outputs set, workspace in the info layout), produced by the
+// info instantiations of the fused sweep / WTA and of the left-view tail kernels; NULL: exactly the kernels of the plain pipeline.
 static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
                        const float *validhints, float *disp_out, int H, int W, int C, int D, int flags, const float *rcp_lut,
                        void *workspace, size_t workspace_bytes, int n, void *stream, const vppb200_rsgm_taps *taps, int phases,
-                       int sets, int set, const vppb200_sgm_params *params, uint32_t uf)
+                       int sets, int set, const vppb200_sgm_params *params, uint32_t uf, uint8_t *state_out = nullptr,
+                       uint16_t *cost_out = nullptr, uint16_t *rival_out = nullptr)
 {
     SgmParams prm;
     if (sgm_params_from(params, &prm)) return VPPB200_ERR_ARG;
@@ -465,12 +471,13 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
     if (taps && phases != 7) return VPPB200_ERR_ARG;
     const RsgmDims d = make_dims(H, W, C, D);
     if (d.Hp < 8) return VPPB200_ERR_ARG;
-    if (!workspace || workspace_bytes < rsgm_ws_layout(d, n, sets, 0, nullptr, nullptr)) return VPPB200_ERR_WORKSPACE;
+    const bool info = state_out != nullptr;
+    if (!workspace || workspace_bytes < rsgm_ws_layout(d, n, sets, 0, nullptr, nullptr, info)) return VPPB200_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     if (!rcp_lut) rcp_lut = device_rcp_lut(st);
     if (!rcp_lut) return cuda_fail("device_rcp_lut", cudaGetLastError());
     RsgmWs w;
-    rsgm_ws_layout(d, n, sets, set, workspace, &w);
+    rsgm_ws_layout(d, n, sets, set, workspace, &w, info);
     int rc;
     StageMarks tm;
     if (phases == 7) tm.begin(st);                           // per-stage timing covers whole-pipeline calls only
@@ -516,7 +523,7 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
             if (!want_volume) {
                 // the last sweep consumes the final S on the fly: WTA left (+ sub-pixel) and right come out of the aggregation
                 if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, w.dl, w.dr, rcp_lut, hints == nullptr, prm, &hook,
-                                                uf, st)))
+                                                uf, st, w.cost, w.rival)))
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
             } else {
                 if ((rc = launch_aggregate_tile(w.guide, w.dsi, w.S, w.halo, d.Wp, d.Hp, D, n, nullptr, nullptr, nullptr, hints == nullptr, prm,
@@ -524,12 +531,12 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
                     return rc < 0 ? rc : VPPB200_ERR_ARG;
                 if ((rc = launch_s_tile_to_xyd(w.S, w.S_xyd, d.Wp, d.Hp, D, n, st))) return rc;
                 S_final = w.S_xyd;
-                if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st))) return rc;
+                if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st, w.cost, w.rival))) return rc;
             }
         } else {
             if ((rc = launch_aggregate_generic(w.guide, w.dsi, w.S, d.Wp, d.Hp, D, prm, n, st))) return rc;
             tm.done(VPPB200_STAGE_SGM_H_BWD);                // the per-path fallback is booked on the last sweep's slot
-            if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st))) return rc;
+            if ((rc = launch_wta_both_subpix(S_final, w.dl, w.dr, d.Wp, d.Hp, D, rcp_lut, n, uf, st, w.cost, w.rival))) return rc;
         }
         tm.done(VPPB200_STAGE_WTA);
     }
@@ -540,11 +547,13 @@ static int rsgm_phases(const uint8_t *left, const uint8_t *left_vpp, const uint8
         if ((rc = launch_median(w.dr, w.drf, d.Wp, d.Hp, n, side))) return rc;
         if ((rc = launch_interp_clip(w.drf, d.Wp, d.Hp, n, side))) return rc;
         if ((rc = launch_median(w.dl, w.dlf, d.Wp, d.Hp, n, st))) return rc;
-        if ((rc = launch_interp_clip(w.dlf, d.Wp, d.Hp, n, st))) return rc;
+        if ((rc = info ? launch_interp_clip_info(w.dlf, d, n, state_out, st) : launch_interp_clip(w.dlf, d.Wp, d.Hp, n, st))) return rc;
         if (side != st && (rc = stream_chain(side, st))) return rc;
         tm.done(VPPB200_STAGE_MEDIAN_INTERP);
         // rsgm.py:275-292  crop, LR check, speckle filter, sub-pixel restore, background fill
-        if ((rc = launch_tail(w.dlf, w.drf, disp_out, d, flags & 1, w.tail, n, st))) return rc;
+        if ((rc = info ? launch_tail_info(w.dlf, w.drf, disp_out, d, flags & 1, w.tail, n, state_out, w.cost, w.rival, cost_out, rival_out, st)
+                       : launch_tail(w.dlf, w.drf, disp_out, d, flags & 1, w.tail, n, st)))
+            return rc;
         tm.done(VPPB200_STAGE_TAIL);
     }
     tm.end();
@@ -605,6 +614,27 @@ extern "C" int vppb200_compute_rsgm_uniq(const uint8_t *left, const uint8_t *lef
     if (rc) return rc;
     return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
                        workspace_bytes, n, stream, taps, phases, sets, set, params, uf);
+}
+
+extern "C" size_t vppb200_rsgm_info_workspace_bytes(int H, int W, int C, int D, int n, int sets)
+{
+    if (H <= 0 || W <= 0 || n <= 0 || D <= 0 || D % 8 || D > 256 || (C != 1 && C != 3) || sets < 1 || sets > 4) return 0;
+    return rsgm_ws_layout(make_dims(H, W, C, D), n, sets, 0, nullptr, nullptr, true);
+}
+
+extern "C" int vppb200_compute_rsgm_info(const uint8_t *left, const uint8_t *left_vpp, const uint8_t *right_vpp, const float *hints,
+                                         const float *validhints, float *disp_out, int H, int W, int C, int D, int flags,
+                                         const float *rcp_lut, void *workspace, size_t workspace_bytes, int n, void *stream,
+                                         int phases, int sets, int set, const vppb200_rsgm_taps *taps,
+                                         const vppb200_sgm_params *params, float uniqueness, uint8_t *state_out, uint16_t *cost_out,
+                                         uint16_t *rival_out)
+{
+    uint32_t uf;
+    const int rc = uniq_factor(uniqueness, &uf);
+    if (rc) return rc;
+    if (!state_out || !cost_out || !rival_out) return VPPB200_ERR_ARG;
+    return rsgm_phases(left, left_vpp, right_vpp, hints, validhints, disp_out, H, W, C, D, flags, rcp_lut, workspace,
+                       workspace_bytes, n, stream, taps, phases, sets, set, params, uf, state_out, cost_out, rival_out);
 }
 
 extern "C" int vppb200_sgm_params_fast(const vppb200_sgm_params *params, int guided)

@@ -132,9 +132,10 @@ struct StageHook { void (*fn)(void *, int); void *ctx; };   // called with VPPB2
 size_t sweep_halo_bytes(int W, int H, int D, int n);       // workspace of the v-sweep: inter-CTA halo lines, abort flag, P2 table
 // plain_costs: the costs are plain Hamming distances (<= 24, no guided modulation): un-normalised path state in the v-sweeps
 // p must satisfy sweep_params_supported(p, plain_costs)
+// info_cost / info_rival: NULL, or [n][H][W] outputs of the per-pixel match info (left best / least rival cost; needs dl)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost, uint16_t *S, void *halo_ws, int W, int H, int D, int n, float *dl,
                           float *dr, const float *lut, bool plain_costs, const SgmParams &p, const StageHook *hook, uint32_t uf,
-                          cudaStream_t st);
+                          cudaStream_t st, uint16_t *info_cost = nullptr, uint16_t *info_rival = nullptr);
 int sweep_take_abort_flag(int *out);
 int launch_s_tile_to_xyd(const uint16_t *St, uint16_t *Sx, int W, int H, int D, int n, cudaStream_t st);
 void sweep_set_max_strip(int cols);
@@ -143,9 +144,9 @@ void sweep_set_clusters(int c);
 void vpp_set_rows_kernel(int on);
 void vpp_set_md_wave(int on);
 int vpp_take_md_abort_flag(int *out);
-// uf: uniqueness factor (UNIQ_OFF = none)
+// uf: uniqueness factor (UNIQ_OFF = none); info_cost / info_rival as for launch_aggregate_tile
 int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
-                           cudaStream_t st);
+                           cudaStream_t st, uint16_t *info_cost = nullptr, uint16_t *info_rival = nullptr);
 int launch_wta_left(const uint16_t *S, float *disp, int W, int H, int D, int n, uint32_t uf, cudaStream_t st);
 int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n, uint32_t uf, cudaStream_t st);
 int launch_subpixel(const uint16_t *S, float *disp, int W, int H, int D, int method, const float *lut, int n, cudaStream_t st);
@@ -154,6 +155,11 @@ int launch_interp_clip(float *disp, int W, int H, int n, cudaStream_t st);   // 
 struct TailBufs { uint8_t *u8; int *label; int *count; };       // rows of tail_stride(W) elements
 static inline int tail_stride(int W) { return (W + 3) & ~3; }
 int launch_tail(const float *dl, const float *dr, float *out, const RsgmDims &d, int subpixel, TailBufs tb, int n, cudaStream_t st);
+// The per-pixel match info of the left view (include/vppstereo_b200.h): the same stages, each writing the part of the state it
+// decides.  state / cost_out / rival_out are cropped [n][H][W]; cost_pad / rival_pad the padded maps of the fused sweep or WTA.
+int launch_interp_clip_info(float *disp, const RsgmDims &d, int n, uint8_t *state, cudaStream_t st);
+int launch_tail_info(const float *dl, const float *dr, float *out, const RsgmDims &d, int subpixel, TailBufs tb, int n, uint8_t *state,
+                     const uint16_t *cost_pad, const uint16_t *rival_pad, uint16_t *cost_out, uint16_t *rival_out, cudaStream_t st);
 const float *device_rcp_lut(cudaStream_t st);   // library-owned table for this host CPU (lazy, per device)
 
 

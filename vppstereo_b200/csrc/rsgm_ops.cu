@@ -443,13 +443,16 @@ int launch_guided_u8(uint8_t *dsi, const float *hints, const float *valid, const
 //   sub-pixel (method 0, :1072-1102) optionally fused into the left result.
 //   UNIQ: the uniqueness ratio uf (common.cuh: uniq_accept; left: a second warp reduction over the rivals of the arg-min, right:
 //          the buckets carry uniq_absorb's state); a rejected pixel is -10 in both views.
+//   INFO: (with UNIQ, any uf) the left pixel's best cost and least rival cost also go to info_cost / info_rival [rows][W].
 // ------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int s_at(const uint16_t *Srow, int x, int d, int D) { return Srow[(long)x * D + d]; }
 
-template <int NW, bool LEFT, bool RIGHT, bool SUBPIX, bool UNIQ>
+template <int NW, bool LEFT, bool RIGHT, bool SUBPIX, bool UNIQ, bool INFO = false>
 __device__ __forceinline__ void wta_rows_body(const uint16_t *__restrict__ S, float *__restrict__ disp_l, float *__restrict__ disp_r,
-                                              int W, int H, int D, const float *__restrict__ lut, long total_rows, uint32_t uf)
+                                              int W, int H, int D, const float *__restrict__ lut, long total_rows, uint32_t uf,
+                                              uint16_t *__restrict__ info_cost = nullptr, uint16_t *__restrict__ info_rival = nullptr)
 {
+    static_assert(!INFO || (UNIQ && LEFT), "the match info is the left view's uniqueness candidates");
     const long row = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (row >= total_rows) return;
     const int lane = threadIdx.x & 31;
@@ -505,6 +508,10 @@ __device__ __forceinline__ void wta_rows_body(const uint16_t *__restrict__ S, fl
                 }
                 if (UNIQ && !uniq_accept(m, c2, end, uf)) out = -10.0f;
                 disp_l[row * W + x] = out;
+                if (INFO) {
+                    info_cost[row * W + x] = (uint16_t)(m >> 16);
+                    info_rival[row * W + x] = (uint16_t)c2;
+                }
             }
         }
         if (RIGHT) {
@@ -551,6 +558,15 @@ __global__ void __launch_bounds__(128) wta_rows_uniq_kernel(const uint16_t *__re
 {
     wta_rows_body<NW, LEFT, RIGHT, SUBPIX, true>(S, disp_l, disp_r, W, H, D, lut, total_rows, uf);
 }
+// wta_rows_uniq_kernel (any uf, UNIQ_OFF included) exporting the left view's match info (compute_rsgm's volume paths)
+template <int NW>
+__global__ void __launch_bounds__(128) wta_rows_info_kernel(const uint16_t *__restrict__ S, float *__restrict__ disp_l,
+                                                            float *__restrict__ disp_r, int W, int H, int D,
+                                                            const float *__restrict__ lut, long total_rows, uint32_t uf,
+                                                            uint16_t *__restrict__ info_cost, uint16_t *__restrict__ info_rival)
+{
+    wta_rows_body<NW, true, true, true, true, true>(S, disp_l, disp_r, W, H, D, lut, total_rows, uf, info_cost, info_rival);
+}
 
 template <bool LEFT, bool RIGHT, bool SUBPIX, bool UNIQ>
 static int launch_wta_u(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
@@ -589,9 +605,19 @@ int launch_wta_right(const uint16_t *S, float *disp, int W, int H, int D, int n,
     return launch_wta_t<false, true, false>(S, nullptr, disp, W, H, D, nullptr, n, uf, st);
 }
 int launch_wta_both_subpix(const uint16_t *S, float *dl, float *dr, int W, int H, int D, const float *lut, int n, uint32_t uf,
-                           cudaStream_t st)
+                           cudaStream_t st, uint16_t *info_cost, uint16_t *info_rival)
 {
-    return launch_wta_t<true, true, true>(S, dl, dr, W, H, D, lut, n, uf, st);
+    if (!info_cost) return launch_wta_t<true, true, true>(S, dl, dr, W, H, D, lut, n, uf, st);
+    const long rows = (long)n * H;
+    const int blocks = cdiv(rows * 32, 128);
+    switch ((D + 63) / 64) {
+        case 1: wta_rows_info_kernel<1><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows, uf, info_cost, info_rival); break;
+        case 2: wta_rows_info_kernel<2><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows, uf, info_cost, info_rival); break;
+        case 3: wta_rows_info_kernel<3><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows, uf, info_cost, info_rival); break;
+        default: wta_rows_info_kernel<4><<<blocks, 128, 0, st>>>(S, dl, dr, W, H, D, lut, rows, uf, info_cost, info_rival); break;
+    }
+    VPP_LAUNCH_CHECK("wta_rows_info_kernel");
+    return VPPB200_OK;
 }
 
 // subPixelRefine as a stand-alone operator (RSGM/StereoBMHelper.cpp:1065-1135), one thread per pixel
@@ -697,7 +723,12 @@ int launch_median(const float *src, float *dst, int W, int H, int n, cudaStream_
 // The rewritten anchors round back to themselves in float32, runs never chain (their anchors are original pixels), so
 // every pixel is independent: one warp stages a row in shared memory, all lanes resolve their pixels, coalesced write.
 // ------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) interp_clip_kernel(float *__restrict__ disp, int W, long total_rows)
+// INFO: the pixels of the crop [pt, pt+H) x [pl, pl+W) of state (cropped [n][H][W]) are set to VPPB200_STATE_INTERPOLATED where the
+// map was <= 0 before this step (the value, if positive now, came from the interpolation), VPPB200_STATE_MATCHED elsewhere; the
+// tail kernels overwrite the codes of the later stages.
+template <bool INFO>
+__device__ __forceinline__ void interp_clip_body(float *__restrict__ disp, int W, long total_rows, uint8_t *__restrict__ state,
+                                                 const RsgmDims &d)
 {
     extern __shared__ float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -728,7 +759,21 @@ __global__ void __launch_bounds__(128) interp_clip_kernel(float *__restrict__ di
             }
         }
         g[x] = fmaxf(v, 0.0f);
+        if (INFO) {
+            const int y = (int)(row % d.Hp) - d.pt, xc = x - d.pl;
+            if (y >= 0 && y < d.H && xc >= 0 && xc < d.W)
+                state[((row / d.Hp) * d.H + y) * d.W + xc] = r[x] <= 0 ? VPPB200_STATE_INTERPOLATED : VPPB200_STATE_MATCHED;
+        }
     }
+}
+__global__ void __launch_bounds__(128) interp_clip_kernel(float *__restrict__ disp, int W, long total_rows)
+{
+    interp_clip_body<false>(disp, W, total_rows, nullptr, RsgmDims{});
+}
+__global__ void __launch_bounds__(128) interp_clip_info_kernel(float *__restrict__ disp, long total_rows, uint8_t *__restrict__ state,
+                                                               RsgmDims d)
+{
+    interp_clip_body<true>(disp, d.Wp, total_rows, state, d);
 }
 int launch_interp_clip(float *disp, int W, int H, int n, cudaStream_t st)
 {
@@ -738,6 +783,16 @@ int launch_interp_clip(float *disp, int W, int H, int n, cudaStream_t st)
     if (sm > 48 * 1024) VPP_CUDA_TRY(cudaFuncSetAttribute(interp_clip_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     interp_clip_kernel<<<cdiv(rows, wpb), wpb * 32, sm, st>>>(disp, W, rows);
     VPP_LAUNCH_CHECK("interp_clip_kernel");
+    return VPPB200_OK;
+}
+int launch_interp_clip_info(float *disp, const RsgmDims &d, int n, uint8_t *state, cudaStream_t st)
+{
+    const long rows = (long)n * d.Hp;
+    const int wpb = 4;
+    const size_t sm = (size_t)wpb * d.Wp * sizeof(float);
+    if (sm > 48 * 1024) VPP_CUDA_TRY(cudaFuncSetAttribute(interp_clip_info_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    interp_clip_info_kernel<<<cdiv(rows, wpb), wpb * 32, sm, st>>>(disp, rows, state, d);
+    VPP_LAUNCH_CHECK("interp_clip_info_kernel");
     return VPPB200_OK;
 }
 
@@ -758,9 +813,11 @@ __device__ __forceinline__ bool spk_conn(int a, int b) { return a && b && abs(a 
 
 // rows: crop + _left_right_check(th=1) + zero mask==128 + astype(uint8) (rsgm.py:229-248,:275-284) fused with the run labelling: the warp that labels a row
 // produces the row's uint8 map itself (one pass over the two disparity rows instead of a kernel and a round trip of the map)
-__global__ void __launch_bounds__(128) speckle_rows_kernel(const float *__restrict__ dl, const float *__restrict__ dr,
-                                                           uint8_t *__restrict__ u8, int *__restrict__ label,
-                                                           int *__restrict__ count, RsgmDims d, int Ws, long total_rows)
+// INFO: state (cropped [n][H][W]) gets the code of the step that zeroes a pixel here: NO_MATCH (not positive), LR_REJECTED, BELOW_ONE
+template <bool INFO>
+__device__ __forceinline__ void speckle_rows_body(const float *__restrict__ dl, const float *__restrict__ dr, uint8_t *__restrict__ u8,
+                                                  int *__restrict__ label, int *__restrict__ count, const RsgmDims &d, int Ws,
+                                                  long total_rows, uint8_t *__restrict__ state)
 {
     const long row = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (row >= total_rows) return;
@@ -778,17 +835,21 @@ __global__ void __launch_bounds__(128) speckle_rows_kernel(const float *__restri
         int v = 0;
         if (x < W) {
             float fv = lrow[x];
+            int code = VPPB200_STATE_NO_MATCH;
             if (fv > 0) {
+                code = VPPB200_STATE_BELOW_ONE;
                 const int dd = __float2int_rn(fv);   // numba round(): half to even (rsgm.py:237)
                 const int xd = x - dd;
                 if (xd >= 0 && xd <= W - 1) {
                     const float r = rrow[xd];
-                    if (r > 0 && fabsf(__fsub_rn(fv, r)) > 1.0f) fv = 0.0f;
+                    if (r > 0 && fabsf(__fsub_rn(fv, r)) > 1.0f) { fv = 0.0f; code = VPPB200_STATE_LR_REJECTED; }
                 } else {
                     fv = 0.0f;
+                    code = VPPB200_STATE_LR_REJECTED;
                 }
             }
             v = (int)(uint8_t)fv;
+            if (INFO && !v) state[row * W + x] = (uint8_t)code;
         }
         int left = __shfl_up_sync(0xFFFFFFFFu, v, 1);
         if (lane == 0) left = prev_last;
@@ -807,6 +868,19 @@ __global__ void __launch_bounds__(128) speckle_rows_kernel(const float *__restri
             count[base + x] = 0;
         }
     }
+}
+__global__ void __launch_bounds__(128) speckle_rows_kernel(const float *__restrict__ dl, const float *__restrict__ dr,
+                                                           uint8_t *__restrict__ u8, int *__restrict__ label,
+                                                           int *__restrict__ count, RsgmDims d, int Ws, long total_rows)
+{
+    speckle_rows_body<false>(dl, dr, u8, label, count, d, Ws, total_rows, nullptr);
+}
+__global__ void __launch_bounds__(128) speckle_rows_info_kernel(const float *__restrict__ dl, const float *__restrict__ dr,
+                                                                uint8_t *__restrict__ u8, int *__restrict__ label,
+                                                                int *__restrict__ count, RsgmDims d, int Ws, long total_rows,
+                                                                uint8_t *__restrict__ state)
+{
+    speckle_rows_body<true>(dl, dr, u8, label, count, d, Ws, total_rows, state);
 }
 
 __device__ __forceinline__ int uf_find(const int *L, int i)
@@ -902,9 +976,14 @@ __global__ void __launch_bounds__(256) speckle_count_kernel(const uint8_t *__res
     }
 }
 // apply the speckle verdict, restore sub-pixel values (rsgm.py:286-290) and write the float frame
-__global__ void speckle_apply_kernel(const uint8_t *__restrict__ u8, const int *__restrict__ label, const int *__restrict__ count,
-                                     const float *__restrict__ dl, float *__restrict__ out, RsgmDims d, int Ws, int subpixel,
-                                     long total)
+// INFO: a speckle gets VPPB200_STATE_SPECKLE (every other code is already in state), and the padded cost / rival maps are cropped
+// into cost_out / rival_out
+template <bool INFO>
+__device__ __forceinline__ void speckle_apply_body(const uint8_t *__restrict__ u8, const int *__restrict__ label,
+                                                   const int *__restrict__ count, const float *__restrict__ dl, float *__restrict__ out,
+                                                   const RsgmDims &d, int Ws, int subpixel, long total, uint8_t *__restrict__ state,
+                                                   const uint16_t *__restrict__ cost_pad, const uint16_t *__restrict__ rival_pad,
+                                                   uint16_t *__restrict__ cost_out, uint16_t *__restrict__ rival_out)
 {
     long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= total) return;
@@ -916,11 +995,33 @@ __global__ void speckle_apply_kernel(const uint8_t *__restrict__ u8, const int *
     if (b) {
         const int start = label[ts];                  // a non-start pixel still holds its run start
         const int root = uf_find(label, start);
-        if (count[root] <= 200) b = 0;
+        if (count[root] <= 200) {
+            b = 0;
+            if (INFO) state[t] = VPPB200_STATE_SPECKLE;
+        }
     }
     float v = (float)b;
     if (subpixel && b) v = dl[(f * d.Hp + y + d.pt) * d.Wp + d.pl + x];
     out[t] = v;
+    if (INFO) {
+        const long tp = (f * d.Hp + y + d.pt) * d.Wp + d.pl + x;
+        cost_out[t] = cost_pad[tp];
+        rival_out[t] = rival_pad[tp];
+    }
+}
+__global__ void speckle_apply_kernel(const uint8_t *__restrict__ u8, const int *__restrict__ label, const int *__restrict__ count,
+                                     const float *__restrict__ dl, float *__restrict__ out, RsgmDims d, int Ws, int subpixel,
+                                     long total)
+{
+    speckle_apply_body<false>(u8, label, count, dl, out, d, Ws, subpixel, total, nullptr, nullptr, nullptr, nullptr, nullptr);
+}
+__global__ void speckle_apply_info_kernel(const uint8_t *__restrict__ u8, const int *__restrict__ label, const int *__restrict__ count,
+                                          const float *__restrict__ dl, float *__restrict__ out, RsgmDims d, int Ws, int subpixel,
+                                          long total, uint8_t *__restrict__ state, const uint16_t *__restrict__ cost_pad,
+                                          const uint16_t *__restrict__ rival_pad, uint16_t *__restrict__ cost_out,
+                                          uint16_t *__restrict__ rival_out)
+{
+    speckle_apply_body<true>(u8, label, count, dl, out, d, Ws, subpixel, total, state, cost_pad, rival_pad, cost_out, rival_out);
 }
 
 // _interpolate_background rows (rsgm.py:188-213).  Closed form of the sequential scan (exact): an invalid run with valid
@@ -980,7 +1081,10 @@ __global__ void bg_cols_kernel(float *__restrict__ img, int W, int H, long total
         if (col[(long)v * W] > 0) { const float f = col[(long)v * W]; for (int v2 = v + 1; v2 < H; v2++) col[(long)v2 * W] = f; break; }
 }
 
-int launch_tail(const float *dl, const float *dr, float *out, const RsgmDims &d, int subpixel, TailBufs tb, int n, cudaStream_t st)
+// info: NULL (the default launches) or the match info's outputs (launch_tail_info)
+struct TailInfo { uint8_t *state; const uint16_t *cost_pad, *rival_pad; uint16_t *cost_out, *rival_out; };
+static int tail_impl(const float *dl, const float *dr, float *out, const RsgmDims &d, int subpixel, TailBufs tb, int n,
+                     const TailInfo *info, cudaStream_t st)
 {
     const long total = (long)n * d.H * d.W;
     if ((long)n * d.H * tail_stride(d.W) >= (1L << 31)) return VPPB200_ERR_ARG;
@@ -989,15 +1093,26 @@ int launch_tail(const float *dl, const float *dr, float *out, const RsgmDims &d,
     const long quads = (long)n * d.H * (Ws >> 2);
     {
         const long nrows = (long)n * d.H;
-        speckle_rows_kernel<<<cdiv(nrows * 32, 128), 128, 0, st>>>(dl, dr, tb.u8, tb.label, tb.count, d, Ws, nrows);
-        VPP_LAUNCH_CHECK("speckle_rows_kernel");
+        if (info) {
+            speckle_rows_info_kernel<<<cdiv(nrows * 32, 128), 128, 0, st>>>(dl, dr, tb.u8, tb.label, tb.count, d, Ws, nrows, info->state);
+            VPP_LAUNCH_CHECK("speckle_rows_info_kernel");
+        } else {
+            speckle_rows_kernel<<<cdiv(nrows * 32, 128), 128, 0, st>>>(dl, dr, tb.u8, tb.label, tb.count, d, Ws, nrows);
+            VPP_LAUNCH_CHECK("speckle_rows_kernel");
+        }
     }
     speckle_merge_kernel<<<cdiv(quads, 256), 256, 0, st>>>(tb.u8, tb.label, d.W, Ws, d.H, quads);
     VPP_LAUNCH_CHECK("speckle_merge_kernel");
     speckle_count_kernel<<<cdiv(quads, 256), 256, 0, st>>>(tb.u8, tb.label, tb.count, d.W, Ws, quads);
     VPP_LAUNCH_CHECK("speckle_count_kernel");
-    speckle_apply_kernel<<<blocks, 256, 0, st>>>(tb.u8, tb.label, tb.count, dl, out, d, Ws, subpixel, total);
-    VPP_LAUNCH_CHECK("speckle_apply_kernel");
+    if (info) {
+        speckle_apply_info_kernel<<<blocks, 256, 0, st>>>(tb.u8, tb.label, tb.count, dl, out, d, Ws, subpixel, total, info->state,
+                                                          info->cost_pad, info->rival_pad, info->cost_out, info->rival_out);
+        VPP_LAUNCH_CHECK("speckle_apply_info_kernel");
+    } else {
+        speckle_apply_kernel<<<blocks, 256, 0, st>>>(tb.u8, tb.label, tb.count, dl, out, d, Ws, subpixel, total);
+        VPP_LAUNCH_CHECK("speckle_apply_kernel");
+    }
     const long rows = (long)n * d.H;
     const int wpb = 4;
     const size_t sm = (size_t)wpb * 2 * d.W * sizeof(float);
@@ -1008,6 +1123,16 @@ int launch_tail(const float *dl, const float *dr, float *out, const RsgmDims &d,
     bg_cols_kernel<<<cdiv(cols, 128), 128, 0, st>>>(out, d.W, d.H, cols);
     VPP_LAUNCH_CHECK("bg_cols_kernel");
     return VPPB200_OK;
+}
+int launch_tail(const float *dl, const float *dr, float *out, const RsgmDims &d, int subpixel, TailBufs tb, int n, cudaStream_t st)
+{
+    return tail_impl(dl, dr, out, d, subpixel, tb, n, nullptr, st);
+}
+int launch_tail_info(const float *dl, const float *dr, float *out, const RsgmDims &d, int subpixel, TailBufs tb, int n, uint8_t *state,
+                     const uint16_t *cost_pad, const uint16_t *rival_pad, uint16_t *cost_out, uint16_t *rival_out, cudaStream_t st)
+{
+    const TailInfo info{state, cost_pad, rival_pad, cost_out, rival_out};
+    return tail_impl(dl, dr, out, d, subpixel, tb, n, &info, st);
 }
 
 }  // namespace vppb200

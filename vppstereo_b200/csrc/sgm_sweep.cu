@@ -343,14 +343,18 @@ __device__ __forceinline__ uint32_t &u4c(uint4 &v, int i) { return i == 0 ? v.x 
 // FULLK: K2 == NW * 32, every lane's NW words are real disparities (no validity selects)
 // MODE 3 (opt-in): MODE 2 with the uniqueness ratio uf < UNIQ_OFF (common.cuh: uniq_accept); a rejected pixel is -10 in both
 // views.  The right conveyor carries three times the state.  uf rides in the upper half of `total_rows` (a launch has fewer than
-// 2^31 rows), so that the instantiations of MODE 0..2 keep the signature and the code they had before the opt-in existed.
+// 2^31 rows), so that the instantiations of MODE 0..2 keep the code they had before the opt-in existed.
+// MODE 4 (opt-in, per-pixel match info): MODE 3 (uf may be UNIQ_OFF) that also stores each left pixel's best cost and least rival
+// cost into info_cost / info_rival [rows][W] (the uniqueness test's c[b] and c2, include/vppstereo_b200.h); the other modes
+// never read the two pointers.
 template <int NW, int MODE, int DIR, bool FULLK>
 __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__restrict__ img, const uint16_t *__restrict__ cost,
                                                             uint32_t *__restrict__ S, TL t, long total_rows,
                                                             float *__restrict__ disp_l, float *__restrict__ disp_r,
-                                                            const float *__restrict__ lut, SgmParams prm)
+                                                            const float *__restrict__ lut, SgmParams prm,
+                                                            uint16_t *__restrict__ info_cost, uint16_t *__restrict__ info_rival)
 {
-    constexpr bool STORE = MODE == 0, WTA = MODE >= 2, UNIQ = MODE == 3;
+    constexpr bool STORE = MODE == 0, WTA = MODE >= 2, UNIQ = MODE >= 3, INFO = MODE == 4;
     static_assert(!WTA || DIR < 0, "the fused WTA rides the backward sweep");
     extern __shared__ __align__(16) uint8_t hsm[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -613,6 +617,10 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
                 }
                 disp_l[row * W + x] = o;
                 disp_r[row * W + x] = orr;
+                if (INFO) {
+                    info_cost[row * W + x] = (uint16_t)(m >> 16);
+                    info_rival[row * W + x] = (uint16_t)wout[16 + lane];
+                }
             }
             carry = __shfl_sync(0xFFFFFFFFu, s0[0].x, 0) & 0xFFFFu;         // S(d = 0) of the chunk's first column
         } else {
@@ -640,28 +648,32 @@ __global__ void __launch_bounds__(HWARPS * 32) sgm_h_kernel(const uint8_t *__res
 
 template <int NW, int MODE, int DIR>
 static int run_h_t(const uint8_t *img, const uint16_t *cost, uint32_t *S, const TL &t, int n, float *dl, float *dr,
-                   const float *lut, const SgmParams &prm, uint32_t uf, cudaStream_t st)
+                   const float *lut, const SgmParams &prm, uint32_t uf, cudaStream_t st, uint16_t *info_cost = nullptr,
+                   uint16_t *info_rival = nullptr)
 {
     const long rows = (long)n * t.H;
-    if (MODE == 3 && rows >= (1L << 31)) return VPPB200_ERR_ARG;      // uf rides in the upper half of total_rows
+    if (MODE >= 3 && rows >= (1L << 31)) return VPPB200_ERR_ARG;      // uf rides in the upper half of total_rows
     const int blocks = cdiv(rows, HWARPS);
     const size_t stage = MODE >= 2 ? (size_t)t.K2 * (HCROW + HSROW_WTA) : h_stage_bytes(t.K2);
-    const size_t smem = (size_t)HWARPS * 2 * stage + (MODE >= 2 ? (size_t)HWARPS * (MODE == 3 ? 32 : 16) * 4 : 0);
+    const size_t smem = (size_t)HWARPS * 2 * stage + (MODE >= 2 ? (size_t)HWARPS * (MODE >= 3 ? 32 : 16) * 4 : 0);
     auto kern = t.K2 == NW * 32 ? sgm_h_kernel<NW, MODE, DIR, true> : sgm_h_kernel<NW, MODE, DIR, false>;
     if (smem > 48 * 1024) VPP_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<blocks, HWARPS * 32, smem, st>>>(img, cost, S, t, MODE == 3 ? rows | (long)uf << 32 : rows, dl, dr, lut, prm);
+    kern<<<blocks, HWARPS * 32, smem, st>>>(img, cost, S, t, MODE >= 3 ? rows | (long)uf << 32 : rows, dl, dr, lut, prm, info_cost,
+                                            info_rival);
     VPP_LAUNCH_CHECK("sgm_h_kernel");
     return VPPB200_OK;
 }
 
 // mode 0: forward sweep, S = L;  mode 1: backward sweep, S += L;  mode 2: backward sweep fused with WTA (dl, dr, lut), with the
-// uniqueness ratio (mode 3) when uf < UNIQ_OFF
+// uniqueness ratio (mode 3) when uf < UNIQ_OFF, and with the per-pixel match info (mode 4, any uf) when info_cost != NULL
 static int run_h(const uint8_t *img, const uint16_t *cost, uint32_t *S, const TL &t, int mode, int n, float *dl, float *dr,
-                 const float *lut, const SgmParams &prm, uint32_t uf, cudaStream_t st)
+                 const float *lut, const SgmParams &prm, uint32_t uf, cudaStream_t st, uint16_t *info_cost = nullptr,
+                 uint16_t *info_rival = nullptr)
 {
 #define VPP_RUN_H(NW)                                                                                                  \
     return mode == 0 ? run_h_t<NW, 0, 1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, UNIQ_OFF, st)             \
          : mode == 1 ? run_h_t<NW, 1, -1>(img, cost, S, t, n, nullptr, nullptr, nullptr, prm, UNIQ_OFF, st)            \
+         : info_cost ? run_h_t<NW, 4, -1>(img, cost, S, t, n, dl, dr, lut, prm, uf, st, info_cost, info_rival)          \
          : uf < UNIQ_OFF ? run_h_t<NW, 3, -1>(img, cost, S, t, n, dl, dr, lut, prm, uf, st)                            \
                          : run_h_t<NW, 2, -1>(img, cost, S, t, n, dl, dr, lut, prm, UNIQ_OFF, st)
     switch ((t.K2 + 31) / 32) {
@@ -1444,7 +1456,8 @@ static bool v_norm(bool plain_costs, int H, const SgmParams &p)
 
 // 0 = done; 1 = this shape does not fit the sweep (caller uses sgm.cu); < 0 = error.
 // dl != NULL: the last sweep is fused with the winner-takes-all step (left + sub-pixel into dl, right into dr) and the
-// final S is never written; dl == NULL: S holds the aggregated volume in layout T.
+// final S is never written; dl == NULL: S holds the aggregated volume in layout T.  info_cost != NULL (with dl): the fused sweep
+// also stores every left pixel's best and least rival cost into info_cost / info_rival [n][H][W] (sgm_h_kernel MODE 4).
 // plain_costs: the costs are plain Hamming distances (<= 24, no guided modulation): the v-sweeps keep their path state
 // un-normalised (see sgm_v2_kernel).
 // (Two variants of round 1 were measured again on this kernel generation and removed: uint8 partial-sum volumes instead of one
@@ -1456,7 +1469,7 @@ static bool v_norm(bool plain_costs, int H, const SgmParams &p)
 // 6.78 ms: step 22.3 vs 22.0 ms.)
 int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S16, void *halo_ws, int W, int H, int D, int n,
                           float *dl, float *dr, const float *lut, bool plain_costs, const SgmParams &prm, const StageHook *hook,
-                          uint32_t uf, cudaStream_t st)
+                          uint32_t uf, cudaStream_t st, uint16_t *info_cost, uint16_t *info_rival)
 {
     if (!sweep_params_supported(prm, plain_costs)) return VPPB200_ERR_ARG;
     const TL t = make_tl(W, H, D);
@@ -1480,7 +1493,7 @@ int launch_aggregate_tile(const uint8_t *img, const uint8_t *cost8, uint16_t *S1
     done(VPPB200_STAGE_SGM_V_DOWN);
     if ((rc = sweep(1))) return rc;
     done(VPPB200_STAGE_SGM_V_UP);
-    if ((rc = run_h(img, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, uf, st))) return rc;
+    if ((rc = run_h(img, cost, S, t, dl ? 2 : 1, n, dl, dr, lut, prm, uf, st, dl ? info_cost : nullptr, info_rival))) return rc;
     done(VPPB200_STAGE_SGM_H_BWD);
     return VPPB200_OK;
 }

@@ -18,6 +18,9 @@ maskocc: g_occ = occlusion_heuristic(hints)[1] with the reference's default para
 device; the adaptive patches' operands (bilateral filling, distance-based patch thresholds) are computed on the device too, so
 no option adds a host round trip to run_device.
 
+    pipe = VppRsgmPipeline(H, W, match_info=True)               # + how every left pixel was produced (rsgm.compute_rsgm's info)
+    disp, info = pipe.run_device(left_u8, right_u8, hints_f32)  # info = {"state": uint8, "cost", "rival": uint16 storage} [N,H,W]
+
 Three phases of neighbouring batches run concurrently on three internal streams (software pipeline across calls):
   front(k+1) = [occlusion mask, adaptive-patch operands] + VPP + pad/gray/census/cost volume
   main(k) = 8-path SGM sweeps + WTA   |   tail(k-1) = median ... fills
@@ -44,7 +47,7 @@ class VppRsgmPipeline:
                  interpolate=True, subpixel=True, device=None, seed=1234, sgm_params=None, guided=False, uniqueness=None,
                  method="rnd", wsizeAgg_x=64, wsizeAgg_y=3, discard_occ=False, uniform_color=False, use_distance_patch=False,
                  distance_gamma=0.3, use_bilateral_patch=False, bilateral_o_xy=2, bilateral_o_i=1, bilateral_th=.001,
-                 maskocc=False):
+                 maskocc=False, match_info=False):
         # sgm_params: (p1, p2min, alpha, gamma) honoured by the matcher; None = the reference's effective values (7, 17, 0.25, 50)
         # guided: the matcher is compute_rsgm(left, lv, rv, hints, validhints) -- every entry point then takes `validhints`
         # (float32 [N,H,W], placed like `hints`).  Parameters outside the guided sweep domain run on the per-path kernels.
@@ -55,6 +58,8 @@ class VppRsgmPipeline:
         # use_distance_patch: a batch with a frame whose hints all have one value has no reference output (the reference raises
         # ZeroDivisionError); that frame is projected with patch size 1 and check() / run_host() / collect() raise
         # ZeroDivisionError for it (see _raise_degenerate)
+        # match_info: every entry point also returns the per-pixel match info of compute_rsgm(..., return_info=True) (state uint8,
+        # cost / rival uint16 as _lib.u16_dtype() storage, [N,H,W]); run_device / run_device_serial then take `info_out`
         if method not in ("rnd", "maxDistance"):
             raise ValueError(f"method: expected 'rnd' or 'maxDistance', got {method!r}")
         for name, v in (("wsize", wsize), ("wsizeAgg_x", wsizeAgg_x), ("wsizeAgg_y", wsizeAgg_y)):
@@ -69,6 +74,7 @@ class VppRsgmPipeline:
         self.sgm_params = None if sgm_params is None else _lib.sgm_params(*sgm_params)
         self.uniqueness = 1.0 if uniqueness is None else _lib.uniqueness(uniqueness, "VppRsgmPipeline")
         self.guided = bool(guided)
+        self.match_info = bool(match_info)
         torch = _lib.require_cuda()
         self.torch = torch
         self.H, self.W, self.C, self.N, self.D = int(H), int(W), int(channels), int(batch), int(dmax)
@@ -85,8 +91,8 @@ class VppRsgmPipeline:
         self.calls = 0                                # buffer-set parity
         L = _lib.lib()
         with torch.cuda.device(self.device):
-            self.ws_rsgm = torch.empty(L.vppb200_rsgm_workspace_bytes_sets(self.H, self.W, self.C, self.D, self.N, 2),
-                                       dtype=torch.uint8, device=self.device)
+            ws_bytes = (L.vppb200_rsgm_info_workspace_bytes if self.match_info else L.vppb200_rsgm_workspace_bytes_sets)
+            self.ws_rsgm = torch.empty(ws_bytes(self.H, self.W, self.C, self.D, self.N, 2), dtype=torch.uint8, device=self.device)
             ws_vpp = L.vppb200_vpp_workspace_bytes(self.H, self.W, self.C, self.N)
             if self.method == "maxDistance":     # + the row wavefront's dependency table
                 ws_vpp = max(ws_vpp, L.vppb200_vpp_max_dist_workspace_bytes(self.H, self.W, self.C, self.wsize, self.wsize_agg[1],
@@ -133,6 +139,8 @@ class VppRsgmPipeline:
             self.d_hints = torch.empty((self.N, self.H, self.W), dtype=torch.float32, device=self.device)
             self.d_valid = torch.empty_like(self.d_hints) if self.guided else None
             self.h_disp = torch.empty((self.N, self.H, self.W), dtype=torch.float32).pin_memory()
+            self.info = self._info_buffers(self.device) if self.match_info else None       # run_device's default info_out
+            self.h_info = self._info_buffers("cpu") if self.match_info else None           # run_host's pinned copies
             self._stream_sets = None                  # created by the first submit_host
             self.host_depth = 3                       # staging sets of the streaming host API
             # the zero-filled occlusion mask / status and the tables above were queued on the constructing stream, while the
@@ -190,13 +198,28 @@ class VppRsgmPipeline:
         raise ZeroDivisionError(f"division by zero: every hint of frame {f} of {which} has the same disparity "
                                 "(use_distance_patch); that batch's output is not the reference's")
 
+    _INFO = (("state", "uint8"), ("cost", "int16"), ("rival", "int16"))       # info maps and their torch storage (uint16 as int16)
+
+    def _info_buffers(self, device):
+        torch = self.torch
+        return {k: (torch.empty((self.N, self.H, self.W), dtype=getattr(torch, dt), device=device) if device != "cpu" else
+                    torch.empty((self.N, self.H, self.W), dtype=getattr(torch, dt)).pin_memory()) for k, dt in self._INFO}
+
+    @staticmethod
+    def _info_slice(info, N):
+        return {k: t[:N] for k, t in info.items()}
+
     def workspace_bytes(self):
         return self.ws_rsgm.numel() + self.ws_vpp.numel() + (self.ws_occ.numel() if self.ws_occ is not None else 0)
 
-    def _check(self, left, right, hints, out=None, host=False, validhints=None):
+    def _check(self, left, right, hints, out=None, host=False, validhints=None, info_out=None):
         """Operand validation shared by every entry point: the kernels receive raw pointers, so a wrong dtype, shape, device
         or a non-contiguous view would be read as garbage or out of bounds.  Returns the batch size."""
         torch = self.torch
+        if info_out is not None and not self.match_info:
+            raise ValueError("info_out: given to a pipeline without match info (construct it with match_info=True)")
+        if info_out is not None and (not isinstance(info_out, dict) or set(info_out) != {k for k, _ in self._INFO}):
+            raise TypeError(f"info_out: expected a dict with the keys {[k for k, _ in self._INFO]}")
         if self.guided and validhints is None:
             raise ValueError("validhints: required by a guided pipeline (guided=True)")
         if not self.guided and validhints is not None:
@@ -218,6 +241,11 @@ class VppRsgmPipeline:
             if not isinstance(out, torch.Tensor):
                 raise TypeError("out: expected a torch tensor")
             want += (("out", out, torch.float32, (N, self.H, self.W)),)
+        if info_out is not None:
+            for k, dt in self._INFO:
+                if not isinstance(info_out[k], torch.Tensor):
+                    raise TypeError(f"info_out[{k!r}]: expected a torch tensor")
+                want += ((f"info_out[{k!r}]", info_out[k], getattr(torch, dt), (N, self.H, self.W)),)
         for name, t, dt, shape in want:
             if t.dtype != dt:
                 raise TypeError(f"{name}: expected {dt}, got {t.dtype}")
@@ -283,16 +311,24 @@ class VppRsgmPipeline:
             ev.record(stream)
             self._stage_marks.append((name, ev))
 
-    def _phase(self, phases, b, left, lv, rv, out, N, stream, hints, validhints):
-        # hints / validhints go to every phase of a guided batch (their nullness selects the sweeps' state); FRONT reads them
+    def _phase(self, phases, b, left, lv, rv, out, N, stream, hints, validhints, info=None):
+        # hints / validhints go to every phase of a guided batch (their nullness selects the sweeps' state); FRONT reads them;
+        # info (match_info): the same three maps in every phase of a batch (MAIN fills set b's cost maps, TAIL writes them)
         h, v = (_lib.ptr(hints), _lib.ptr(validhints)) if self.guided else (None, None)
-        _lib.call("vppb200_compute_rsgm_uniq", _lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W,
-                  self.C, self.D, 1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm), self.ws_rsgm.numel(), N,
-                  stream.cuda_stream, phases, 2, b, None, self.sgm_params, self.uniqueness, what="compute_rsgm_phases")
+        args = (_lib.ptr(left), _lib.ptr(lv), _lib.ptr(rv), h, v, _lib.ptr(out), self.H, self.W, self.C, self.D,
+                1 if self.subpixel else 0, None, _lib.ptr(self.ws_rsgm), self.ws_rsgm.numel(), N, stream.cuda_stream, phases, 2, b,
+                None, self.sgm_params, self.uniqueness)
+        if self.match_info:
+            _lib.call("vppb200_compute_rsgm_info", *args, *(_lib.ptr(info[k]) for k, _ in self._INFO), what="compute_rsgm_phases")
+        else:
+            _lib.call("vppb200_compute_rsgm_uniq", *args, what="compute_rsgm_phases")
 
-    def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None, validhints=None):
+    def run_device(self, left, right, hints, out=None, inputs_ready=None, step=None, validhints=None, info_out=None):
         """VPP (in copies) + compute_rsgm; all operands CUDA tensors [N,H,W,C] uint8 / [N,H,W] float32.
         `validhints` (guided pipelines only, required there): compute_rsgm(left, lv, rv, hints, validhints).
+        match_info pipelines return (out, info): info = `info_out` (a dict like the pipeline's own, see __init__) or the
+        pipeline's own buffers, valid in current-stream order like `out` (and like the default `out`, overwritten by the
+        next call); `info_out` to a pipeline without match_info: ValueError.
 
         The work is queued on the pipeline's three streams (front / main / tail, see the module docstring) and the caller's
         current stream is made to wait for the result, so `out` is valid in current-stream order like the output of any
@@ -303,11 +339,18 @@ class VppRsgmPipeline:
         (`self.front_done[k & 1]` of call k).
         `step`: explicit call number for the pattern seed (default: the pipeline's own counter, 1, 2, ...)."""
         torch = self.torch
-        N = self._check(left, right, hints, out, validhints=validhints)
+        N = self._check(left, right, hints, out, validhints=validhints, info_out=info_out)
         with torch.cuda.device(self.device):
-            return self._run_device(left, right, hints, validhints, out, inputs_ready, step, N, self.status)
+            info = self._info_out(info_out, N)
+            out = self._run_device(left, right, hints, validhints, out, inputs_ready, step, N, self.status, info)
+            return (out, info) if self.match_info else out
 
-    def _run_device(self, left, right, hints, validhints, out, inputs_ready, step, N, status):
+    def _info_out(self, info_out, N):
+        if not self.match_info:
+            return None
+        return self._info_slice(self.info, N) if info_out is None else info_out
+
+    def _run_device(self, left, right, hints, validhints, out, inputs_ready, step, N, status, info=None):
         torch = self.torch
         out = self.disp[:N] if out is None else out
         caller = torch.cuda.current_stream(self.device)
@@ -333,36 +376,38 @@ class VppRsgmPipeline:
         with torch.cuda.stream(front):
             lv.copy_(left); rv.copy_(right)              # vpp() returns copies (vpp_standalone.py:397)
             self._vpp(left, lv, rv, hints, seed, N, front, status)
-            self._phase(1, b, left, lv, rv, out, N, front, hints, validhints)
+            self._phase(1, b, left, lv, rv, out, N, front, hints, validhints, info)
             self.front_done[b].record(front)
         # ---- main: the four SGM sweeps + WTA (the critical stream)
         main.wait_event(self.front_done[b])
         if self.tail_done[b] is not None:
             main.wait_event(self.tail_done[b])           # raw disparities of set b were last read by the tail two calls ago
         with torch.cuda.stream(main):
-            self._phase(2, b, left, lv, rv, out, N, main, hints, validhints)
+            self._phase(2, b, left, lv, rv, out, N, main, hints, validhints, info)
             ev = torch.cuda.Event(); ev.record(main)
             self.main_done[b] = ev
         # ---- tail: everything after WTA; `out` may still be read by work the caller queued before this call
         tail.wait_stream(caller)
         tail.wait_event(self.main_done[b])
         with torch.cuda.stream(tail):
-            self._phase(4, b, left, lv, rv, out, N, tail, hints, validhints)
+            self._phase(4, b, left, lv, rv, out, N, tail, hints, validhints, info)
             ev = torch.cuda.Event(); ev.record(tail)
             self.tail_done[b] = ev
         caller.wait_event(ev)
         self.lv, self.rv = self.lv2[b], self.rv2[b]     # the projected pair of the latest call
         return out
 
-    def run_device_serial(self, left, right, hints, out=None, step=None, validhints=None):
+    def run_device_serial(self, left, right, hints, out=None, step=None, validhints=None, info_out=None):
         """The same computation, everything in order on the current stream (no overlap between calls, no internal streams
-        except the right-image branches): what bench.py times stage by stage."""
+        except the right-image branches): what bench.py times stage by stage.  match_info / info_out as in run_device."""
         torch = self.torch
-        N = self._check(left, right, hints, out, validhints=validhints)
+        N = self._check(left, right, hints, out, validhints=validhints, info_out=info_out)
         with torch.cuda.device(self.device):
-            return self._run_device_serial(left, right, hints, validhints, out, step, N)
+            info = self._info_out(info_out, N)
+            out = self._run_device_serial(left, right, hints, validhints, out, step, N, info)
+            return (out, info) if self.match_info else out
 
-    def _run_device_serial(self, left, right, hints, validhints, out, step, N):
+    def _run_device_serial(self, left, right, hints, validhints, out, step, N, info=None):
         torch = self.torch
         out = self.disp[:N] if out is None else out
         st = torch.cuda.current_stream(self.device)
@@ -374,14 +419,15 @@ class VppRsgmPipeline:
         seed = self._next_seed(step)
         lv.copy_(left); rv.copy_(right)
         self._vpp(left, lv, rv, hints, seed, N, st, self.status)
-        self._phase(7, b, left, lv, rv, out, N, st, hints, validhints)
+        self._phase(7, b, left, lv, rv, out, N, st, hints, validhints, info)
         for s in (self.vpp_stream, self.main_stream, self.tail_stream):
             s.wait_stream(st)
         self.lv, self.rv = self.lv2[b], self.rv2[b]
         return out
 
     def run_host(self, left, right, hints, validhints=None):
-        """Host tensors (ideally pinned) in, pinned host float32 [N,H,W] out; the copies are part of the call."""
+        """Host tensors (ideally pinned) in, pinned host float32 [N,H,W] out; the copies are part of the call.  match_info
+        pipelines return (disp, info) with info on pinned host memory too (valid until the next run_host)."""
         torch = self.torch
         N = self._check(left, right, hints, host=True, validhints=validhints)
         with torch.cuda.device(self.device):
@@ -394,13 +440,19 @@ class VppRsgmPipeline:
                 dv.copy_(validhints, non_blocking=True)
             if self.status_host is not None:
                 self.status_host.zero_()          # current stream: the front phase below waits for it (inputs_ready=None)
-            out = self._run_device(self.d_left[:N], self.d_right[:N], self.d_hints[:N], dv, None, None, None, N, self.status_host)
+            info = self._info_out(None, N)
+            out = self._run_device(self.d_left[:N], self.d_right[:N], self.d_hints[:N], dv, None, None, None, N, self.status_host, info)
             self.h_disp[:N].copy_(out, non_blocking=True)
+            if info is not None:
+                for k, t in info.items():
+                    self.h_info[k][:N].copy_(t, non_blocking=True)
             torch.cuda.current_stream(self.device).synchronize()
             if self.status_host is not None:
                 bad = self.status_host[:N].cpu().numpy()     # the current stream is idle: this reads this call's words
                 if bad.any():
                     self._raise_degenerate(bad, "this run_host batch")
+        if self.match_info:
+            return self.h_disp[:N], self._info_slice(self.h_info, N)
         return self.h_disp[:N]
 
     # ---- streaming front-end: overlapped host<->device copies ---------------------------------------------------
@@ -416,6 +468,8 @@ class VppRsgmPipeline:
                                      h_disp=torch.empty((self.N, self.H, self.W), dtype=torch.float32).pin_memory(),
                                      status=torch.empty_like(self.status) if self.status is not None else None,
                                      h_status=torch.zeros(self.N, dtype=torch.int32).pin_memory(),
+                                     info=self._info_buffers(self.device) if self.match_info else None,
+                                     h_info=self._info_buffers("cpu") if self.match_info else None,
                                      copied_in=torch.cuda.Event(), computed=torch.cuda.Event(), copied_out=torch.cuda.Event(),
                                      busy=False))
                 self._stream_sets = dict(sets=sets, h2d=torch.cuda.Stream(self.device), d2h=torch.cuda.Stream(self.device), turn=0)
@@ -447,14 +501,18 @@ class VppRsgmPipeline:
                     st["status"].zero_()                 # this batch's own status words (read back with its disparities)
                 st["copied_in"].record(ss["h2d"])
             compute.wait_event(st["copied_in"])
+            info = self._info_slice(st["info"], N) if self.match_info else None
             self._run_device(st["left"][:N], st["right"][:N], st["hints"][:N], st["valid"][:N] if self.guided else None,
-                             st["disp"][:N], st["copied_in"], None, N, st["status"])
+                             st["disp"][:N], st["copied_in"], None, N, st["status"], info)
             st["computed"].record(compute)
             if on_computed is not None:
                 on_computed(st["disp"][:N])
             with torch.cuda.stream(ss["d2h"]):
                 ss["d2h"].wait_event(st["computed"])
                 st["h_disp"][:N].copy_(st["disp"][:N], non_blocking=True)
+                if info is not None:
+                    for k, t in info.items():
+                        st["h_info"][k][:N].copy_(t, non_blocking=True)
                 if st["status"] is not None:
                     st["h_status"][:N].copy_(st["status"][:N], non_blocking=True)
                 st["copied_out"].record(ss["d2h"])
@@ -464,7 +522,7 @@ class VppRsgmPipeline:
 
     def collect(self, ticket):
         """Wait for a submitted batch; returns its pinned host float32 [N,H,W] disparities (valid until that staging set is
-        reused by the `host_depth`-th submit_host after it was submitted).  use_distance_patch: ZeroDivisionError if this
+        reused by the `host_depth`-th submit_host after it was submitted); match_info pipelines: (disp, info), info pinned too.  use_distance_patch: ZeroDivisionError if this
         batch has a frame whose hints all have one value (see _raise_degenerate); the batches around it are unaffected."""
         st = self._streaming()["sets"][ticket]
         if not st["busy"]:
@@ -473,4 +531,6 @@ class VppRsgmPipeline:
         st["busy"] = False
         if st["status"] is not None and st["h_status"][:st["n"]].any():
             self._raise_degenerate(st["h_status"][:st["n"]].numpy(), f"the batch of ticket {ticket}")
+        if self.match_info:
+            return st["h_disp"][:st["n"]], self._info_slice(st["h_info"], st["n"])
         return st["h_disp"][:st["n"]]
